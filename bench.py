@@ -4,7 +4,7 @@
 One step = one pass of the hot path (`TouchedRegraster.predict5`, need=False, eval) over one batch of 64
 synthetic piece pairs per GPU (BASELINE.json configs[1]).  Prints ONE JSON line (rank 0).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--precision split|bf16|fp32]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--precision split|bf16|fp32] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
   python bench.py --impl reference ...     # the reference algorithm's CPU path (oracle port), same metric and config
 
@@ -25,6 +25,9 @@ e2e   : same metric through the public API from pinned HOST buffers: H2D of both
         twist + both boundary-logit tensors inside the timed region.
 parity: the outputs the LAST e2e step copied to the host, checked against the CPU oracle on 8 pairs of that batch (pairs
         are independent in eval mode), plus the same check of the other precisions' outputs on the same batch.
+--dump-outputs DIR : what predict5 returned in the last step of the value leg (twist `out` [64,6], boundary logits
+        `de_fpcb` / `de_mrpcb` [64,2,1024]) as DIR/<name>.npy.  Inputs and weights are seeded, so two builds run with the
+        same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -177,7 +180,7 @@ def cpu_baseline_protocol():
     cores = os.cpu_count() or 1
     out = {"cpu_model": _cpu_model(), "cores": cores, "kind": "port",
            "what": "oracle.puzzle_oracle.predict5 = the reference's torch-CPU op sequence (pinned against the unmodified "
-                   "reference by tests/test_oracle_vs_reference.py), fp32, eval mode"}
+                   "reference's stored outputs by tests/test_oracle_golden.py), fp32, eval mode"}
 
     def summarise(times, pairs):
         return {"pairs_per_call": pairs, "reps": len(times), "s_min": min(times), "s_median": statistics.median(times),
@@ -580,11 +583,14 @@ def run_gpu_arm(args):
     h2d = sum(t.numel() * t.element_size() for t in host[0])
     d2h = sum(t.numel() * t.element_size() for t in out_hosts[0])
 
+    last_resident = {}        # what predict5 returned in the last step of the latest run_resident (--dump-outputs)
+
     def run_resident(n):
         for i in range(n):
             with torch.cuda.stream(pipes[i % len(pipes)]):
                 bt, st_ = rot[i % n_rot]
-                model.predict5(bt, 0, starts=st_)
+                r = model.predict5(bt, 0, starts=st_)
+        last_resident.update(out=r[0], de_fpcb=r[2], de_mrpcb=r[3])
 
     def step_e2e(i):
         f, m, s = host[i % nsets]
@@ -633,6 +639,8 @@ def run_gpu_arm(args):
         return v, e
 
     value_regions, e2e_regions = pipelined(args.precision, args.repeats)
+    # the headline's last timed step (last value region, step K-1, batch rot[(K-1) % n_rot]): its outputs for --dump-outputs
+    dump = {k: v.float().cpu().numpy() for k, v in last_resident.items()} if args.dump_outputs else None
     # the outputs of the LAST e2e step are in its pinned host slot: keep them for the parity check below
     last = args.steps - 1
     e2e_last = tuple(t.clone() for t in out_hosts[last % len(out_hosts)])
@@ -875,6 +883,11 @@ def run_gpu_arm(args):
         "wall_s_single_stream_region": wall,
     }
     line = {k: v for k, v in line.items() if not (k.endswith("_path") and v is None)}
+    if dump is not None:
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dump.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     emit_line(line)
     if world > 1:
         dist.destroy_process_group()
@@ -921,7 +934,11 @@ def main():
     ap.add_argument("--pipes", type=int, default=4, help="CUDA streams the value / e2e legs alternate batches over")
     ap.add_argument("--no-graphs", action="store_true", help="value / e2e legs: eager launches instead of CUDA-graph replay")
     ap.add_argument("--no-extras", action="store_true", help="skip the short config 3 / 4 / 5 / EMD runs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline path returned (rank 0) as DIR/<name>.npy, float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     args.repeats = max(args.repeats, 1)
     # stdout carries exactly ONE JSON line: libraries that write to file descriptor 1 themselves (NCCL prints its version

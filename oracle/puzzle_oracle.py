@@ -9,8 +9,7 @@ reference`` legs may import it.
 Pinning: the reference has no golden vectors for this part of the path
 (SURVEY.md §8c) -- it is pinned by executing the unmodified reference torch
 code in the build container (``oracle/make_golden.py`` -> ``tests/golden/``)
-and by ``tests/test_oracle_vs_reference.py`` which runs both side by side
-when ``/root/reference`` is present.
+and comparing with those stored outputs (``tests/test_oracle_golden.py``).
 
 Everything is functional: weights come in as a ``state_dict``-style mapping
 with the reference's key names (SURVEY.md Appendix C), so the same dictionary

@@ -4,8 +4,7 @@ Only usable in the build container, where ``/root/reference`` exists; nothing
 under ``tests/ -m gpu``, ``smoke()`` or ``bench.py`` may import this module
 (the GPU box has no reference tree).  It is used by ``oracle/make_golden.py``
 to execute the reference's own torch code on the CPU and freeze the results
-as fixtures under ``tests/golden/``, and by ``tests/test_oracle_vs_reference.py``
-(auto-skipped when the tree is absent) to pin the restatement in
+as fixtures under ``tests/golden/``, which pin the restatement in
 ``oracle/puzzle_oracle.py`` against the real thing.
 
 Why a shim is needed (SURVEY.md D4): ``model5_b.py`` imports modules that are

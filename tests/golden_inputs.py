@@ -53,6 +53,25 @@ def training_inputs(batch, se3_exp):
     return [fpc, mrpc, igt, rpc, fpcb, rpcb, fpc_idx, rpc_idx]
 
 
+EMD_CASES = [(4, 1024, 1024), (3, 128, 128), (2, 96, 200)]      # (b, n, m) of the EMD kernel goldens
+EMD_MATCH_SAMPLE = 49152                                       # match entries stored per case (all of them if fewer)
+
+
+def emd_inputs(b, n, m):
+    """Clouds xyz1 (b,n,3), xyz2 (b,m,3) of one EMD kernel golden case, and the flat indices into match (b,m,n) whose
+    values are stored: every entry of a small match, a fixed random sample of a large one (the full (4,1024,1024)
+    match is 16 MB)."""
+    g = torch.Generator().manual_seed(n)
+    x1 = torch.randn(b, n, 3, generator=g) * 0.5
+    x2 = torch.randn(b, m, 3, generator=g) * 0.5
+    total = b * m * n
+    if total <= EMD_MATCH_SAMPLE:
+        idx = torch.arange(total)
+    else:
+        idx = torch.randperm(total, generator=torch.Generator().manual_seed(total))[:EMD_MATCH_SAMPLE].sort().values
+    return x1, x2, idx
+
+
 def pointnet_block_inputs():
     g = torch.Generator().manual_seed(17)
     return torch.rand(2, 200, 3, generator=g) - 0.5, torch.randn(2, 200, 8, generator=g)
