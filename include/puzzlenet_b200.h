@@ -42,7 +42,7 @@ typedef void* pz_stream_t; /* cudaStream_t */
 #define PZ_PREC_SPLIT 2 /* every operand as an fp16 hi/lo pair, three tcgen05 MMAs per product (hi*hi + hi*lo + lo*hi),
                          * fp32 accumulate: the tensor-core path that meets the fp32 tolerances (1e-4, 0.01 deg) */
 
-#define PZ_ABI_VERSION 5
+#define PZ_ABI_VERSION 6
 
 /* pz_predict5 flags */
 #define PZ_FLAG_NEED 1          /* also return x2 / attention of both clouds (predict5 need=True) */
@@ -237,6 +237,46 @@ int pz_predict5(const PzEncoderWeights* enc_host /*[2]*/, const PzHeadWeights* h
                 int flags, float* out6, float* de_fpcb, float* de_mrpcb, float* x2_fpc,
                 float* attention_fpc, float* x2_mrpc, float* attention_mrpc, void* workspace,
                 size_t workspace_bytes, pz_stream_t stream);
+
+/* Pair scoring from per-piece encodings: pz_predict5 split at its pair boundary.  Everything pz_predict5 computes
+ * before the pair meets -- both encoders, MLPLocalPre{Fpc,Rpc} and the mrpc boundary head -- depends on one cloud
+ * only, so pz_encode_pieces runs it once per piece, and pz_predict_pairs evaluates any list of (i, j) pairs from that
+ * state with the pose MLP and the fpc boundary head alone.  Per-piece state, caller-owned, for P pieces:
+ * role 0 = the piece as fpc (Encoder, MLPLocalPreFpc), role 1 = the piece as mrpc (Encoder2, MLPLocalPreRpc).
+ * Every buffer must be 16-byte aligned (PZ_ERR_ARG otherwise). */
+#define PZ_MAX_PIECES 4095      /* pieces per pz_encode_pieces call */
+#define PZ_MAX_PAIRS (1 << 20)  /* pairs per pz_predict_pairs call */
+typedef struct PzPieceEmbeddings {
+  float* f_global; /* [2,P,1024]    f_global of the piece through Encoder (role 0) and Encoder2 (role 1) */
+  float* local;    /* [2,P,1024,64] MLPLocalPreFpc(x_feature_E) (role 0), MLPLocalPreRpc(x_feature_E2) (role 1) */
+  float* tilemax;  /* [2,P,8,64]    column maxima of each role's local features per 128-point tile; the max over a
+                    *               role-1 piece's 8 tiles is the D6 global feature of that piece as mrpc */
+  float* de_mrpcb; /* [P,2,1024]    mrpc boundary logits: they depend on the mrpc piece only */
+} PzPieceEmbeddings;
+
+/* clouds [P,1024,3]; starts [4,P] in pz_predict5's order (Encoder s1, Encoder s2, Encoder2 s1, Encoder2 s2).
+ * Runs pz_predict5's front half on the batch [clouds; clouds] and fills every field of *emb_host.  With the same
+ * clouds and starts, the embeddings of piece p are those pz_predict5(fpc = mrpc = clouds) forms for pair p.
+ * flags: PZ_FLAG_REUSE_PACKS as in pz_predict5 (PZ_FLAG_NEED is not supported).  Supported: 1 <= P <= PZ_MAX_PIECES
+ * (encode larger sets in several calls), precision
+ * fp32 / bf16 / split; the legacy bf16 heads selected by the environment variable PZ_HEADS_BF16=1 are not supported
+ * (PZ_ERR_UNSUPPORTED). */
+size_t pz_encode_pieces_workspace_bytes(int P);
+int pz_encode_pieces(const PzEncoderWeights* enc_host /*[2]*/, const PzHeadWeights* heads_host, const float* clouds,
+                     int P, const int64_t* starts, int precision, int flags, const PzPieceEmbeddings* emb_host,
+                     void* workspace, size_t workspace_bytes, pz_stream_t stream);
+
+/* pairs [n,2] int64 (i = fpc piece, j = mrpc piece; i == j and repeats allowed; indices must lie in [0,P))
+ * -> out6 [n,6], de_fpcb [n,2,1024], de_mrpcb [n,2,1024]: what pz_predict5 returns for the pair (clouds[i], clouds[j])
+ * with the starts the pieces were encoded with, computed by the same kernels (pose MLP on [f_global[0,i],
+ * f_global[1,j]]; fpc boundary head on local[0,i] with the global feature of piece j; de_mrpcb[j] copied).
+ * emb_host must have been filled by pz_encode_pieces with the same weights and precision.  n == 0 is a no-op.
+ * de_mrpcb must be 16-byte aligned.  Supported: P >= 1, n <= PZ_MAX_PAIRS (split larger lists).
+ * flags: PZ_FLAG_REUSE_PACKS as in pz_predict5. */
+size_t pz_predict_pairs_workspace_bytes(int n);
+int pz_predict_pairs(const PzHeadWeights* heads_host, const PzPieceEmbeddings* emb_host, int P, const int64_t* pairs,
+                     int n, int precision, int flags, float* out6, float* de_fpcb, float* de_mrpcb, void* workspace,
+                     size_t workspace_bytes, pz_stream_t stream);
 
 /* se3.exp(x) -- se_math/se3.py:57-80.  twist [B,6] (omega, v) -> g [B,4,4]. */
 int pz_se3_exp(const float* twist, int B, float* g, pz_stream_t stream);

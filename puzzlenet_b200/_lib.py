@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libpuzzlenet_sm100.so")
 PZ_PREC_FP32 = 0
 PZ_PREC_BF16 = 1
 PZ_PREC_SPLIT = 2
-ABI_VERSION = 5
+ABI_VERSION = 6
 PZ_SCORE_COLS = 12
 PZ_FLAG_NEED = 1
 PZ_FLAG_REUSE_PACKS = 2
@@ -41,6 +41,10 @@ class PzEncoderOutputs(C.Structure):
 class PzHeadWeights(C.Structure):
     _fields_ = ([("tf_w", C.c_void_p * 5), ("tf_b", C.c_void_p * 5)]
                 + [(f"{n}_{s}", C.c_void_p * 3) for n in ("pre_fpc", "pre_rpc", "seg_fpc", "seg_rpc") for s in ("w", "b")])
+
+
+class PzPieceEmbeddings(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("f_global", "local", "tilemax", "de_mrpcb")]
 
 
 # name -> (restype, argtypes); mirrors include/puzzlenet_b200.h one to one
@@ -79,6 +83,12 @@ SIGNATURES = {
     "pz_predict5": (C.c_int, [C.POINTER(PzEncoderWeights), C.POINTER(PzHeadWeights), c_f32p, c_f32p, C.c_int, c_i64p,
                               C.c_int, C.c_int, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, c_f32p, C.c_void_p,
                               C.c_size_t, c_stream]),
+    "pz_encode_pieces_workspace_bytes": (C.c_size_t, [C.c_int]),
+    "pz_encode_pieces": (C.c_int, [C.POINTER(PzEncoderWeights), C.POINTER(PzHeadWeights), c_f32p, C.c_int, c_i64p,
+                                   C.c_int, C.c_int, C.POINTER(PzPieceEmbeddings), C.c_void_p, C.c_size_t, c_stream]),
+    "pz_predict_pairs_workspace_bytes": (C.c_size_t, [C.c_int]),
+    "pz_predict_pairs": (C.c_int, [C.POINTER(PzHeadWeights), C.POINTER(PzPieceEmbeddings), C.c_int, c_i64p, C.c_int,
+                                   C.c_int, C.c_int, c_f32p, c_f32p, c_f32p, C.c_void_p, C.c_size_t, c_stream]),
     "pz_se3_exp": (C.c_int, [c_f32p, C.c_int, c_f32p, c_stream]),
     "pz_chamfer": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, c_f32p, c_f32p, C.c_void_p, C.c_void_p, c_stream]),
     "pz_chamfer_grad": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, c_f32p, c_f32p,

@@ -6,8 +6,9 @@ alignment -- the quantity ``test_step`` computes as ``cd_fpc`` / ``cd_rpc`` (mod
 greedily.  This module supplies
 
 * :func:`downsample_pieces` -- FPS 11000 -> 1024 of every piece, pieces sharded over ranks, one ``all_gather``;
-* :func:`score_pairs` / :func:`score_all_pairs` -- batched ``predict5`` + one ``pz_pair_score`` launch per batch,
-  candidate pairs sharded over ranks, ONE ``all_gather`` of ``[n_pairs, 8]`` rows (twist 6, score, 1.0);
+* :func:`score_pairs` / :func:`score_all_pairs` -- batched ``predict5`` + one ``pz_pair_score`` launch per batch
+  (:class:`ModelScorer`), or per-piece encodings + pair heads (:class:`EmbeddingScorer`), candidate pairs sharded over
+  ranks, ONE ``all_gather`` of ``[n_pairs, 8]`` rows (twist 6, score, 1.0);
 * :func:`greedy_assemble` -- host-side greedy merge (Kruskal over the score table) composing the pair poses into one
   pose per piece;
 * :func:`assemble` -- the optional re-scoring loop: after each merge the merged piece is re-sampled to 1024 points
@@ -57,6 +58,61 @@ class ModelScorer:
         return rows
 
 
+class EmbeddingScorer:
+    """``scorer.score_indexed(clouds [P,1024,3], pairs [n,2]) -> rows [n, ROW_COLS]``: the rows :class:`ModelScorer`
+    gives, computed from per-piece encodings -- every piece goes through both encoders once
+    (``TouchedRegraster.encode_pieces``), each pair through the pose MLP and the fpc boundary head only
+    (``predict_pairs``), then one ``pz_pair_score`` launch.
+
+    The scorer keeps the embeddings of the clouds it last saw and a device copy of those clouds.  On each call it
+    compares the copy with ``clouds`` (one host synchronisation) and re-encodes only the pieces whose rows changed, so
+    ``assemble(rescore=True)`` re-encodes one piece per merge; a change of the model's parameters or precision
+    re-encodes every piece.  FPS starts are drawn from the CPU generator as ``encode_pieces`` / ``reencode`` draw them.
+    Under ``torch.distributed`` the pairs stay sharded by :func:`score_all_pairs` and every rank encodes all P pieces
+    itself (replicated work, cheap at P = 32); the ranks' CPU generators must then be seeded alike, as they are for
+    ``ModelScorer``.  Pairs are scored ``chunk`` at a time (one ``predict_pairs`` and one ``pz_pair_score`` per chunk),
+    which bounds the memory of a call."""
+
+    def __init__(self, model, chunk: int = 4096):
+        self.model = model
+        self.chunk = max(1, int(chunk))
+        self.emb = None
+        self._clouds = None
+        self.encoded = 0          # pieces encoded so far
+
+    def _refresh(self, clouds: torch.Tensor) -> None:
+        emb, m = self.emb, self.model
+        if (emb is None or self._clouds.shape != clouds.shape or self._clouds.device != clouds.device
+                or not emb.is_current(m)):
+            self.emb = m.encode_pieces(clouds)
+            self._clouds = clouds.clone()
+            self.encoded += clouds.shape[0]
+            return
+        changed = torch.nonzero((self._clouds != clouds).flatten(1).any(1)).flatten().tolist()
+        if changed:
+            emb.reencode(m, changed, clouds[changed])
+            self._clouds[changed] = clouds[changed]
+            self.encoded += len(changed)
+
+    def score_indexed(self, clouds: torch.Tensor, pairs: torch.Tensor) -> torch.Tensor:
+        from . import losses
+        rows = torch.empty(pairs.shape[0], ROW_COLS, device=clouds.device, dtype=torch.float32)
+        if pairs.shape[0] == 0:
+            return rows
+        clouds = clouds.contiguous().float()
+        self._refresh(clouds)
+        for lo in range(0, pairs.shape[0], self.chunk):
+            sel = pairs[lo:lo + self.chunk]
+            out6, _, de_f, de_m = self.model.predict_pairs(self.emb, sel)
+            idx = sel.to(clouds.device)
+            s = losses.pair_score(out6, de_f, de_m, clouds[idx[:, 0]], clouds[idx[:, 1]])
+            r = rows[lo:lo + sel.shape[0]]
+            r[:, :6] = out6
+            r[:, 6] = s[:, 10]
+            r[:, 7] = 1.0
+        return rows
+
+
 def downsample_pieces(pieces: Sequence, npoints: int = 1024, starts: Optional[Sequence[int]] = None,
                       device=None) -> torch.Tensor:
     """[P, npoints, 3]: every raw piece ([N_i, 3], N_i <= 16384) farthest-point-sampled on the GPU
@@ -78,7 +134,10 @@ def downsample_pieces(pieces: Sequence, npoints: int = 1024, starts: Optional[Se
 
 def score_pairs(clouds: torch.Tensor, pairs: torch.Tensor, scorer: Callable, batch: int = 64) -> torch.Tensor:
     """rows [len(pairs), ROW_COLS] for the given (i, j) index pairs: piece i is the fixed cloud (``fpc``), piece j
-    the one the predicted pose moves (``mrpc``).  Local, no communication."""
+    the one the predicted pose moves (``mrpc``).  Local, no communication.  A scorer with ``score_indexed`` (such as
+    :class:`EmbeddingScorer`) gets the whole list at once."""
+    if hasattr(scorer, "score_indexed"):
+        return scorer.score_indexed(clouds, pairs)
     n = pairs.shape[0]
     rows = torch.empty(n, ROW_COLS, device=clouds.device, dtype=torch.float32)
     pairs = pairs.to(clouds.device)

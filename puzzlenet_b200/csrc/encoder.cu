@@ -676,22 +676,32 @@ __global__ void __launch_bounds__(128) head_local_kernel(const float* __restrict
                          outs[(i * 4 + 3) * 128 + tid]);
 }
 
-// gbias[set][b][k] = W0_set[k, 0:64] . g[b] + b0_set[k]   (the "global" half of MLP{F,R}pcb.0)
-__global__ void __launch_bounds__(64) seg_bias_kernel(const float* __restrict__ g, const float* w0a,
+// gbias[set][b][k] = W0_set[k, 0:64] . g[r] + b0_set[k]   (the "global" half of MLP{F,R}pcb.0), r = b, or pairs[b,1]
+// when a pair list is given.  g [rows, tiles, 64]: the global feature of row r is the max over its `tiles` vectors.
+__global__ void __launch_bounds__(64) seg_bias_kernel(const float* __restrict__ g, int tiles,
+                                                      const int64_t* __restrict__ pairs, const float* w0a,
                                                       const float* b0a, const float* w0b, const float* b0b, int B,
                                                       float* __restrict__ gbias) {
   const int b = blockIdx.x, set = blockIdx.y, k = threadIdx.x;
   const float* w0 = set == 0 ? w0a : w0b;
   const float* b0 = set == 0 ? b0a : b0b;
+  const float* gr = g + (size_t)(pairs ? pairs[2 * b + 1] : b) * tiles * 64;
   float v = b0[k];
-  for (int i = 0; i < 64; ++i) v = fmaf(w0[k * 128 + i], g[b * 64 + i], v);
+  for (int i = 0; i < 64; ++i) {
+    float gi = gr[i];
+    for (int t = 1; t < tiles; ++t) gi = fmaxf(gi, gr[t * 64 + i]);
+    v = fmaf(w0[k * 128 + i], gi, v);
+  }
   gbias[((size_t)set * B + b) * 64 + k] = v;
 }
 
-// MLP{F,R}pcb on cat([global, local]): 128-64-32-2, logits stored as [B,2,1024] (model5_b.py:751-754)
+// MLP{F,R}pcb on cat([global, local]): 128-64-32-2, logits stored as [B,2,1024] (model5_b.py:751-754).
+// pairs == null: cloud c of the 2B (set = c / B, b = c % B) reads local[c].  pairs [B,2]: every cloud is a pair of
+// set 0 and pair b reads local[pairs[b,0]].  Either way the bias is gbias[set][b] and the logits go to row b.
 __global__ void __launch_bounds__(128) head_seg_kernel(const float* __restrict__ local, Mlp3W wa, Mlp3W wb,
                                                        const float* __restrict__ gbias, int B,
-                                                       float* __restrict__ de_a, float* __restrict__ de_b) {
+                                                       float* __restrict__ de_a, float* __restrict__ de_b,
+                                                       const int64_t* __restrict__ pairs) {
   extern __shared__ __align__(16) float hs_smem[];
   float* w0s = hs_smem;            // [64][64] local half of layer 0
   float* w1s = w0s + 64 * 64;      // [32][64]
@@ -716,7 +726,8 @@ __global__ void __launch_bounds__(128) head_seg_kernel(const float* __restrict__
   if (tid < 2) b2s[tid] = w.b2[tid];
   __syncthreads();
   float a[64];
-  const float4* src = reinterpret_cast<const float4*>(local + p * 64);
+  const size_t row = pairs ? (size_t)pairs[2 * b] * NPTS + n : p;
+  const float4* src = reinterpret_cast<const float4*>(local + row * 64);
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
     float4 x = src[i];
@@ -1770,6 +1781,19 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
   return 0;
 }
 
+// PZ_HEADS_BF16=1 selects the former bf16 boundary heads on the bf16 path (A/B hook)
+static bool old_bf16_heads() {
+  static const bool v = getenv("PZ_HEADS_BF16") && getenv("PZ_HEADS_BF16")[0] == '1';
+  return v;
+}
+constexpr size_t HL_SMEM = (3 * 4160 + 64 * 128) * sizeof(float);
+constexpr size_t HS_SMEM = (64 * 64 + 32 * 64 + 64 + 32 + 64 + 4 + 64 * 128) * sizeof(float);
+static int set_head_fp32_smem() {
+  PZ_CUDA(cudaFuncSetAttribute(head_seg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HS_SMEM));
+  PZ_CUDA(cudaFuncSetAttribute(head_local_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)HL_SMEM));
+  return 0;
+}
+
 }  // namespace pz
 
 using namespace pz;
@@ -1847,30 +1871,15 @@ extern "C" size_t pz_predict5_workspace_bytes(int B) {
   return align_up(predict_layout(B, a, s), 256);
 }
 
-extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights* heads_host, const float* fpc,
-                           const float* mrpc, int B, const int64_t* starts, int precision, int flags, float* out6,
-                           float* de_fpcb, float* de_mrpcb, float* x2_fpc, float* attention_fpc, float* x2_mrpc,
-                           float* attention_mrpc, void* workspace, size_t workspace_bytes, pz_stream_t stream) {
-  PZ_REQUIRE(enc_host && heads_host && fpc && mrpc && starts && out6 && de_fpcb && de_mrpcb, PZ_ERR_ARG,
-             "pz_predict5: null pointer");
-  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "pz_predict5: B must be >= 1");
-  const int need = flags & PZ_FLAG_NEED;
-  const bool reuse_pack = (flags & PZ_FLAG_REUSE_PACKS) != 0;
-  if (need)
-    PZ_REQUIRE(x2_fpc && attention_fpc && x2_mrpc && attention_mrpc, PZ_ERR_ARG,
-               "pz_predict5: need=1 requires the x2/attention outputs");
-  {
-    const void* const* p = reinterpret_cast<const void* const*>(heads_host);
-    for (size_t i = 0; i < sizeof(PzHeadWeights) / sizeof(void*); ++i)
-      PZ_REQUIRE(p[i], PZ_ERR_ARG, "pz_predict5: head weight %zu is null", i);
-  }
-  cudaStream_t st = as_stream(stream);
-  Arena arena(workspace, workspace_bytes);
-  PredictScratch s;
-  predict_layout(B, arena, s);
-  PZ_REQUIRE(workspace && arena.ok(), PZ_ERR_WORKSPACE, "pz_predict5: workspace %zu B < required %zu B",
-             workspace_bytes, arena.used);
-  prof_begin(st);
+namespace {
+// pz_predict5's front half, shared with pz_encode_pieces: both clouds into one [2B,1024,3] batch, both encoders, and
+// the boundary heads from the encoder's after-stem hook.  local [2B,1024,64] and tilemax [2B,8,64] receive the heads'
+// per-cloud state (tilemax on the tensor-core paths only; the fp32 heads pool into s.gmax); the rest of `eo` and
+// fglob_pair are as in encoder_forward_impl.
+int predict_front(const PzEncoderWeights* enc_host, const PzHeadWeights& h, const float* fpc, const float* mrpc, int B,
+                  const int64_t* starts, int precision, bool reuse_pack, const PredictScratch& s,
+                  const PzEncoderOutputs& eo, float* fglob_pair, float* local, float* tilemax, float* de_fpcb,
+                  float* de_mrpcb, cudaStream_t st) {
   const size_t cloud_bytes = (size_t)B * NPTS * 3 * sizeof(float);
   // both clouds into one [2B, 1024, 3] batch; starts [4,B]: (Encoder s1, Encoder s2, Encoder2 s1, Encoder2 s2) -> st1 =
   // rows 0,2; st2 = rows 1,3.  One launch instead of six copy operations (each ~4 us of stream time).
@@ -1889,19 +1898,6 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
   }
 
   prof_mark("stage_inputs", st);
-  PzEncoderOutputs eo = {};
-  float* x2_all = nullptr;
-  float* attn_all = nullptr;
-  // need=True: the encoder writes contiguous [2B,..] tensors but the caller's four outputs are
-  // separate, so attention [2B,256,256] and x2 [2B,256,3] go through scratch that is free until
-  // the heads run (`local`, `partial`) and are copied out per half.
-  if (need) {
-    attn_all = s.local;                                    // 2B*65536 floats == 2B*1024*64
-    x2_all = s.partial;                                    // 2B*768 floats  <= 16*B*1024
-    eo.attention = attn_all;
-    eo.x2 = x2_all;
-  }
-  const PzHeadWeights& h = *heads_host;
   const Mlp3W pre_f = {h.pre_fpc_w[0], h.pre_fpc_b[0], h.pre_fpc_w[1], h.pre_fpc_b[1], h.pre_fpc_w[2], h.pre_fpc_b[2]};
   const Mlp3W pre_r = {h.pre_rpc_w[0], h.pre_rpc_b[0], h.pre_rpc_w[1], h.pre_rpc_b[1], h.pre_rpc_w[2], h.pre_rpc_b[2]};
   const Mlp3W seg_f = {h.seg_fpc_w[0], h.seg_fpc_b[0], h.seg_fpc_w[1], h.seg_fpc_b[1], h.seg_fpc_w[2], h.seg_fpc_b[2]};
@@ -1909,12 +1905,11 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
   const int P = 2 * B * NPTS;
 
   // boundary heads (model5_b.py:738-754): they only need x_feature, so the encoder runs them right after its stem
-  static const bool old_bf16_heads = getenv("PZ_HEADS_BF16") && getenv("PZ_HEADS_BF16")[0] == '1';   // A/B hook
   AfterStem heads_fn = [&](const float* xfeat, const __nv_bfloat16* xfeat_b) -> int {
-    if (precision == PZ_PREC_SPLIT || (precision == PZ_PREC_BF16 && !old_bf16_heads)) {
+    if (precision == PZ_PREC_SPLIT || (precision == PZ_PREC_BF16 && !old_bf16_heads())) {
       // split-fp16 chained-MMA heads on the fp32 x_feature (heads_split.cu): logits at fp32 tolerance in both
       // tensor-core precisions (the bf16 path's stem is a split product too, so its x_feature is fp32-accurate)
-      PZ_TRY(launch_heads_split(xfeat, pre_f, pre_r, seg_f, seg_r, B, reuse_pack, s.himg_split, s.local, s.tilemax, de_fpcb,
+      PZ_TRY(launch_heads_split(xfeat, pre_f, pre_r, seg_f, seg_r, B, reuse_pack, s.himg_split, local, tilemax, de_fpcb,
                                 de_mrpcb, st));
       prof_mark("boundary_heads", st);
       return 0;
@@ -1948,26 +1943,80 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
       prof_mark("boundary_heads", st);
       return 0;
     }
-    const size_t hl_smem = (3 * 4160 + 64 * 128) * sizeof(float);
-    const size_t hs_smem = (64 * 64 + 32 * 64 + 64 + 32 + 64 + 4 + 64 * 128) * sizeof(float);
-    PZ_CUDA(cudaFuncSetAttribute(head_seg_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hs_smem));
-    PZ_CUDA(cudaFuncSetAttribute(head_local_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hl_smem));
-    head_local_kernel<<<P / 128, 128, hl_smem, st>>>(xfeat, pre_f, pre_r, B, s.local);
+    PZ_TRY(set_head_fp32_smem());
+    head_local_kernel<<<P / 128, 128, HL_SMEM, st>>>(xfeat, pre_f, pre_r, B, local);
     PZ_LAUNCH_CHECK();
     // D6: BOTH heads use the max-pool of the *mrpc* local features (model5_b.py:741-744)
-    rowblock_max_kernel<<<dim3(1, B), 256, 0, st>>>(s.local + (size_t)B * NPTS * 64, 64, NPTS, 64, B, B, 0, s.gmax, 64);
+    rowblock_max_kernel<<<dim3(1, B), 256, 0, st>>>(local + (size_t)B * NPTS * 64, 64, NPTS, 64, B, B, 0, s.gmax, 64);
     PZ_LAUNCH_CHECK();
-    seg_bias_kernel<<<dim3(B, 2), 64, 0, st>>>(s.gmax, h.seg_fpc_w[0], h.seg_fpc_b[0], h.seg_rpc_w[0], h.seg_rpc_b[0], B, s.gbias);
+    seg_bias_kernel<<<dim3(B, 2), 64, 0, st>>>(s.gmax, 1, nullptr, h.seg_fpc_w[0], h.seg_fpc_b[0], h.seg_rpc_w[0],
+                                               h.seg_rpc_b[0], B, s.gbias);
     PZ_LAUNCH_CHECK();
-    head_seg_kernel<<<P / 128, 128, hs_smem, st>>>(s.local, seg_f, seg_r, s.gbias, B, de_fpcb, de_mrpcb);
+    head_seg_kernel<<<P / 128, 128, HS_SMEM, st>>>(local, seg_f, seg_r, s.gbias, B, de_fpcb, de_mrpcb, nullptr);
     PZ_LAUNCH_CHECK();
     prof_mark("boundary_heads", st);
     return 0;
   };
 
-  const float* xfeat = nullptr;
-  PZ_TRY(encoder_forward_impl(enc_host, 2, B, s.xyz, s.st1, s.st2, precision, eo, s.enc, s.enc_bytes, s.fpair,
-                              &xfeat, &heads_fn, reuse_pack, st));
+  return encoder_forward_impl(enc_host, 2, B, s.xyz, s.st1, s.st2, precision, eo, s.enc, s.enc_bytes, fglob_pair,
+                              nullptr, &heads_fn, reuse_pack, st);
+}
+
+// null-pointer check of every head weight
+int check_heads(const PzHeadWeights* heads_host, const char* who) {
+  const void* const* p = reinterpret_cast<const void* const*>(heads_host);
+  for (size_t i = 0; i < sizeof(PzHeadWeights) / sizeof(void*); ++i)
+    PZ_REQUIRE(p[i], PZ_ERR_ARG, "%s: head weight %zu is null", who, i);
+  return 0;
+}
+
+// pose MLP on rows of cat(ffpc, fmrpc) (model5_b.py:723-725): 2048-1024-512-512-256-6, fp32 in every precision
+int pose_mlp(const PzHeadWeights& h, const float* fpair, int n, float* h0, float* h1, float* out6, cudaStream_t st) {
+  PZ_TRY(skinny_linear(fpair, 2048, h.tf_w[0], h.tf_b[0], n, 1024, 2048, 1, h0, 1024, nullptr, 0, st));
+  PZ_TRY(skinny_linear(h0, 1024, h.tf_w[1], h.tf_b[1], n, 512, 1024, 1, h1, 512, nullptr, 0, st));
+  PZ_TRY(skinny_linear(h1, 512, h.tf_w[2], h.tf_b[2], n, 512, 512, 1, h0, 512, nullptr, 0, st));
+  PZ_TRY(skinny_linear(h0, 512, h.tf_w[3], h.tf_b[3], n, 256, 512, 1, h1, 256, nullptr, 0, st));
+  PZ_TRY(skinny_linear(h1, 256, h.tf_w[4], h.tf_b[4], n, 6, 256, 0, out6, 6, nullptr, 0, st));
+  prof_mark("pose_mlp", st);
+  return 0;
+}
+}  // namespace
+
+extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights* heads_host, const float* fpc,
+                           const float* mrpc, int B, const int64_t* starts, int precision, int flags, float* out6,
+                           float* de_fpcb, float* de_mrpcb, float* x2_fpc, float* attention_fpc, float* x2_mrpc,
+                           float* attention_mrpc, void* workspace, size_t workspace_bytes, pz_stream_t stream) {
+  PZ_REQUIRE(enc_host && heads_host && fpc && mrpc && starts && out6 && de_fpcb && de_mrpcb, PZ_ERR_ARG,
+             "pz_predict5: null pointer");
+  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "pz_predict5: B must be >= 1");
+  const int need = flags & PZ_FLAG_NEED;
+  const bool reuse_pack = (flags & PZ_FLAG_REUSE_PACKS) != 0;
+  if (need)
+    PZ_REQUIRE(x2_fpc && attention_fpc && x2_mrpc && attention_mrpc, PZ_ERR_ARG,
+               "pz_predict5: need=1 requires the x2/attention outputs");
+  PZ_TRY(check_heads(heads_host, "pz_predict5"));
+  cudaStream_t st = as_stream(stream);
+  Arena arena(workspace, workspace_bytes);
+  PredictScratch s;
+  predict_layout(B, arena, s);
+  PZ_REQUIRE(workspace && arena.ok(), PZ_ERR_WORKSPACE, "pz_predict5: workspace %zu B < required %zu B",
+             workspace_bytes, arena.used);
+  prof_begin(st);
+  PzEncoderOutputs eo = {};
+  float* x2_all = nullptr;
+  float* attn_all = nullptr;
+  // need=True: the encoder writes contiguous [2B,..] tensors but the caller's four outputs are
+  // separate, so attention [2B,256,256] and x2 [2B,256,3] go through scratch that is free until
+  // the heads run (`local`, `partial`) and are copied out per half.
+  if (need) {
+    attn_all = s.local;                                    // 2B*65536 floats == 2B*1024*64
+    x2_all = s.partial;                                    // 2B*768 floats  <= 16*B*1024
+    eo.attention = attn_all;
+    eo.x2 = x2_all;
+  }
+  const PzHeadWeights& h = *heads_host;
+  PZ_TRY(predict_front(enc_host, h, fpc, mrpc, B, starts, precision, reuse_pack, s, eo, s.fpair, s.local, s.tilemax,
+                       de_fpcb, de_mrpcb, st));
   if (need) {
     const size_t ab = (size_t)B * LATT * LATT * sizeof(float), xb = (size_t)B * S2 * 3 * sizeof(float);
     PZ_CUDA(cudaMemcpyAsync(attention_fpc, attn_all, ab, cudaMemcpyDeviceToDevice, st));
@@ -1975,14 +2024,150 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
     PZ_CUDA(cudaMemcpyAsync(x2_fpc, x2_all, xb, cudaMemcpyDeviceToDevice, st));
     PZ_CUDA(cudaMemcpyAsync(x2_mrpc, x2_all + (size_t)B * S2 * 3, xb, cudaMemcpyDeviceToDevice, st));
   }
-  // pose MLP on cat(ffpc, fmrpc): 2048-1024-512-512-256-6 (model5_b.py:723-725), fp32 in both paths
-  PZ_TRY(skinny_linear(s.fpair, 2048, h.tf_w[0], h.tf_b[0], B, 1024, 2048, 1, s.h0, 1024, s.partial, s.partial_floats, st));
-  PZ_TRY(skinny_linear(s.h0, 1024, h.tf_w[1], h.tf_b[1], B, 512, 1024, 1, s.h1, 512, s.partial, s.partial_floats, st));
-  PZ_TRY(skinny_linear(s.h1, 512, h.tf_w[2], h.tf_b[2], B, 512, 512, 1, s.h0, 512, s.partial, s.partial_floats, st));
-  PZ_TRY(skinny_linear(s.h0, 512, h.tf_w[3], h.tf_b[3], B, 256, 512, 1, s.h1, 256, s.partial, s.partial_floats, st));
-  PZ_TRY(skinny_linear(s.h1, 256, h.tf_w[4], h.tf_b[4], B, 6, 256, 0, out6, 6, s.partial, s.partial_floats, st));
-  prof_mark("pose_mlp", st);
+  return pose_mlp(h, s.fpair, B, s.h0, s.h1, out6, st);
+}
+
+// ------------------------------------------------------------- pair scoring from per-piece encodings
+namespace {
+size_t encode_layout(int P, Arena& a, PredictScratch& s, float** de_fpcb_diag) {
+  predict_layout(P, a, s);
+  *de_fpcb_diag = a.take<float>((size_t)P * 2 * NPTS);   // the fpc head of the diagonal pairs: computed, not kept
+  return a.used;
+}
+// every embedding buffer is read or written with 16-byte vector accesses
+bool embeddings_aligned(const PzPieceEmbeddings& e) {
+  return ((((uintptr_t)e.f_global | (uintptr_t)e.local | (uintptr_t)e.tilemax | (uintptr_t)e.de_mrpcb)) & 15) == 0;
+}
+struct PairScratch {
+  float *fpair, *h0, *h1, *gbias;
+  __half* himg_split;
+};
+size_t pairs_layout(int n, Arena& a, PairScratch& s) {
+  s.himg_split = a.take<__half>(2 * HEAD_SPLIT_IMG_SET);   // first: its offset does not depend on n
+  s.fpair = a.take<float>((size_t)n * 2048);
+  s.h0 = a.take<float>((size_t)n * 1024);
+  s.h1 = a.take<float>((size_t)n * 1024);
+  s.gbias = a.take<float>((size_t)n * 64);
+  return a.used;
+}
+}  // namespace
+
+namespace pz {
+namespace {
+// per pair p = (i, j): fpair[p] = [f_global[0,i], f_global[1,j]] (the pose MLP's input row) and de_out[p] = de_mrpcb[j]
+__global__ void __launch_bounds__(256) gather_pair_rows_kernel(const float4* __restrict__ fg, int P,
+                                                               const float4* __restrict__ de_mrpcb,
+                                                               const int64_t* __restrict__ pairs,
+                                                               float4* __restrict__ fpair, float4* __restrict__ de_out) {
+  pdl_enter();
+  const int p = blockIdx.x, t = threadIdx.x;   // 256 threads x 2 float4 = one 2048-float row of each output
+  const size_t i = (size_t)pairs[2 * p], j = (size_t)pairs[2 * p + 1];
+  fpair[(size_t)p * 512 + t] = fg[i * 256 + t];
+  fpair[(size_t)p * 512 + 256 + t] = fg[((size_t)P + j) * 256 + t];
+  de_out[(size_t)p * 512 + t] = de_mrpcb[j * 512 + t];
+  de_out[(size_t)p * 512 + 256 + t] = de_mrpcb[j * 512 + 256 + t];
+}
+}  // namespace
+}  // namespace pz
+
+extern "C" size_t pz_encode_pieces_workspace_bytes(int P) {
+  if (P < 1) return 0;
+  Arena a(nullptr, 0);
+  PredictScratch s;
+  float* de;
+  return align_up(encode_layout(P, a, s, &de), 256);
+}
+
+extern "C" int pz_encode_pieces(const PzEncoderWeights* enc_host, const PzHeadWeights* heads_host, const float* clouds,
+                                int P, const int64_t* starts, int precision, int flags, const PzPieceEmbeddings* emb_host,
+                                void* workspace, size_t workspace_bytes, pz_stream_t stream) {
+  PZ_REQUIRE(enc_host && heads_host && clouds && starts && emb_host, PZ_ERR_ARG, "pz_encode_pieces: null pointer");
+  const PzPieceEmbeddings& e = *emb_host;
+  PZ_REQUIRE(e.f_global && e.local && e.tilemax && e.de_mrpcb, PZ_ERR_ARG, "pz_encode_pieces: null embedding pointer");
+  PZ_REQUIRE(P >= 1, PZ_ERR_ARG, "pz_encode_pieces: P must be >= 1");
+  PZ_REQUIRE(P <= PZ_MAX_PIECES, PZ_ERR_UNSUPPORTED, "pz_encode_pieces: P = %d > %d", P, PZ_MAX_PIECES);
+  PZ_REQUIRE(embeddings_aligned(e), PZ_ERR_ARG, "pz_encode_pieces: embedding buffers must be 16-byte aligned");
+  PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
+             "pz_encode_pieces: unknown precision %d", precision);
+  PZ_REQUIRE(!(flags & PZ_FLAG_NEED), PZ_ERR_UNSUPPORTED, "pz_encode_pieces: PZ_FLAG_NEED is not supported");
+  PZ_REQUIRE(!(precision == PZ_PREC_BF16 && old_bf16_heads()), PZ_ERR_UNSUPPORTED,
+             "pz_encode_pieces: the legacy bf16 heads (PZ_HEADS_BF16=1) are not supported");
+  PZ_TRY(check_heads(heads_host, "pz_encode_pieces"));
+  cudaStream_t st = as_stream(stream);
+  Arena arena(workspace, workspace_bytes);
+  PredictScratch s;
+  float* de_fpcb_diag = nullptr;
+  encode_layout(P, arena, s, &de_fpcb_diag);
+  PZ_REQUIRE(workspace && arena.ok(), PZ_ERR_WORKSPACE, "pz_encode_pieces: workspace %zu B < required %zu B",
+             workspace_bytes, arena.used);
+  prof_begin(st);
+  PzEncoderOutputs eo = {};
+  eo.f_global = e.f_global;   // [2P,1024] == [2,P,1024]: cloud c < P is piece c through Encoder, c >= P through Encoder2
+  PZ_TRY(predict_front(enc_host, *heads_host, clouds, clouds, P, starts, precision, (flags & PZ_FLAG_REUSE_PACKS) != 0,
+                       s, eo, nullptr, e.local, e.tilemax, de_fpcb_diag, e.de_mrpcb, st));
+  if (precision == PZ_PREC_FP32) {   // the fp32 heads pool whole clouds; the embeddings keep the per-tile maxima
+    rowblock_max_kernel<<<dim3(1, 2 * P * 8), 256, 0, st>>>(e.local, 64, 128, 64, 2 * P * 8, 2 * P * 8, 0, e.tilemax, 64);
+    PZ_LAUNCH_CHECK();
+  }
   return 0;
+}
+
+extern "C" size_t pz_predict_pairs_workspace_bytes(int n) {
+  if (n < 1) return 0;
+  Arena a(nullptr, 0);
+  PairScratch s;
+  return align_up(pairs_layout(n, a, s), 256);
+}
+
+extern "C" int pz_predict_pairs(const PzHeadWeights* heads_host, const PzPieceEmbeddings* emb_host, int P,
+                                const int64_t* pairs, int n, int precision, int flags, float* out6, float* de_fpcb,
+                                float* de_mrpcb, void* workspace, size_t workspace_bytes, pz_stream_t stream) {
+  PZ_REQUIRE(n >= 0, PZ_ERR_ARG, "pz_predict_pairs: n < 0");
+  if (n == 0) return 0;
+  PZ_REQUIRE(heads_host && emb_host && pairs && out6 && de_fpcb && de_mrpcb, PZ_ERR_ARG, "pz_predict_pairs: null pointer");
+  const PzPieceEmbeddings& e = *emb_host;
+  PZ_REQUIRE(e.f_global && e.local && e.tilemax && e.de_mrpcb, PZ_ERR_ARG, "pz_predict_pairs: null embedding pointer");
+  PZ_REQUIRE(P >= 1, PZ_ERR_ARG, "pz_predict_pairs: P must be >= 1");
+  PZ_REQUIRE(n <= PZ_MAX_PAIRS, PZ_ERR_UNSUPPORTED, "pz_predict_pairs: n = %d > %d", n, PZ_MAX_PAIRS);
+  PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
+             "pz_predict_pairs: unknown precision %d", precision);
+  PZ_REQUIRE(!(flags & PZ_FLAG_NEED), PZ_ERR_UNSUPPORTED, "pz_predict_pairs: PZ_FLAG_NEED is not supported");
+  PZ_REQUIRE(!(precision == PZ_PREC_BF16 && old_bf16_heads()), PZ_ERR_UNSUPPORTED,
+             "pz_predict_pairs: the legacy bf16 heads (PZ_HEADS_BF16=1) are not supported");
+  PZ_TRY(check_heads(heads_host, "pz_predict_pairs"));
+  PZ_REQUIRE(embeddings_aligned(e) && ((uintptr_t)de_mrpcb & 15) == 0, PZ_ERR_ARG,
+             "pz_predict_pairs: embedding buffers and de_mrpcb must be 16-byte aligned");
+  cudaStream_t st = as_stream(stream);
+  Arena arena(workspace, workspace_bytes);
+  PairScratch s;
+  pairs_layout(n, arena, s);
+  PZ_REQUIRE(workspace && arena.ok(), PZ_ERR_WORKSPACE, "pz_predict_pairs: workspace %zu B < required %zu B",
+             workspace_bytes, arena.used);
+  prof_begin(st);
+  const PzHeadWeights& h = *heads_host;
+  const Mlp3W pre_f = {h.pre_fpc_w[0], h.pre_fpc_b[0], h.pre_fpc_w[1], h.pre_fpc_b[1], h.pre_fpc_w[2], h.pre_fpc_b[2]};
+  const Mlp3W pre_r = {h.pre_rpc_w[0], h.pre_rpc_b[0], h.pre_rpc_w[1], h.pre_rpc_b[1], h.pre_rpc_w[2], h.pre_rpc_b[2]};
+  const Mlp3W seg_f = {h.seg_fpc_w[0], h.seg_fpc_b[0], h.seg_fpc_w[1], h.seg_fpc_b[1], h.seg_fpc_w[2], h.seg_fpc_b[2]};
+  const Mlp3W seg_r = {h.seg_rpc_w[0], h.seg_rpc_b[0], h.seg_rpc_w[1], h.seg_rpc_b[1], h.seg_rpc_w[2], h.seg_rpc_b[2]};
+  const float* tilemax_mrpc = e.tilemax + (size_t)P * 8 * 64;
+  PZ_CUDA(launch_pdl(gather_pair_rows_kernel, dim3(n), dim3(256), 0, st, reinterpret_cast<const float4*>(e.f_global), P,
+                     reinterpret_cast<const float4*>(e.de_mrpcb), pairs, reinterpret_cast<float4*>(s.fpair),
+                     reinterpret_cast<float4*>(de_mrpcb)));
+  PZ_LAUNCH_CHECK();
+  prof_mark("gather_pairs", st);
+  if (precision == PZ_PREC_FP32) {
+    PZ_TRY(set_head_fp32_smem());
+    seg_bias_kernel<<<dim3(n, 1), 64, 0, st>>>(tilemax_mrpc, 8, pairs, h.seg_fpc_w[0], h.seg_fpc_b[0], h.seg_rpc_w[0],
+                                               h.seg_rpc_b[0], n, s.gbias);
+    PZ_LAUNCH_CHECK();
+    head_seg_kernel<<<n * NPTS / 128, 128, HS_SMEM, st>>>(e.local, seg_f, seg_r, s.gbias, n, de_fpcb, nullptr, pairs);
+    PZ_LAUNCH_CHECK();
+  } else {
+    PZ_TRY(launch_seg_pairs_split(pre_f, pre_r, seg_f, seg_r, (flags & PZ_FLAG_REUSE_PACKS) != 0, s.himg_split, e.local,
+                                  tilemax_mrpc, pairs, n, de_fpcb, st));
+  }
+  prof_mark("boundary_heads", st);
+  return pose_mlp(h, s.fpair, n, s.h0, s.h1, out6, st);
 }
 
 extern "C" int pz_se3_exp(const float* twist, int B, float* g, pz_stream_t stream) {

@@ -200,10 +200,13 @@ __global__ void __launch_bounds__(128) head_pre_split_kernel(const float* __rest
 // MLP{Fpcb,Rpcb} (model5_b.py:745-754): relu(W0 [g ; local] + b0) -> relu(W1 . + b1) -> W2 . + b2, logits as [B,2,1024].
 // g = the MRPC cloud's global max for BOTH heads (D6); its half of layer 0 is a per-cloud bias computed in the prologue
 // (fp32 FMAs); the last layer (32 -> 2) runs on the fp32 fragments.
+// pairs == null: cloud c of the 2B (set = c / B, b = c % B) reads local[c] and the tile maxima of cloud B + b, and writes
+// row b of de_a / de_b.  pairs [B,2]: every cloud is a pair of set 0: pair b reads local[pairs[b,0]] and the tile maxima
+// of row pairs[b,1], and writes row b of de_a.
 __global__ void __launch_bounds__(128) head_seg_split_kernel(const float* __restrict__ local, HeadMlp3 wa, HeadMlp3 wb,
                                                              const __half* __restrict__ img, int B, int reps,
                                                              const float* __restrict__ tilemax, float* __restrict__ de_a,
-                                                             float* __restrict__ de_b) {
+                                                             float* __restrict__ de_b, const int64_t* __restrict__ pairs) {
   __shared__ __align__(16) __half wseg[2 * SEG_ROWS * HS_WS];   // [hi: W0 local 64 rows, W1 32 rows][lo: same]
   __shared__ float gs[64], gb[64], b1s[32], w2s[64], b2s[2];
   const __half *w0h = wseg, *w1h = wseg + 64 * HS_WS, *w0l = wseg + SEG_ROWS * HS_WS, *w1l = w0l + 64 * HS_WS;
@@ -216,8 +219,9 @@ __global__ void __launch_bounds__(128) head_seg_split_kernel(const float* __rest
     uint4* dst = reinterpret_cast<uint4*>(wseg);
     for (int i = tid; i < 2 * SEG_ROWS * HS_WS / 8; i += 128) dst[i] = src[i];
   }
+  const size_t src = pairs ? (size_t)pairs[2 * b] : (size_t)cloud;   // cloud of the local features
   if (tid < 64) {
-    const float* tm = tilemax + ((size_t)(B + b) * 8) * 64 + tid;   // the mrpc cloud of pair b
+    const float* tm = tilemax + ((size_t)(pairs ? pairs[2 * b + 1] : B + b) * 8) * 64 + tid;   // the mrpc cloud of pair b
     float m = tm[0];
 #pragma unroll
     for (int i = 1; i < 8; ++i) m = fmaxf(m, tm[i * 64]);
@@ -239,7 +243,7 @@ __global__ void __launch_bounds__(128) head_seg_split_kernel(const float* __rest
     const size_t p0 = ((size_t)blockIdx.x * reps + rep) * 128 + warp * 32;
     const int n0 = (int)(p0 - (size_t)cloud * NPTS_H);
     Frags a;
-    load_frags(local + p0 * 64, g, q, a);
+    load_frags(local + (src * NPTS_H + n0) * 64, g, q, a);
     float acc[2][8][4];
     zero<8>(acc);
     layer<8>(a, w0h, w0l, g, q, acc);
@@ -287,18 +291,25 @@ __global__ void __launch_bounds__(128) head_seg_split_kernel(const float* __rest
 
 }  // namespace
 
+// fp16 plane images of both heads' weights (img: 2 * HEAD_SPLIT_IMG_SET halves), skipped when the caller vouches for them
+static int build_images(const HeadMlp3& pre_f, const HeadMlp3& pre_r, const HeadMlp3& seg_f, const HeadMlp3& seg_r,
+                        bool reuse_images, __half* img, cudaStream_t st) {
+  if (!reuse_images) {
+    head_images_kernel<<<dim3(8, 2), 256, 0, st>>>(pre_f, pre_r, seg_f, seg_r, img);
+    PZ_LAUNCH_CHECK();
+  }
+  return 0;
+}
+
 // boundary heads of predict5 for 2B clouds (clouds [0,B) = fpc -> *_fpc weights and de_fpcb, [B,2B) = mrpc):
-// xfeat [2B*1024, 64] fp32 -> de_fpcb / de_mrpcb [B,2,1024].  local [2B*1024, 64] fp32 and tilemax [2B*8*64] are scratch,
-// img (2 * HEAD_SPLIT_IMG_SET halves) holds the weight images: rebuilt unless reuse_images.
+// xfeat [2B*1024, 64] fp32 -> de_fpcb / de_mrpcb [B,2,1024].  local [2B*1024, 64] fp32 and tilemax [2B*8*64] receive the
+// per-cloud state, img (2 * HEAD_SPLIT_IMG_SET halves) holds the weight images: rebuilt unless reuse_images.
 int launch_heads_split(const float* xfeat, const HeadMlp3& pre_f, const HeadMlp3& pre_r, const HeadMlp3& seg_f,
                        const HeadMlp3& seg_r, int B, bool reuse_images, void* img, float* local, float* tilemax,
                        float* de_fpcb, float* de_mrpcb, cudaStream_t st) {
   PZ_REQUIRE(xfeat && img && local && tilemax && de_fpcb && de_mrpcb, PZ_ERR_ARG, "heads_split: null pointer");
   __half* im = static_cast<__half*>(img);
-  if (!reuse_images) {
-    head_images_kernel<<<dim3(8, 2), 256, 0, st>>>(pre_f, pre_r, seg_f, seg_r, im);
-    PZ_LAUNCH_CHECK();
-  }
+  PZ_TRY(build_images(pre_f, pre_r, seg_f, seg_r, reuse_images, im, st));
   const int P = 2 * B * NPTS_H, reps = 4;
   const size_t pre_smem = (size_t)2 * PRE_ROWS * HS_WS * sizeof(__half) + (3 * 64 + 4 * 64) * sizeof(float);
   PZ_CUDA(cudaFuncSetAttribute(head_pre_split_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pre_smem));
@@ -306,7 +317,22 @@ int launch_heads_split(const float* xfeat, const HeadMlp3& pre_f, const HeadMlp3
                      local, tilemax));
   PZ_LAUNCH_CHECK();
   PZ_CUDA(launch_pdl(head_seg_split_kernel, dim3(P / (128 * reps)), dim3(128), 0, st, (const float*)local, seg_f, seg_r, (const __half*)im, B,
-                     reps, (const float*)tilemax, de_fpcb, de_mrpcb));
+                     reps, (const float*)tilemax, de_fpcb, de_mrpcb, (const int64_t*)nullptr));
+  PZ_LAUNCH_CHECK();
+  return 0;
+}
+
+// the fpc boundary head of n pairs from per-piece state (pz_predict_pairs): pair p reads local_fpc[pairs[p,0]]
+// ([P*1024, 64]) and the tile maxima tilemax_mrpc[pairs[p,1]] ([P*8*64]) and writes de_fpcb[p] ([n,2,1024])
+int launch_seg_pairs_split(const HeadMlp3& pre_f, const HeadMlp3& pre_r, const HeadMlp3& seg_f, const HeadMlp3& seg_r,
+                           bool reuse_images, void* img, const float* local_fpc, const float* tilemax_mrpc,
+                           const int64_t* pairs, int n, float* de_fpcb, cudaStream_t st) {
+  PZ_REQUIRE(img && local_fpc && tilemax_mrpc && pairs && de_fpcb, PZ_ERR_ARG, "heads_split: null pointer");
+  __half* im = static_cast<__half*>(img);
+  PZ_TRY(build_images(pre_f, pre_r, seg_f, seg_r, reuse_images, im, st));
+  const int reps = 4;   // 8 tiles per pair: every CTA stays inside one pair
+  PZ_CUDA(launch_pdl(head_seg_split_kernel, dim3(n * NPTS_H / (128 * reps)), dim3(128), 0, st, local_fpc, seg_f, seg_f,
+                     (const __half*)im, n, reps, tilemax_mrpc, de_fpcb, (float*)nullptr, pairs));
   PZ_LAUNCH_CHECK();
   return 0;
 }

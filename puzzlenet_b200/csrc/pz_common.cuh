@@ -243,6 +243,9 @@ constexpr size_t HEAD_SPLIT_IMG_SET = (size_t)(2 * 3 * 64 + 2 * (64 + 32)) * 72;
 int launch_heads_split(const float* xfeat, const HeadMlp3& pre_f, const HeadMlp3& pre_r, const HeadMlp3& seg_f,
                        const HeadMlp3& seg_r, int B, bool reuse_images, void* img, float* local, float* tilemax,
                        float* de_fpcb, float* de_mrpcb, cudaStream_t st);
+int launch_seg_pairs_split(const HeadMlp3& pre_f, const HeadMlp3& pre_r, const HeadMlp3& seg_f, const HeadMlp3& seg_r,
+                           bool reuse_images, void* img, const float* local_fpc, const float* tilemax_mrpc,
+                           const int64_t* pairs, int n, float* de_fpcb, cudaStream_t st);
 int launch_tc_rowgemm(const TcGemm& g, cudaStream_t st);   // gemm_tc_rows.cu: same struct, row-major store epilogue
 // attention_tc.cu: per cloud  r = x - softmax(q k^T / sqrt(64)) v   on tcgen05 (L == 256, d_k == 64, C == 256)
 int launch_attention_tc(const __nv_bfloat16* qk, const __nv_bfloat16* vT, const __nv_bfloat16* x, int ldx, int clouds,

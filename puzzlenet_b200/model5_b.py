@@ -226,6 +226,103 @@ def _seq(*sizes):
     return nn.Sequential(*layers)
 
 
+def _draw_starts(B: int) -> torch.Tensor:
+    """predict5's four FPS-start draws on the CPU generator, in the reference's order -> int64 [4,B]."""
+    return torch.stack([torch.randint(0, 1024, (B,), dtype=torch.long),
+                        torch.randint(0, 512, (B,), dtype=torch.long),
+                        torch.randint(0, 1024, (B,), dtype=torch.long),
+                        torch.randint(0, 512, (B,), dtype=torch.long)])
+
+
+def _pieces_arg(clouds) -> torch.Tensor:
+    _lib.require_cuda(clouds)
+    clouds = clouds.contiguous().float()
+    if clouds.dim() != 3 or clouds.shape[0] < 1 or clouds.shape[1:] != (1024, 3):
+        raise ValueError(f"expected pieces [P,1024,3] with P >= 1; got {tuple(clouds.shape)}")
+    return clouds
+
+
+ENCODE_CHUNK = 64     # pieces per pz_encode_pieces call: bounds the workspace (that of predict5 with B = 64)
+PAIR_CHUNK = 4096     # pairs per pz_predict_pairs call: bounds its workspace (~70 MB)
+
+
+class PieceEmbeddings:
+    """Per-piece state of :meth:`TouchedRegraster.encode_pieces` (layout: ``PzPieceEmbeddings`` in
+    include/puzzlenet_b200.h): ``f_global [2,P,1024]``, ``local [2,P,1024,64]``, ``tilemax [2,P,8,64]`` (role 0 = the
+    piece as fpc, role 1 = as mrpc), ``de_mrpcb [P,2,1024]``, plus the FPS ``starts [4,P]`` (CPU) they were encoded
+    with, the precision, the device and the model's weights key (``TouchedRegraster._weights_key``) at encode time."""
+
+    def __init__(self, P: int, device, starts, precision: str, param_key):
+        starts = torch.as_tensor(starts)
+        if starts.shape != (4, P):
+            raise ValueError(f"starts must be [4,{P}]; got {tuple(starts.shape)}")
+        f32 = dict(device=device, dtype=torch.float32)
+        self.f_global = torch.empty(2, P, 1024, **f32)
+        self.local = torch.empty(2, P, 1024, 64, **f32)
+        self.tilemax = torch.empty(2, P, 8, 64, **f32)
+        self.de_mrpcb = torch.empty(P, 2, 1024, **f32)
+        self.starts = starts.to("cpu", torch.int64).clone()
+        self.precision = precision
+        self.device = torch.device(device)
+        self.param_key = param_key
+
+    @property
+    def P(self) -> int:
+        return self.de_mrpcb.shape[0]
+
+    def struct(self) -> _lib.PzPieceEmbeddings:
+        return _lib.PzPieceEmbeddings(self.f_global.data_ptr(), self.local.data_ptr(), self.tilemax.data_ptr(),
+                                      self.de_mrpcb.data_ptr())
+
+    def is_current(self, model) -> bool:
+        """False once the model's parameters or precision changed after these embeddings were encoded."""
+        return model.precision == self.precision and model._weights_key() == self.param_key
+
+    def _check_current(self, model):
+        if not self.is_current(model):
+            raise ValueError("these piece embeddings are stale: the model's parameters or precision changed since "
+                             "they were encoded (encode the pieces again)")
+
+    def reencode(self, model, rows, clouds, starts=None) -> None:
+        """Encode ``clouds [k,1024,3]`` again as pieces ``rows`` (k indices in ``[0,P)``), in place; ``starts [4,k]``
+        default to predict5's draws for ``B = k``.  The model must be the one the embeddings were built with."""
+        self._check_current(model)
+        rows = [int(r) for r in rows]
+        if any(r < 0 or r >= self.P for r in rows):
+            raise IndexError(f"reencode: piece index outside [0, {self.P})")
+        clouds = _pieces_arg(clouds)
+        if clouds.shape[0] != len(rows):
+            raise ValueError("reencode: one cloud per row")
+        starts = _draw_starts(len(rows)) if starts is None else torch.as_tensor(starts).to(torch.int64)
+        self.starts[:, rows] = starts
+        self._encode(model, clouds, starts.to(self.device, non_blocking=True), rows)
+
+    def _encode(self, model, clouds, starts, rows):
+        """pz_encode_pieces over ``clouds`` (device starts [4,k]) into pieces ``rows``, ENCODE_CHUNK pieces a call;
+        a call that covers every piece in order writes straight into the tensors, others go through a chunk buffer."""
+        for m in (model.Encoder, model.Encoder2, model.tfMLP, model.fpc_decoder, model.rpc_decoder):
+            m.eval()
+        enc = (_lib.PzEncoderWeights * 2)(_encoder_struct(model.Encoder), _encoder_struct(model.Encoder2))
+        heads = model._head_struct()
+        for lo in range(0, len(rows), ENCODE_CHUNK):
+            sel = rows[lo:lo + ENCODE_CHUNK]
+            k = len(sel)
+            direct = sel == list(range(self.P))
+            dst = self if direct else PieceEmbeddings(k, self.device, self.starts[:, sel], self.precision, self.param_key)
+            ws = model._workspace(k, self.device, "pz_encode_pieces")
+            flags = _lib.PZ_FLAG_REUSE_PACKS if model._packs_reusable(ws) else 0
+            with torch.cuda.device(self.device):
+                _lib.call("pz_encode_pieces", enc, ctypes.byref(heads), clouds[lo:lo + k].data_ptr(), k,
+                          starts[:, lo:lo + k].contiguous().data_ptr(), PRECISIONS[self.precision], flags,
+                          ctypes.byref(dst.struct()), ws.buf.data_ptr(), ws.buf.numel(), _lib.stream_ptr())
+            if not direct:
+                idx = torch.tensor(sel, device=self.device)
+                self.f_global[:, idx] = dst.f_global
+                self.local[:, idx] = dst.local
+                self.tilemax[:, idx] = dst.tilemax
+                self.de_mrpcb[idx] = dst.de_mrpcb
+
+
 class TouchedRegraster(_Base):
     """model5_b.py:519-759.  ``predict5(batch, batch_indic, need=False, training=False)`` is the forward
     that train/test execute; ``batch`` is the 8-tuple ``(fpc, mrpc, igt, rpc, fpcb, mrpcb, fpc_idx, rpc_idx)``
@@ -254,6 +351,7 @@ class TouchedRegraster(_Base):
         self._graphs = {}
         self._capture_stream = None
         self._trainer_state = None
+        self._weights_generation = 0  # bumped whenever the weights change behind torch's back (see _weights_key)
         self.cuda_graphs = False      # opt-in: replay one captured CUDA graph per forward (see _graph_replay)
         self.graph_static_outputs = False   # True: return the graph's own output buffers (overwritten by the next replay)
         self.max_graphs = 16          # captured graphs kept (one per batch size, need, precision, device, stream); LRU
@@ -271,25 +369,44 @@ class TouchedRegraster(_Base):
                 getattr(h, f"{field}_b")[j] = _param(mod[li].bias).data_ptr()
         return h
 
-    def _workspace(self, B: int, device) -> "_Workspace":
-        """One workspace per (batch size, device, CUDA stream): calls issued on different streams may overlap on
-        the GPU (a pipelined caller alternates streams), so they must not share scratch.  At most four are kept.
-        The validity of the bf16 / split weight packs stored inside a workspace is a property of the workspace OBJECT
-        (``_Workspace.pack_key``), never of its address: an evicted workspace takes its key with it, so a block the
-        caching allocator hands to a workspace of another batch size (other pack offset) can never be taken for a
-        packed one."""
-        key = (B, str(device), torch.cuda.current_stream(device).cuda_stream)
+    def _workspace(self, B: int, device, kind: str = "pz_predict5") -> "_Workspace":
+        """One workspace per (entry point, batch size, device, CUDA stream): calls issued on different streams may
+        overlap on the GPU (a pipelined caller alternates streams), so they must not share scratch.  At most four are
+        kept per entry point.  The validity of the bf16 / split weight packs stored inside a workspace is a property
+        of the workspace OBJECT (``_Workspace.pack_key``), never of its address: an evicted workspace takes its key
+        with it, so a block the caching allocator hands to a workspace of another batch size (other pack offset) can
+        never be taken for a packed one."""
+        key = (kind, B, str(device), torch.cuda.current_stream(device).cuda_stream)
         ws = self._ws.get(key)
         if ws is None:
-            nbytes = _lib.load().pz_predict5_workspace_bytes(B)
+            nbytes = getattr(_lib.load(), kind + "_workspace_bytes")(B)
             ws = _Workspace(torch.empty(nbytes, device=device, dtype=torch.uint8))
-            if len(self._ws) >= 4:
-                self._ws.pop(next(iter(self._ws)))
+            same = [k for k in self._ws if k[0] == kind]
+            if len(same) >= 4:
+                self._ws.pop(same[0])
             self._ws[key] = ws
         return ws
 
     def _param_key(self):
         return tuple((p.data_ptr(), p._version) for p in self.parameters())
+
+    def _weights_key(self):
+        """Identifies the weights state that piece embeddings were computed from: ``_param_key`` misses writes that
+        bypass torch (the Trainer's Adam step, parameter broadcasts, train-mode BatchNorm statistics), so those bump
+        ``_weights_generation`` (``Trainer._invalidate_inference_state``)."""
+        return self._param_key(), self._weights_generation
+
+    def _packs_reusable(self, ws: "_Workspace", shared: bool = False) -> bool:
+        """Whether the weight packs inside ``ws`` are still valid, and record that they will be after this call: they
+        are reusable while no parameter was touched (in-place writes bump _version, reallocation changes data_ptr) and
+        the workspace object / precision are the same."""
+        if self.precision not in PACKED_PRECISIONS:
+            ws.pack_key = None
+            return False
+        key = (self._param_key(), shared, self.precision)
+        reuse = ws.pack_key == key
+        ws.pack_key = key
+        return reuse
 
     def _launch(self, fpc, mrpc, starts, need, ws, outs, reuse_packs=None, shared=False):
         """Allocate (unless given) the outputs and the workspace and enqueue pz_predict5 on the current stream.
@@ -310,14 +427,9 @@ class TouchedRegraster(_Base):
         if ws is None:
             ws = self._workspace(B, dev)
         flags = _lib.PZ_FLAG_NEED if need else 0
-        packed = self.precision in PACKED_PRECISIONS
-        if reuse_packs is None and packed:
-            # the weight packs live in the workspace: reusable while no parameter was touched (in-place writes
-            # bump _version, reallocation changes data_ptr) and the workspace object / precision are the same
-            key = (self._param_key(), shared, self.precision)
-            reuse_packs = ws.pack_key == key
-            ws.pack_key = key
-        elif not packed:
+        if reuse_packs is None:
+            reuse_packs = self._packs_reusable(ws, shared)
+        elif self.precision not in PACKED_PRECISIONS:
             ws.pack_key = None
         if reuse_packs:
             flags |= _lib.PZ_FLAG_REUSE_PACKS
@@ -409,6 +521,56 @@ class TouchedRegraster(_Base):
             return r[0]
         return r[0], [0], r[2], r[3], r[4], r[5]
 
+    # ---- pair scoring from per-piece encodings (not in the reference): predict5 split at its pair boundary
+    def encode_pieces(self, clouds, starts=None) -> "PieceEmbeddings":
+        """Everything ``predict5`` computes per cloud, once per piece: both encoders, ``MLPLocalPre{Fpc,Rpc}`` and the
+        mrpc boundary head (``pz_encode_pieces``).  ``clouds [P,1024,3]`` on the GPU; ``starts`` int64 [4,P] FPS starts
+        in predict5's order (Encoder s1, Encoder s2, Encoder2 s1, Encoder2 s2) -- when omitted they are drawn exactly
+        as ``predict5`` with ``B = P`` draws them, so ``encode_pieces(c)`` consumes the same random numbers as
+        ``predict5(make_batch(c, c), P)``.  Eval mode only; pieces are encoded in chunks of at most
+        ``ENCODE_CHUNK``."""
+        clouds = _pieces_arg(clouds)
+        P, dev = clouds.shape[0], clouds.device
+        starts = _draw_starts(P) if starts is None else starts
+        emb = PieceEmbeddings(P, dev, starts, self.precision, self._weights_key())
+        emb._encode(self, clouds, emb.starts.to(dev, non_blocking=True), list(range(P)))
+        return emb
+
+    def predict_pairs(self, emb: "PieceEmbeddings", pairs):
+        """``(out6, out6, de_fpcb, de_mrpcb)`` -- what ``predict5(need=False)`` returns for the pairs
+        ``(clouds[i], clouds[j])`` of ``pairs [n,2]`` (i = fpc piece, j = mrpc piece) with the pieces' FPS starts, from
+        the embeddings of :meth:`encode_pieces` (``pz_predict_pairs``: the pose MLP and the fpc boundary head only).
+        Raises ``IndexError`` for an index outside ``[0,P)`` and ``ValueError`` when the parameters or the precision
+        changed since ``emb`` was built."""
+        emb._check_current(self)
+        pairs = torch.as_tensor(pairs)
+        if pairs.dim() != 2 or pairs.shape[1] != 2 or pairs.dtype.is_floating_point:
+            raise ValueError(f"predict_pairs expects integer pairs [n,2]; got {pairs.dtype} {tuple(pairs.shape)}")
+        n = pairs.shape[0]
+        if n:
+            lo, hi = (int(v) for v in torch.aminmax(pairs))       # one host synchronisation for device pairs
+            if lo < 0 or hi >= emb.P:
+                raise IndexError(f"predict_pairs: piece index {lo if lo < 0 else hi} outside [0, {emb.P})")
+        pairs = pairs.to(device=emb.device, dtype=torch.int64, non_blocking=True).contiguous()
+        f32 = dict(device=emb.device, dtype=torch.float32)
+        out6, de_fpcb, de_mrpcb = torch.empty(n, 6, **f32), torch.empty(n, 2, 1024, **f32), torch.empty(n, 2, 1024, **f32)
+        for lo in range(0, n, PAIR_CHUNK):
+            hi = min(n, lo + PAIR_CHUNK)
+            self._launch_pairs(emb, pairs[lo:hi], out6[lo:hi], de_fpcb[lo:hi], de_mrpcb[lo:hi])
+        return out6, out6, de_fpcb, de_mrpcb
+
+    def _launch_pairs(self, emb, pairs, out6, de_fpcb, de_mrpcb):
+        """Enqueue pz_predict_pairs on the current stream (no checks: ``pairs`` int64 [n,2] on emb's device, in range);
+        CUDA-graph capturable once the workspace's weight images are built."""
+        n = pairs.shape[0]
+        ws = self._workspace(max(64, 1 << (n - 1).bit_length()), emb.device, "pz_predict_pairs")
+        flags = _lib.PZ_FLAG_REUSE_PACKS if self._packs_reusable(ws) else 0
+        heads = self._head_struct()
+        with torch.cuda.device(emb.device):
+            _lib.call("pz_predict_pairs", ctypes.byref(heads), ctypes.byref(emb.struct()), emb.P, pairs.data_ptr(), n,
+                      PRECISIONS[self.precision], flags, out6.data_ptr(), de_fpcb.data_ptr(), de_mrpcb.data_ptr(),
+                      ws.buf.data_ptr(), ws.buf.numel(), _lib.stream_ptr())
+
     def _predict(self, batch, need, starts, shared):
         for m in (self.Encoder, self.Encoder2, self.tfMLP, self.fpc_decoder, self.rpc_decoder):
             m.eval()                                              # model5_b.py:677-683
@@ -422,10 +584,7 @@ class TouchedRegraster(_Base):
             raise ValueError(f"predict5 expects two [B,1024,3] clouds; got {tuple(fpc.shape)} and {tuple(mrpc.shape)}")
         B, dev = fpc.shape[0], fpc.device
         if starts is None:
-            starts = torch.stack([torch.randint(0, 1024, (B,), dtype=torch.long),
-                                  torch.randint(0, 512, (B,), dtype=torch.long),
-                                  torch.randint(0, 1024, (B,), dtype=torch.long),
-                                  torch.randint(0, 512, (B,), dtype=torch.long)])
+            starts = _draw_starts(B)
         starts = starts.to(device=dev, dtype=torch.int64, non_blocking=True).contiguous()
         if self.cuda_graphs:
             out6, de_fpcb, de_mrpcb, x2f, af, x2m, am = self._graph_replay(fpc, mrpc, starts, need, shared)

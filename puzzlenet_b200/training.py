@@ -229,10 +229,12 @@ class Trainer:
 
     def _invalidate_inference_state(self):
         """Parameters were written behind torch's back (no _version bump): drop what the inference path derived from
-        them -- the weight packs inside its workspaces and the captured CUDA graphs."""
+        them -- the weight packs inside its workspaces and the captured CUDA graphs -- and mark piece embeddings
+        encoded before now as stale."""
         for ws in getattr(self.model, "_ws", {}).values():
             ws.pack_key = None
         getattr(self.model, "_graphs", {}).clear()
+        self.model._weights_generation = getattr(self.model, "_weights_generation", 0) + 1
 
     # -------------------------------------------------------------------------------------------- scratch
     def buf(self, name, *shape, dtype=torch.float32):
@@ -511,6 +513,7 @@ class Trainer:
                 res += [e.x2.clone(), att]
         de_f = fw["logit_f"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
         de_m = fw["logit_m"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
+        self._invalidate_inference_state()            # the BatchNorm running statistics were updated in place
         return fw["out6"].clone(), [0], res[0], res[1], res[2], res[3], de_f, de_m
 
     def _pose_losses(self, out6, mrpc, rpc, igt, B):
