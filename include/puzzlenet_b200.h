@@ -259,8 +259,7 @@ typedef struct PzPieceEmbeddings {
  * clouds and starts, the embeddings of piece p are those pz_predict5(fpc = mrpc = clouds) forms for pair p.
  * flags: PZ_FLAG_REUSE_PACKS as in pz_predict5 (PZ_FLAG_NEED is not supported).  Supported: 1 <= P <= PZ_MAX_PIECES
  * (encode larger sets in several calls), precision
- * fp32 / bf16 / split; the legacy bf16 heads selected by the environment variable PZ_HEADS_BF16=1 are not supported
- * (PZ_ERR_UNSUPPORTED). */
+ * fp32 / bf16 / split. */
 size_t pz_encode_pieces_workspace_bytes(int P);
 int pz_encode_pieces(const PzEncoderWeights* enc_host /*[2]*/, const PzHeadWeights* heads_host, const float* clouds,
                      int P, const int64_t* starts, int precision, int flags, const PzPieceEmbeddings* emb_host,

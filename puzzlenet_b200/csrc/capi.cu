@@ -65,14 +65,8 @@ void prof_mark(const char* stage, cudaStream_t st, int lane) {
 }
 
 bool prof_serial() { return g_prof_serial; }
-bool pdl_enabled() {
-  static const bool on = getenv("PZ_NO_PDL") == nullptr;
-  return on;
-}
 bool pdl_for_stream(cudaStream_t st) {
-  static const bool in_graphs = getenv("PZ_PDL_IN_GRAPHS") != nullptr;   // A/B hook
-  if (!pdl_enabled() || g_prof_on) return false;
-  if (in_graphs) return true;
+  if (g_prof_on) return false;
   cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(st, &cs) != cudaSuccess) {
     cudaGetLastError();

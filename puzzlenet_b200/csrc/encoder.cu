@@ -5,7 +5,6 @@
 // Both encoders of predict5 run as ONE batch of 2B clouds (cloud c uses weight set c / B), so
 // every launch covers 128 clouds at B=64 instead of 64 -- FPS, the latency-bound stage, then
 // occupies 128 of the 148 SMs.
-#include <stdlib.h>
 
 #include <functional>
 
@@ -27,9 +26,7 @@ struct StemW {
 };
 
 __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ xyz, StemW wa, StemW wb,
-                                                   int clouds_per_set, float* __restrict__ out,
-                                                   __nv_bfloat16* __restrict__ out_b, __half* __restrict__ out_hi,
-                                                   __half* __restrict__ out_lo) {
+                                                   int clouds_per_set, float* __restrict__ out) {
   __shared__ __align__(16) float w2s[64 * 64];
   __shared__ float w1s[64 * 3], b1s[64], b2s[64];
   const size_t p = (size_t)blockIdx.x * 128 + threadIdx.x;  // global point id
@@ -77,21 +74,6 @@ __global__ void __launch_bounds__(128) stem_kernel(const float* __restrict__ xyz
       r[u] = fmaxf(fmaf(v, a2, c2), 0.f);
     }
     *reinterpret_cast<float4*>(o + k0) = make_float4(r[0], r[1], r[2], r[3]);
-    if (out_b) {
-      __nv_bfloat162 lo = __floats2bfloat162_rn(r[0], r[1]), hi = __floats2bfloat162_rn(r[2], r[3]);
-      uint2 pk = make_uint2(*reinterpret_cast<uint32_t*>(&lo), *reinterpret_cast<uint32_t*>(&hi));
-      *reinterpret_cast<uint2*>(out_b + p * 64 + k0) = pk;
-    }
-    if (out_hi) {   // split path: the fp16 hi / lo planes of x_feature, straight from the registers
-      uint2 ph, pl;
-      const __half2 h0 = __floats2half2_rn(r[0], r[1]), h1 = __floats2half2_rn(r[2], r[3]);
-      const float2 f0 = __half22float2(h0), f1 = __half22float2(h1);
-      const __half2 l0 = __floats2half2_rn(r[0] - f0.x, r[1] - f0.y), l1 = __floats2half2_rn(r[2] - f1.x, r[3] - f1.y);
-      ph.x = *reinterpret_cast<const uint32_t*>(&h0); ph.y = *reinterpret_cast<const uint32_t*>(&h1);
-      pl.x = *reinterpret_cast<const uint32_t*>(&l0); pl.y = *reinterpret_cast<const uint32_t*>(&l1);
-      *reinterpret_cast<uint2*>(out_hi + p * 64 + k0) = ph;
-      *reinterpret_cast<uint2*>(out_lo + p * 64 + k0) = pl;
-    }
   }
 }
 
@@ -107,16 +89,8 @@ __device__ __forceinline__ void stem_mma_f16(float (&d)[4], const uint32_t (&a)[
                : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
                : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
-// 128-point tiles per CTA of the stem / boundary-head kernels (the tiles of one CTA belong to one cloud: reps | 8)
+// 128-point tiles per CTA of stem_tc_kernel (the tiles of one CTA belong to one cloud: reps | 8)
 constexpr int HD_REPS = 4;
-static int head_reps() {
-  static const int r = [] {
-    const char* e = getenv("PZ_HD_REPS");   // tuning hook
-    const int v = e ? atoi(e) : HD_REPS;
-    return (v == 1 || v == 2 || v == 4 || v == 8) ? v : HD_REPS;
-  }();
-  return r;
-}
 constexpr int STEM_WS = 72;
 constexpr size_t STEM_TC_SMEM = 4 * 32 * STEM_WS * sizeof(float) + 64 * sizeof(float4) + 64 * sizeof(float) +
                                 2 * 64 * STEM_WS * sizeof(__nv_bfloat16);
@@ -749,263 +723,6 @@ __global__ void __launch_bounds__(128) head_seg_kernel(const float* __restrict__
   de[((size_t)b * 2 + 1) * NPTS + n] = o1;
 }
 
-// ---- bf16 path, boundary heads as two chained-MMA kernels (mma.sync m16n8k16; the accumulator fragments of one layer,
-// rounded to bf16, ARE the A fragments of the next, so activations never leave registers).  One warp = 32 points.
-constexpr int HD_WS = 72;   // padded bf16 row stride: conflict-free fragment loads
-// packed head weights of one set (bf16, rows of HD_WS): pre.w0, pre.w1, pre.w2 [64 rows each], seg.w0[:, 64:128] [64],
-// seg.w1 hi [32], seg.w1 lo [32]
-constexpr size_t HEAD_IMG_SET = (size_t)(3 * 64 + 64 + 32 + 32) * HD_WS;
-
-// 32-point tile (contiguous 4 KB of a bf16 [P,64] tensor) -> padded smem tile -> A fragments
-__device__ __forceinline__ void head_load_tile(const __nv_bfloat16* __restrict__ src, __nv_bfloat16* tile, int lane) {
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    const int idx = it * 32 + lane, row = idx >> 3, c8 = idx & 7;
-    *reinterpret_cast<uint4*>(tile + row * HD_WS + c8 * 8) = *reinterpret_cast<const uint4*>(src + idx * 8);
-  }
-}
-__device__ __forceinline__ void head_a_frags(const __nv_bfloat16* tile, int g, int q, uint32_t (&a)[2][4][4]) {
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int kt = 0; kt < 4; ++kt) {
-      const __nv_bfloat16* t0 = tile + (mt * 16 + g) * HD_WS + kt * 16 + q * 2;
-      a[mt][kt][0] = *reinterpret_cast<const uint32_t*>(t0);
-      a[mt][kt][1] = *reinterpret_cast<const uint32_t*>(t0 + 8 * HD_WS);
-      a[mt][kt][2] = *reinterpret_cast<const uint32_t*>(t0 + 8);
-      a[mt][kt][3] = *reinterpret_cast<const uint32_t*>(t0 + 8 * HD_WS + 8);
-    }
-}
-// acc[mt][nt] += A[mt] . W^T for NT n-tiles of a [NT*8, 64] bf16 weight block in smem (row stride HD_WS)
-template <int NT>
-__device__ __forceinline__ void head_layer(const uint32_t (&a)[2][4][4], const __nv_bfloat16* w, int g, int q,
-                                           float (&acc)[2][NT][4]) {
-#pragma unroll
-  for (int nt = 0; nt < NT; ++nt)
-#pragma unroll
-    for (int kt = 0; kt < 4; ++kt) {
-      const __nv_bfloat16* bp = w + (nt * 8 + g) * HD_WS + kt * 16 + q * 2;
-      const uint32_t b0 = *reinterpret_cast<const uint32_t*>(bp), b1 = *reinterpret_cast<const uint32_t*>(bp + 8);
-#pragma unroll
-      for (int mt = 0; mt < 2; ++mt) stem_mma(acc[mt][nt], a[mt][kt], b0, b1);
-    }
-}
-__device__ __forceinline__ uint32_t pack_bf2(float x, float y) {
-  const __nv_bfloat162 h = __floats2bfloat162_rn(x, y);
-  return *reinterpret_cast<const uint32_t*>(&h);
-}
-// act(acc + bias) of a 64-wide layer, rounded to bf16 -> the next layer's A fragments
-__device__ __forceinline__ void head_next_frags(const float (&acc)[2][8][4], const float* bias, int q, bool relu,
-                                                uint32_t (&a)[2][4][4]) {
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt) {
-      const float bA = bias[nt * 8 + q * 2], bB = bias[nt * 8 + q * 2 + 1];
-      float v0 = acc[mt][nt][0] + bA, v1 = acc[mt][nt][1] + bB, v2 = acc[mt][nt][2] + bA, v3 = acc[mt][nt][3] + bB;
-      if (relu) { v0 = fmaxf(v0, 0.f); v1 = fmaxf(v1, 0.f); v2 = fmaxf(v2, 0.f); v3 = fmaxf(v3, 0.f); }
-      a[mt][nt >> 1][(nt & 1) * 2] = pack_bf2(v0, v1);       // row g
-      a[mt][nt >> 1][(nt & 1) * 2 + 1] = pack_bf2(v2, v3);   // row g + 8
-    }
-}
-
-// MLPLocalPre{Fpc,Rpc} (model5_b.py:738-739): three 64 -> 64 layers (ReLU after the first two); writes the local
-// features (bf16 [P,64]) and, per CTA, the column maxima of its 128 points (tilemax [cloud][8][64]) for the global
-// max-pool of model5_b.py:741-744
-__global__ void __launch_bounds__(128) head_pre_tc_kernel(const __nv_bfloat16* __restrict__ xfeat_b, Mlp3W wa, Mlp3W wb,
-                                                          const __nv_bfloat16* __restrict__ wimg, int B, int reps,
-                                                          __nv_bfloat16* __restrict__ local,
-                                                          float* __restrict__ tilemax) {
-  __shared__ __align__(16) __nv_bfloat16 ws[3][64 * HD_WS];
-  __shared__ __align__(16) __nv_bfloat16 tiles[4][32 * HD_WS];
-  __shared__ float bs[3][64];
-  __shared__ float cmax[4][64];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, q = lane & 3;
-  const int cloud = (int)(((size_t)blockIdx.x * reps * 128) / NPTS);
-  const Mlp3W& w = cloud / B == 0 ? wa : wb;
-  const float* bsrc[3] = {w.b0, w.b1, w.b2};
-  {   // the set's three [64, HD_WS] bf16 weight images (head_pack_layout), a straight 16-byte copy
-    const uint4* src = reinterpret_cast<const uint4*>(wimg + (size_t)(cloud / B) * HEAD_IMG_SET);
-    uint4* dst = reinterpret_cast<uint4*>(&ws[0][0]);
-    for (int i = tid; i < 3 * 64 * HD_WS / 8; i += 128) dst[i] = src[i];
-  }
-#pragma unroll
-  for (int l = 0; l < 3; ++l)
-    if (tid < 64) bs[l][tid] = bsrc[l][tid];
-  __nv_bfloat16* tile = tiles[warp];
-  __syncthreads();
-#pragma unroll 1
-  for (int rep = 0; rep < reps; ++rep) {
-  const int tile_id = blockIdx.x * reps + rep;
-  const size_t p0 = (size_t)tile_id * 128;
-  head_load_tile(xfeat_b + (p0 + warp * 32) * 64, tile, lane);
-  __syncwarp();
-  uint32_t a[2][4][4];
-  head_a_frags(tile, g, q, a);
-  float acc[2][8][4];
-#pragma unroll 1
-  for (int l = 0; l < 2; ++l) {
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) acc[mt][nt][i] = 0.f;
-    head_layer<8>(a, ws[l], g, q, acc);
-    head_next_frags(acc, bs[l], q, true, a);
-  }
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) acc[mt][nt][i] = 0.f;
-  head_layer<8>(a, ws[2], g, q, acc);
-  // local features (no ReLU), rounded to bf16: staged in the warp's tile, column maxima of the ROUNDED values
-  __syncwarp();
-#pragma unroll
-  for (int nt = 0; nt < 8; ++nt) {
-    const int col = nt * 8 + q * 2;
-    const float bA = bs[2][col], bB = bs[2][col + 1];
-    float mA = -INFINITY, mB = -INFINITY;
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt) {
-      const __nv_bfloat162 r0 = __floats2bfloat162_rn(acc[mt][nt][0] + bA, acc[mt][nt][1] + bB);
-      const __nv_bfloat162 r1 = __floats2bfloat162_rn(acc[mt][nt][2] + bA, acc[mt][nt][3] + bB);
-      *reinterpret_cast<__nv_bfloat162*>(tile + (mt * 16 + g) * HD_WS + col) = r0;
-      *reinterpret_cast<__nv_bfloat162*>(tile + (mt * 16 + g + 8) * HD_WS + col) = r1;
-      const float2 f0 = __bfloat1622float2(r0), f1 = __bfloat1622float2(r1);
-      mA = fmaxf(mA, fmaxf(f0.x, f1.x));
-      mB = fmaxf(mB, fmaxf(f0.y, f1.y));
-    }
-#pragma unroll
-    for (int o = 4; o < 32; o <<= 1) {   // over the 8 row groups g
-      mA = fmaxf(mA, __shfl_xor_sync(0xffffffffu, mA, o));
-      mB = fmaxf(mB, __shfl_xor_sync(0xffffffffu, mB, o));
-    }
-    if (g == 0) {
-      cmax[warp][col] = mA;
-      cmax[warp][col + 1] = mB;
-    }
-  }
-  __syncwarp();
-  __nv_bfloat16* dst = local + (p0 + warp * 32) * 64;
-#pragma unroll
-  for (int it = 0; it < 8; ++it) {
-    const int idx = it * 32 + lane, row = idx >> 3, c8 = idx & 7;
-    *reinterpret_cast<uint4*>(dst + idx * 8) = *reinterpret_cast<const uint4*>(tile + row * HD_WS + c8 * 8);
-  }
-  __syncthreads();
-  if (tid < 64)
-    tilemax[((size_t)cloud * 8 + (tile_id & 7)) * 64 + tid] =
-        fmaxf(fmaxf(cmax[0][tid], cmax[1][tid]), fmaxf(cmax[2][tid], cmax[3][tid]));
-  __syncthreads();   // cmax and the tiles are rewritten by the next repetition
-  }
-}
-
-// MLP{Fpcb,Rpcb} (model5_b.py:745-754): relu(W0 [g ; local] + b0) -> relu(W1 . + b1) -> W2 . + b2, logits as [B,2,1024].
-// g = the MRPC cloud's global max for BOTH heads (D6); its half of layer 0 is a per-cloud bias computed in the prologue.
-// Layer 1 uses split weights (hi + lo) so that, as before, only the activations are rounded to bf16.
-__global__ void __launch_bounds__(128) head_seg_tc_kernel(const __nv_bfloat16* __restrict__ local, Mlp3W wa, Mlp3W wb,
-                                                          const __nv_bfloat16* __restrict__ wimg, int B, int reps,
-                                                          const float* __restrict__ tilemax, float* __restrict__ de_a,
-                                                          float* __restrict__ de_b) {
-  __shared__ __align__(16) __nv_bfloat16 wseg[128 * HD_WS];   // W0 local half [64], W1 hi [32], W1 lo [32]
-  const __nv_bfloat16 *w0s = wseg, *w1h = wseg + 64 * HD_WS, *w1l = wseg + 96 * HD_WS;
-  __shared__ __align__(16) __nv_bfloat16 tiles[4][32 * HD_WS];
-  __shared__ float gs[64], gb[64], b1s[32], w2s[64], b2s[2];
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, q = lane & 3;
-  const int cloud = (int)(((size_t)blockIdx.x * reps * 128) / NPTS), set = cloud / B, b = cloud - set * B;
-  const Mlp3W& w = set == 0 ? wa : wb;
-  {
-    const uint4* src = reinterpret_cast<const uint4*>(wimg + (size_t)set * HEAD_IMG_SET + 3 * 64 * HD_WS);
-    uint4* dst = reinterpret_cast<uint4*>(wseg);
-    for (int i = tid; i < 128 * HD_WS / 8; i += 128) dst[i] = src[i];
-  }
-  if (tid < 64) {
-    const float* tm = tilemax + ((size_t)(B + b) * 8) * 64 + tid;   // the mrpc cloud of pair b
-    float m = tm[0];
-#pragma unroll
-    for (int i = 1; i < 8; ++i) m = fmaxf(m, tm[i * 64]);
-    gs[tid] = m;
-    w2s[tid] = w.w2[tid];
-  }
-  if (tid < 32) b1s[tid] = w.b1[tid];
-  if (tid < 2) b2s[tid] = w.b2[tid];
-  __nv_bfloat16* tile = tiles[warp];
-  __syncthreads();
-  if (tid < 64) {
-    float v = w.b0[tid];
-    const float* wr = w.w0 + tid * 128;
-    for (int i = 0; i < 64; ++i) v = fmaf(wr[i], gs[i], v);
-    gb[tid] = v;
-  }
-  __syncthreads();
-#pragma unroll 1
-  for (int rep = 0; rep < reps; ++rep) {
-  const size_t p0 = ((size_t)blockIdx.x * reps + rep) * 128;
-  const int n0 = (int)(p0 - (size_t)cloud * NPTS) + warp * 32;
-  head_load_tile(local + (p0 + warp * 32) * 64, tile, lane);
-  __syncwarp();
-  uint32_t a[2][4][4];
-  head_a_frags(tile, g, q, a);
-  float acc[2][8][4];
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) acc[mt][nt][i] = 0.f;
-  head_layer<8>(a, w0s, g, q, acc);
-  head_next_frags(acc, gb, q, true, a);
-  float h1[2][4][4];
-#pragma unroll
-  for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-    for (int nt = 0; nt < 4; ++nt)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) h1[mt][nt][i] = 0.f;
-  head_layer<4>(a, w1l, g, q, h1);
-  head_layer<4>(a, w1h, g, q, h1);
-  // layer 2 (32 -> 2) on the fp32 fragments: this thread holds 8 of the 32 hidden channels of its 4 rows
-  float o[4][2];
-#pragma unroll
-  for (int j = 0; j < 4; ++j) o[j][0] = o[j][1] = 0.f;
-#pragma unroll
-  for (int nt = 0; nt < 4; ++nt) {
-    const int col = nt * 8 + q * 2;
-    const float bA = b1s[col], bB = b1s[col + 1];
-    const float wA0 = w2s[col], wB0 = w2s[col + 1], wA1 = w2s[32 + col], wB1 = w2s[32 + col + 1];
-#pragma unroll
-    for (int mt = 0; mt < 2; ++mt)
-#pragma unroll
-      for (int hf = 0; hf < 2; ++hf) {
-        const float hA = fmaxf(h1[mt][nt][2 * hf] + bA, 0.f), hB = fmaxf(h1[mt][nt][2 * hf + 1] + bB, 0.f);
-        const int j = 2 * mt + hf;
-        o[j][0] = fmaf(wA0, hA, fmaf(wB0, hB, o[j][0]));
-        o[j][1] = fmaf(wA1, hA, fmaf(wB1, hB, o[j][1]));
-      }
-  }
-#pragma unroll
-  for (int j = 0; j < 4; ++j)
-#pragma unroll
-    for (int c = 0; c < 2; ++c) {
-      o[j][c] += __shfl_xor_sync(0xffffffffu, o[j][c], 1);
-      o[j][c] += __shfl_xor_sync(0xffffffffu, o[j][c], 2);
-    }
-  if (q == 0) {
-    float* de = set == 0 ? de_a : de_b;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int n = n0 + g + 8 * j;
-      de[((size_t)b * 2 + 0) * NPTS + n] = o[j][0] + b2s[0];
-      de[((size_t)b * 2 + 1) * NPTS + n] = o[j][1] + b2s[1];
-    }
-  }
-  __syncwarp();   // the tile is rewritten by the next repetition
-  }
-}
-
 // ------------------------------------------------------------ se3.exp (se_math/se3.py:57-80)
 __global__ void se3_exp_kernel(const float* __restrict__ x, int B, float* __restrict__ g) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1127,10 +844,9 @@ struct EncoderScratch {
 };
 
 // bf16 weight pack of ONE encoder (elements): W3f[128,64] W4[128,128] W5f[256,128] W6[256,256]
-// 4 x (Wqkv[384,256] Wo[256,256]) Wout[1024,1280]  4 x (20 tile images of Wqkv|Wo for the fused attention layer)
+// Wout[1024,1280]  4 x (20 tile images of Wqkv|Wo for the fused attention layer)
 constexpr size_t WP_W3F = 0, WP_W4 = WP_W3F + 128 * 64, WP_W5F = WP_W4 + 128 * 128, WP_W6 = WP_W5F + 256 * 128,
-                 WP_ATT = WP_W6 + 256 * 256, WP_ATT_STRIDE = 384 * 256 + 256 * 256, WP_WOUT = WP_ATT + 4 * WP_ATT_STRIDE,
-                 WP_ATTIMG = WP_WOUT + 1024 * 1280, WP_STEM = WP_ATTIMG + 4 * ATTN_WIMG_ELEMS,
+                 WP_WOUT = WP_W6 + 256 * 256, WP_ATTIMG = WP_WOUT + 1024 * 1280, WP_STEM = WP_ATTIMG + 4 * ATTN_WIMG_ELEMS,
                  WP_TOTAL = WP_STEM + 2 * 64 * STEM_WS;   // stem: W2 hi, lo as [64, STEM_WS] images
 
 // split path: fp16 planes of ONE encoder (elements per plane): W3f[128,64] W4[128,128] W5f[256,128] W6[256,256]
@@ -1179,7 +895,7 @@ static size_t encoder_scratch_layout(int C, Arena& a, EncoderScratch& s) {
 // ---------------------------------------------------------------------------------------------
 // runs on the caller's stream right after the stem: work that only needs x_feature (the boundary heads of predict5)
 // fills the time the stream would otherwise spend waiting for the stage-1 geometry
-using AfterStem = std::function<int(const float* xfeat, const __nv_bfloat16* xfeat_b)>;
+using AfterStem = std::function<int(const float* xfeat)>;
 
 static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
                                 const int64_t* start2, const PzEncoderOutputs& o, EncoderScratch& s, float* fglob_pair,
@@ -1208,11 +924,6 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
       add(we.mlp5_w + 3, 3 + C1B, C2A, C1B, wp + WP_W5F, C1B, 1);
       add(we.mlp6_w, C2A, C2B, C2A, wp + WP_W6, C2A, 1);
       for (int l = 0; l < 4; ++l) {
-        __nv_bfloat16* wl = wp + WP_ATT + (size_t)l * WP_ATT_STRIDE;
-        add(we.q_w[l], CATT, 64, CATT, wl, CATT, 1);
-        add(we.k_w[l], CATT, 64, CATT, wl + 64 * CATT, CATT, 1);
-        add(we.v_w[l], CATT, CATT, CATT, wl + 128 * CATT, CATT, 1);
-        add(we.o_w[l], CATT, CATT, CATT, wl + 384 * CATT, CATT, 1);
         __nv_bfloat16* wi = wp + WP_ATTIMG + (size_t)l * ATTN_WIMG_ELEMS;
         add(we.q_w[l], CATT, 64, CATT, wi, 0, 2);
         add(we.k_w[l], CATT, 64, CATT, wi, 64, 2);
@@ -1240,8 +951,7 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
   // it runs on the side stream while the feature chain (stem, layer-1 GEMM) runs on the caller's stream.
   SideStream* ss = nullptr;
   PZ_TRY(side_stream(&ss, st));
-  static const bool env_serial = getenv("PZ_NO_SIDE_STREAM") != nullptr;   // profiling aid: clean per-stage times
-  const bool serial = env_serial || prof_serial();
+  const bool serial = prof_serial();
   cudaStream_t sg = serial ? st : ss->stream;
   const int gl = serial ? 0 : 1;   // profiler lane of the geometry marks
   PZ_CUDA(cudaEventRecord(ss->fork, st));
@@ -1258,13 +968,9 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
   prof_mark("knn2", sg, gl);
   PZ_CUDA(cudaEventRecord(ss->join_b, sg));
 
-  static const bool stem_fp32 = getenv("PZ_STEM_FP32") && getenv("PZ_STEM_FP32")[0] == '1';   // A/B hook
-  if (stem_fp32) stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, xfeat, s.xfeat_b, nullptr, nullptr);
-  else {
-    PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
-    stem_tc_kernel<false><<<C * NPTS / (128 * head_reps()), 128, STEM_TC_SMEM, st>>>(xyz, stem_of(wa), stem_of(wb), wpa + WP_STEM,
-                                                                              wpb + WP_STEM, B, head_reps(), xfeat, s.xfeat_b, nullptr);
-  }
+  PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
+  stem_tc_kernel<false><<<C * NPTS / (128 * HD_REPS), 128, STEM_TC_SMEM, st>>>(xyz, stem_of(wa), stem_of(wb), wpa + WP_STEM,
+                                                                          wpb + WP_STEM, B, HD_REPS, xfeat, s.xfeat_b, nullptr);
   PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
   {
@@ -1275,7 +981,7 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     PZ_TRY(launch_tc_rowgemm(g, st));
     prof_mark("sg1_layer1", st);
   }
-  if (after_stem) PZ_TRY((*after_stem)(xfeat, s.xfeat_b));
+  if (after_stem) PZ_TRY((*after_stem)(xfeat));
   PZ_CUDA(cudaStreamWaitEvent(st, ss->join_a, 0));   // kNN of stage 1 (and FPS 1, Q1) are done
   prof_mark("_wait_geometry1", st);
   {
@@ -1314,8 +1020,7 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
 
   // ---- 4 x offset attention
   const int rows = C * LATT;
-  static const bool fused_attn = !(getenv("PZ_FUSED_ATTN") && getenv("PZ_FUSED_ATTN")[0] == '0');
-  if (fused_attn) {   // the four layers of a cloud in one launch: nothing but the layer inputs / outputs touches HBM
+  {   // the four layers of a cloud in one launch: nothing but the layer inputs / outputs touches HBM
     AttnLayerTc p;
     p.nlayers = 4;
     p.x = cat_b + 4 * CATT; p.ldx = 1280;
@@ -1330,37 +1035,6 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     p.attn = o.attention;
     PZ_TRY(launch_attention_layer_tc(p, C, st));
     prof_mark("attn_layer_fused", st);
-  }
-  for (int l = 0; l < 4 && !fused_attn; ++l) {
-    const __nv_bfloat16* xb = l == 0 ? cat_b + 4 * CATT : cat_b + (l - 1) * CATT;
-    const __nv_bfloat16* wla = wpa + WP_ATT + (size_t)l * WP_ATT_STRIDE;
-    const __nv_bfloat16* wlb = wpb + WP_ATT + (size_t)l * WP_ATT_STRIDE;
-    {
-      // [q | k] = x Wqk^T + b  (row-major bf16, row-per-thread epilogue) and v^T = (x Wv^T + b)^T per cloud
-      // (channel-per-thread epilogue: the transposed store is contiguous there, and K-major for the P v MMA)
-      TcGemm gq;
-      gq.X = xb; gq.ldx = 1280; gq.W[0] = wla; gq.W[1] = wlb; gq.ldw = CATT;
-      gq.bias[0] = s.bqkv + (size_t)l * 384; gq.bias[1] = s.bqkv + ((size_t)(E - 1) * 4 + l) * 384;
-      gq.rows_per_wset = B * LATT; gq.M = rows; gq.Nout = 128; gq.K = CATT; gq.Yb = s.qk_b; gq.ldyb = 128;
-      PZ_TRY(launch_tc_rowgemm(gq, st));
-      TcGemm gv = gq;
-      gv.W[0] = wla + 128 * CATT; gv.W[1] = wlb + 128 * CATT; gv.bias[0] = gq.bias[0] + 128; gv.bias[1] = gq.bias[1] + 128;
-      gv.Nout = CATT; gv.Yb = nullptr; gv.YT = s.vT_b; gv.t_ch_begin = 0;
-      PZ_TRY(launch_tc_gemm(gv, st));
-      prof_mark("attn_qkv_proj", st);
-    }
-    const int amode = o.attention ? (l == 0 ? 1 : (l == 3 ? 3 : 2)) : 0;
-    PZ_TRY(launch_attention_tc(s.qk_b, s.vT_b, xb, 1280, C, s.r_b, o.attention, amode, st));
-    prof_mark("attn_softmax_av", st);
-    {
-      TcGemm g;  // out = x + relu(Wo r + bo)
-      g.X = s.r_b; g.ldx = CATT; g.W[0] = wla + 384 * CATT; g.W[1] = wlb + 384 * CATT; g.ldw = CATT;
-      g.bias[0] = wa.o_b[l]; g.bias[1] = wb.o_b[l]; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = CATT; g.K = CATT;
-      g.relu = 1; g.Rb = xb; g.ldrb = 1280; g.Yb = cat_b + l * CATT; g.ldyb = 1280;
-      if (cat_f) { g.Yf = cat_f + l * CATT; g.ldyf = 1280; }
-      PZ_TRY(launch_tc_rowgemm(g, st));
-      prof_mark("attn_out_proj", st);
-    }
   }
   // ---- tail
   {
@@ -1468,51 +1142,31 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
   // programmatic launch chain is broken by the memset node
   PZ_CUDA(cudaMemsetAsync(s.tailp, 0, (size_t)3 * C * sizeof(int), st));
 
-  // ---- geometry (FPS -> centre projection -> kNN, both stages): ahead of the feature chain on the caller's stream
-  SideStream* ss = nullptr;
-  PZ_TRY(side_stream(&ss, st));
-  // ONE chain by default: every GEMM CTA of this path fills an SM (shared memory), so a geometry kernel on a second stream
-  // does not share SMs with them, it delays some of the CTAs of a persistent GEMM and the whole launch waits for those
-  // (eager forward 1.70 ms with the side stream, 1.59 without, 1.51 with programmatic dependent launch on the one chain;
-  // the 4-stream graph schedule 1.39 vs 1.37 ms per step).  PZ_SIDE_STREAM=1 restores the second stream (A/B hook).
-  static const bool env_serial = getenv("PZ_SIDE_STREAM") == nullptr || getenv("PZ_NO_SIDE_STREAM") != nullptr;
-  const bool serial = env_serial || prof_serial();
-  cudaStream_t sg = serial ? st : ss->stream;
-  const int gl = serial ? 0 : 1;
-  if (!serial) {
-    PZ_CUDA(cudaEventRecord(ss->fork, st));
-    PZ_CUDA(cudaStreamWaitEvent(sg, ss->fork, 0));
-  }
-  prof_mark("_side_begin", sg, gl);
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, sg));
-  prof_mark("fps1", sg, gl);
-  PZ_TRY(launch_knn(s.nx1, xyz, C, S1, NPTS, KNN, o.knn1, s.knn1r, nullptr, sg));
-  prof_mark("knn1", sg, gl);
-  PZ_TRY(launch_centre_proj_f32(s.nx1, wa.mlp3_w, wb.mlp3_w, 3 + D0, B * S1, C * S1, C1A, Q1, sg));
-  if (!serial) PZ_CUDA(cudaEventRecord(ss->join_a, sg));
-  PZ_TRY(launch_fps(s.nx1, C, S1, start2, S2, o.fps2, nullptr, nx2, sg));
-  prof_mark("fps2", sg, gl);
-  PZ_TRY(launch_knn(nx2, s.nx1, C, S2, S1, KNN, o.knn2, s.knn2r, nullptr, sg));
-  prof_mark("knn2", sg, gl);
-  PZ_TRY(launch_centre_proj_f32(nx2, wa.mlp5_w, wb.mlp5_w, 3 + C1B, B * S2, C * S2, C2A, Q2, sg));
-  if (!serial) PZ_CUDA(cudaEventRecord(ss->join_b, sg));
+  // ---- geometry (FPS -> centre projection -> kNN, both stages): ahead of the feature chain on the caller's stream.
+  // ONE chain: every GEMM CTA of this path fills an SM (shared memory), so a geometry kernel on a second stream does not
+  // share SMs with them, it delays some of the CTAs of a persistent GEMM and the whole launch waits for those (eager
+  // forward 1.70 ms with a side stream, 1.59 without, 1.51 with programmatic dependent launch on the one chain; the
+  // 4-stream graph schedule 1.39 vs 1.37 ms per step).
+  prof_mark("_side_begin", st);
+  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, st));
+  prof_mark("fps1", st);
+  PZ_TRY(launch_knn(s.nx1, xyz, C, S1, NPTS, KNN, o.knn1, s.knn1r, nullptr, st));
+  prof_mark("knn1", st);
+  PZ_TRY(launch_centre_proj_f32(s.nx1, wa.mlp3_w, wb.mlp3_w, 3 + D0, B * S1, C * S1, C1A, Q1, st));
+  PZ_TRY(launch_fps(s.nx1, C, S1, start2, S2, o.fps2, nullptr, nx2, st));
+  prof_mark("fps2", st);
+  PZ_TRY(launch_knn(nx2, s.nx1, C, S2, S1, KNN, o.knn2, s.knn2r, nullptr, st));
+  prof_mark("knn2", st);
+  PZ_TRY(launch_centre_proj_f32(nx2, wa.mlp5_w, wb.mlp5_w, 3 + C1B, B * S2, C * S2, C2A, Q2, st));
 
   // ---- feature chain
   // stem: layer 2 as a split-fp16 mma.sync product (x_feature within ~1e-6 of the fp32 stem), the fp16 hi / lo planes of
-  // x_feature written by the same kernel; PZ_STEM_FFMA=1 keeps the FFMA stem + a separate plane pass (A/B hook)
-  static const bool stem_ffma = getenv("PZ_STEM_FFMA") && getenv("PZ_STEM_FFMA")[0] == '1';
-  const int reps = head_reps();
-  if (stem_ffma || (C * NPTS) % (128 * reps) != 0) {
-    stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, xfeat, nullptr, nullptr, nullptr);
-    PZ_LAUNCH_CHECK();
-    PZ_TRY(launch_split_planes(xfeat, D0, (size_t)C * NPTS, D0, xfeat_h[0], xfeat_h[1], D0, st));
-  } else {
-    PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
-    PZ_CUDA(launch_pdl(stem_tc_kernel<true>, dim3(C * NPTS / (128 * reps)), dim3(128), STEM_TC_SMEM, st, xyz, stem_of(wa), stem_of(wb),
-                       (const __nv_bfloat16*)nullptr, (const __nv_bfloat16*)nullptr, B, reps, xfeat,
-                       reinterpret_cast<__nv_bfloat16*>(xfeat_h[0]), reinterpret_cast<__half*>(xfeat_h[1])));
-    PZ_LAUNCH_CHECK();
-  }
+  // x_feature written by the same kernel (C * 1024 points always tile by 128 * HD_REPS)
+  PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
+  PZ_CUDA(launch_pdl(stem_tc_kernel<true>, dim3(C * NPTS / (128 * HD_REPS)), dim3(128), STEM_TC_SMEM, st, xyz, stem_of(wa),
+                     stem_of(wb), (const __nv_bfloat16*)nullptr, (const __nv_bfloat16*)nullptr, B, HD_REPS, xfeat,
+                     reinterpret_cast<__nv_bfloat16*>(xfeat_h[0]), reinterpret_cast<__half*>(xfeat_h[1])));
+  PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
   {
     TcGemm g;  // P1 = x_feature W3[:,3:]^T + b3 + W3[:,0:3] xyz   (fp32 out)
@@ -1522,8 +1176,7 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
     PZ_TRY(launch_split_rowgemm(g, st));
     prof_mark("sg1_layer1", st);
   }
-  if (after_stem) PZ_TRY((*after_stem)(xfeat, nullptr));
-  if (!serial) PZ_CUDA(cudaStreamWaitEvent(st, ss->join_a, 0));
+  if (after_stem) PZ_TRY((*after_stem)(xfeat));
   prof_mark("_wait_geometry1", st);
   {
     TcGemm g;  // f1f = max_k relu(W4 relu(P1[j] - Q1[s]) + b4)
@@ -1541,7 +1194,6 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
     PZ_TRY(launch_split_rowgemm(g, st));
     prof_mark("sg2_layer1", st);
   }
-  if (!serial) PZ_CUDA(cudaStreamWaitEvent(st, ss->join_b, 0));
   prof_mark("_wait_geometry2", st);
   float* cat_f = o.att_cat;
   {
@@ -1563,20 +1215,16 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
   // the out-projection  out = x + relu(Wo r + bo)  runs inside the attention kernel (r never leaves the SM: 67 MB of HBM
   // traffic and one launch per layer less), and so do the NEXT layer's q|k|v projections of the same rows (chained: two
   // more launches per layer less); q|k and v^T planes then alternate between two buffer sets, because the CTAs of a launch
-  // still read the current ones.  PZ_ATTN_NO_FUSE / PZ_ATTN_NO_CHAIN keep them separate row GEMMs (A/B hooks).
-  static const bool attn_no_fuse = getenv("PZ_ATTN_NO_FUSE") != nullptr;
-  static const bool attn_no_chain = attn_no_fuse || getenv("PZ_ATTN_NO_CHAIN") != nullptr;
+  // still read the current ones.
   // chained launches hand over per cloud (AttnSplit::dep_flags): 3 x C counters in the tail's scratch, idle until the tail
-  static const bool attn_no_pdl = getenv("PZ_ATTN_NO_PDL") != nullptr;   // A/B hook
   int* aflags = reinterpret_cast<int*>(s.tailp);
-  const bool handover = !attn_no_chain && !attn_no_pdl && pdl_enabled();
   h16* qk_set[2][2] = {{qk_h[0], qk_h[1]}, {s.xfeat_b, reinterpret_cast<h16*>(s.k)}};   // second set: idle buffers of equal size
-  h16* vT_set[2][2] = {{vT_h[0], vT_h[1]}, {r_h[0], r_h[1]}};                           // (r is not materialised when fused)
+  h16* vT_set[2][2] = {{vT_h[0], vT_h[1]}, {r_h[0], r_h[1]}};                           // (r is not materialised)
   for (int l = 0; l < 4; ++l) {
     const size_t xoff = l == 0 ? 4 * CATT : (size_t)(l - 1) * CATT;
     const size_t wl = WS_ATT + (size_t)l * WS_ATT_STRIDE;
-    const int cur = attn_no_chain ? 0 : (l & 1);
-    if (l == 0 || attn_no_chain) {
+    const int cur = l & 1;
+    if (l == 0) {
       TcGemm gq;  // [q | k] = x Wqk^T + b
       gq.X = cat_h[0] + xoff; gq.Xlo = cat_h[1] + xoff; gq.ldx = 1280; set_w(gq, wl); gq.ldw = CATT;
       gq.bias[0] = s.bqkv + (size_t)l * 384; gq.bias[1] = s.bqkv + ((size_t)(E - 1) * 4 + l) * 384;
@@ -1592,34 +1240,21 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
     ap.qk_hi = qk_set[cur][0]; ap.qk_lo = qk_set[cur][1]; ap.vT_hi = vT_set[cur][0]; ap.vT_lo = vT_set[cur][1];
     ap.x_hi = cat_h[0] + xoff; ap.x_lo = cat_h[1] + xoff; ap.ldx = 1280; ap.r_hi = r_h[0]; ap.r_lo = r_h[1];
     ap.attn = o.attention; ap.attn_mode = o.attention ? (l == 0 ? 1 : (l == 3 ? 3 : 2)) : 0;
-    if (!attn_no_fuse) {
-      ap.wo_hi[0] = wp_[0][0] + wl + 384 * CATT; ap.wo_lo[0] = wp_[0][1] + wl + 384 * CATT;
-      ap.wo_hi[1] = wp_[1][0] + wl + 384 * CATT; ap.wo_lo[1] = wp_[1][1] + wl + 384 * CATT;
-      ap.bo[0] = wa.o_b[l]; ap.bo[1] = wb.o_b[l]; ap.clouds_per_set = B;
-      ap.y_hi = cat_h[0] + (size_t)l * CATT; ap.y_lo = cat_h[1] + (size_t)l * CATT; ap.ldy = 1280;
-      if (cat_f) { ap.yf = cat_f + (size_t)l * CATT; ap.ldyf = 1280; }
-      if (!attn_no_chain && l < 3) {   // the next layer's projections of these rows
-        const size_t wn = WS_ATT + (size_t)(l + 1) * WS_ATT_STRIDE;
-        ap.wqkv_hi[0] = wp_[0][0] + wn; ap.wqkv_lo[0] = wp_[0][1] + wn; ap.wqkv_hi[1] = wp_[1][0] + wn; ap.wqkv_lo[1] = wp_[1][1] + wn;
-        ap.bqkv[0] = s.bqkv + (size_t)(l + 1) * 384; ap.bqkv[1] = s.bqkv + ((size_t)(E - 1) * 4 + l + 1) * 384;
-        ap.qk2_hi = qk_set[cur ^ 1][0]; ap.qk2_lo = qk_set[cur ^ 1][1]; ap.vT2_hi = vT_set[cur ^ 1][0]; ap.vT2_lo = vT_set[cur ^ 1][1];
-        if (handover) ap.sig_flags = aflags + (size_t)l * C;
-      }
-      if (handover && l > 0) ap.dep_flags = aflags + (size_t)(l - 1) * C;
-      PZ_TRY(launch_attention_split(ap, C, st));
-      prof_mark("attn_softmax_av", st);
-      continue;
+    ap.wo_hi[0] = wp_[0][0] + wl + 384 * CATT; ap.wo_lo[0] = wp_[0][1] + wl + 384 * CATT;
+    ap.wo_hi[1] = wp_[1][0] + wl + 384 * CATT; ap.wo_lo[1] = wp_[1][1] + wl + 384 * CATT;
+    ap.bo[0] = wa.o_b[l]; ap.bo[1] = wb.o_b[l]; ap.clouds_per_set = B;
+    ap.y_hi = cat_h[0] + (size_t)l * CATT; ap.y_lo = cat_h[1] + (size_t)l * CATT; ap.ldy = 1280;
+    if (cat_f) { ap.yf = cat_f + (size_t)l * CATT; ap.ldyf = 1280; }
+    if (l < 3) {   // the next layer's projections of these rows
+      const size_t wn = WS_ATT + (size_t)(l + 1) * WS_ATT_STRIDE;
+      ap.wqkv_hi[0] = wp_[0][0] + wn; ap.wqkv_lo[0] = wp_[0][1] + wn; ap.wqkv_hi[1] = wp_[1][0] + wn; ap.wqkv_lo[1] = wp_[1][1] + wn;
+      ap.bqkv[0] = s.bqkv + (size_t)(l + 1) * 384; ap.bqkv[1] = s.bqkv + ((size_t)(E - 1) * 4 + l + 1) * 384;
+      ap.qk2_hi = qk_set[cur ^ 1][0]; ap.qk2_lo = qk_set[cur ^ 1][1]; ap.vT2_hi = vT_set[cur ^ 1][0]; ap.vT2_lo = vT_set[cur ^ 1][1];
+      ap.sig_flags = aflags + (size_t)l * C;
     }
+    if (l > 0) ap.dep_flags = aflags + (size_t)(l - 1) * C;
     PZ_TRY(launch_attention_split(ap, C, st));
     prof_mark("attn_softmax_av", st);
-    TcGemm g;  // out = x + relu(Wo r + bo)
-    g.X = r_h[0]; g.Xlo = r_h[1]; g.ldx = CATT; set_w(g, wl + 384 * CATT); g.ldw = CATT;
-    g.bias[0] = wa.o_b[l]; g.bias[1] = wb.o_b[l]; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = CATT; g.K = CATT;
-    g.relu = 1; g.Rb = cat_h[0] + xoff; g.Rblo = cat_h[1] + xoff; g.ldrb = 1280;
-    g.Yb = cat_h[0] + (size_t)l * CATT; g.Yblo = cat_h[1] + (size_t)l * CATT; g.ldyb = 1280;
-    if (cat_f) { g.Yf = cat_f + (size_t)l * CATT; g.ldyf = 1280; }
-    PZ_TRY(launch_split_rowgemm(g, st));
-    prof_mark("attn_out_proj", st);
   }
   // ---- tail: Linear(1280, 1024), then the max over the 256 points of a cloud
   {
@@ -1673,10 +1308,10 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
   if (xfeat_out) *xfeat_out = xfeat;
 
   // stem: Linear(3,64)+BN+ReLU, Linear(64,64)+BN+ReLU -> x_feature [C,1024,64]
-  stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, xfeat, nullptr, nullptr, nullptr);
+  stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, xfeat);
   PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
-  if (after_stem) PZ_TRY((*after_stem)(xfeat, nullptr));
+  if (after_stem) PZ_TRY((*after_stem)(xfeat));
 
   // ---- stage 1: FPS 1024->512, kNN 32, grouped MLP 67->128->128, max over K
   PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, st));
@@ -1781,11 +1416,6 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
   return 0;
 }
 
-// PZ_HEADS_BF16=1 selects the former bf16 boundary heads on the bf16 path (A/B hook)
-static bool old_bf16_heads() {
-  static const bool v = getenv("PZ_HEADS_BF16") && getenv("PZ_HEADS_BF16")[0] == '1';
-  return v;
-}
 constexpr size_t HL_SMEM = (3 * 4160 + 64 * 128) * sizeof(float);
 constexpr size_t HS_SMEM = (64 * 64 + 32 * 64 + 64 + 32 + 64 + 4 + 64 * 128) * sizeof(float);
 static int set_head_fp32_smem() {
@@ -1819,7 +1449,7 @@ extern "C" int pz_encoder_forward(const PzEncoderWeights* weights_host, int E, i
 namespace {
 struct PredictScratch {
   float *xyz, *fpair, *h0, *h1, *partial, *local, *gmax, *gbias, *tilemax;
-  __nv_bfloat16 *ha, *himg, *himg_split;
+  __nv_bfloat16* himg_split;
   int64_t *st1, *st2;
   void* enc;
   size_t enc_bytes, partial_floats;
@@ -1837,8 +1467,6 @@ size_t predict_layout(int B, Arena& a, PredictScratch& s) {
   s.gmax = a.take<float>((size_t)B * 64);
   s.gbias = a.take<float>((size_t)2 * B * 64);
   s.tilemax = a.take<float>((size_t)2 * B * 8 * 128);
-  s.ha = a.take<__nv_bfloat16>((size_t)2 * B * NPTS * 64);
-  s.himg = a.take<__nv_bfloat16>(2 * HEAD_IMG_SET);
   s.himg_split = a.take<__nv_bfloat16>(2 * HEAD_SPLIT_IMG_SET);
   s.enc_bytes = pz_encoder_workspace_bytes(2, B);
   s.enc = a.take<char>(s.enc_bytes);
@@ -1905,41 +1533,12 @@ int predict_front(const PzEncoderWeights* enc_host, const PzHeadWeights& h, cons
   const int P = 2 * B * NPTS;
 
   // boundary heads (model5_b.py:738-754): they only need x_feature, so the encoder runs them right after its stem
-  AfterStem heads_fn = [&](const float* xfeat, const __nv_bfloat16* xfeat_b) -> int {
-    if (precision == PZ_PREC_SPLIT || (precision == PZ_PREC_BF16 && !old_bf16_heads())) {
+  AfterStem heads_fn = [&](const float* xfeat) -> int {
+    if (precision == PZ_PREC_SPLIT || precision == PZ_PREC_BF16) {
       // split-fp16 chained-MMA heads on the fp32 x_feature (heads_split.cu): logits at fp32 tolerance in both
       // tensor-core precisions (the bf16 path's stem is a split product too, so its x_feature is fp32-accurate)
       PZ_TRY(launch_heads_split(xfeat, pre_f, pre_r, seg_f, seg_r, B, reuse_pack, s.himg_split, local, tilemax, de_fpcb,
                                 de_mrpcb, st));
-      prof_mark("boundary_heads", st);
-      return 0;
-    }
-    if (precision == PZ_PREC_BF16) {
-      // two chained-MMA kernels (activations stay in registers between layers): the three local layers + per-CTA
-      // column maxima, then the segmentation head with the mrpc cloud's global feature folded into a per-cloud bias
-      if (!reuse_pack) {   // bf16 weight images of both heads (one launch; skipped while the caller vouches for the weights)
-        PackJobs jobs;
-        int n = 0;
-        for (int e = 0; e < 2; ++e) {
-          const Mlp3W& pre = e == 0 ? pre_f : pre_r;
-          const Mlp3W& seg = e == 0 ? seg_f : seg_r;
-          __nv_bfloat16* wp = s.himg + (size_t)e * HEAD_IMG_SET;
-          jobs.j[n++] = PackJob{pre.w0, wp, 64, 64, 64, HD_WS, 1};
-          jobs.j[n++] = PackJob{pre.w1, wp + 64 * HD_WS, 64, 64, 64, HD_WS, 1};
-          jobs.j[n++] = PackJob{pre.w2, wp + 128 * HD_WS, 64, 64, 64, HD_WS, 1};
-          jobs.j[n++] = PackJob{seg.w0 + 64, wp + 192 * HD_WS, 128, 64, 64, HD_WS, 1};   // local half: columns 64..127
-          jobs.j[n++] = PackJob{seg.w1, wp + 256 * HD_WS, 64, 32, 64, HD_WS, 1};
-          jobs.j[n++] = PackJob{seg.w1, wp + 288 * HD_WS, 64, 32, 64, HD_WS, 3};
-        }
-        jobs.n = n;
-        pack_weights_kernel<<<dim3(16, n), 256, 0, st>>>(jobs);
-        PZ_LAUNCH_CHECK();
-      }
-      head_pre_tc_kernel<<<P / (128 * head_reps()), 128, 0, st>>>(xfeat_b, pre_f, pre_r, s.himg, B, head_reps(), s.ha, s.tilemax);
-      PZ_LAUNCH_CHECK();
-      head_seg_tc_kernel<<<P / (128 * head_reps()), 128, 0, st>>>(s.ha, seg_f, seg_r, s.himg, B, head_reps(), s.tilemax, de_fpcb,
-                                                                  de_mrpcb);
-      PZ_LAUNCH_CHECK();
       prof_mark("boundary_heads", st);
       return 0;
     }
@@ -2090,8 +1689,6 @@ extern "C" int pz_encode_pieces(const PzEncoderWeights* enc_host, const PzHeadWe
   PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
              "pz_encode_pieces: unknown precision %d", precision);
   PZ_REQUIRE(!(flags & PZ_FLAG_NEED), PZ_ERR_UNSUPPORTED, "pz_encode_pieces: PZ_FLAG_NEED is not supported");
-  PZ_REQUIRE(!(precision == PZ_PREC_BF16 && old_bf16_heads()), PZ_ERR_UNSUPPORTED,
-             "pz_encode_pieces: the legacy bf16 heads (PZ_HEADS_BF16=1) are not supported");
   PZ_TRY(check_heads(heads_host, "pz_encode_pieces"));
   cudaStream_t st = as_stream(stream);
   Arena arena(workspace, workspace_bytes);
@@ -2132,8 +1729,6 @@ extern "C" int pz_predict_pairs(const PzHeadWeights* heads_host, const PzPieceEm
   PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
              "pz_predict_pairs: unknown precision %d", precision);
   PZ_REQUIRE(!(flags & PZ_FLAG_NEED), PZ_ERR_UNSUPPORTED, "pz_predict_pairs: PZ_FLAG_NEED is not supported");
-  PZ_REQUIRE(!(precision == PZ_PREC_BF16 && old_bf16_heads()), PZ_ERR_UNSUPPORTED,
-             "pz_predict_pairs: the legacy bf16 heads (PZ_HEADS_BF16=1) are not supported");
   PZ_TRY(check_heads(heads_host, "pz_predict_pairs"));
   PZ_REQUIRE(embeddings_aligned(e) && ((uintptr_t)de_mrpcb & 15) == 0, PZ_ERR_ARG,
              "pz_predict_pairs: embedding buffers and de_mrpcb must be 16-byte aligned");

@@ -14,7 +14,7 @@
 //   split_rowgemm_pair_kernel : Y[row, ch] row-major GEMM on a CTA PAIR (tcgen05.mma.cta_group::2, M = 256 rows), operands
 //                               by TMA, the CTA's weight half resident where it fits; every plain nn.Linear (layer 1 of the
 //                               grouped MLPs over source points, q|k and v projections, out-projection with residual, tail)
-//   split_rowgemm_kernel      : the one-CTA cp.async version (shapes that do not tile by 256 rows; PZ_RG_NO_PAIR)
+//   split_rowgemm_kernel      : the one-CTA cp.async version (shapes that do not tile by 256 rows)
 //   split_gather_kernel       : grouped-MLP layer 2 with the gathered operand relu(P[j] - Q[s]) formed IN REGISTERS from
 //                               fp32 P rows (global -> registers -> swizzled st.shared per plane) and the max over the 32
 //                               neighbours in the epilogue (pointnet_util.py:123-130 + model5_b.py:452-454, :459-461)
@@ -866,10 +866,9 @@ int launch_split_rowgemm(const TcGemm& g, cudaStream_t st) {
   if (g.n_valid > 0) PZ_REQUIRE(g.n_valid % 32 == 0, PZ_ERR_ARG, "split_rowgemm: n_valid must be a multiple of 32");
   if (g.YT) PZ_REQUIRE(g.t_rows % 128 == 0, PZ_ERR_ARG, "split_rowgemm: t_rows must be a multiple of 128");
   // 256-column tiles halve the re-reads of X but leave at most two tiles per CTA at M = 32768 (the epilogue of a tile then
-  // has little to overlap with); PZ_SPLIT_NCOLS=128 forces 128-column tiles everywhere (A/B hook)
+  // has little to overlap with)
   // CTA-pair kernels (cta_group::2) whenever the rows tile by 256 per weight set
-  static const bool no_pair = getenv("PZ_RG_NO_PAIR") != nullptr;   // A/B hook
-  if (!no_pair && g.M % (256 * nsets) == 0) {
+  if (g.M % (256 * nsets) == 0) {
     if (g.Nout == 256 && !g.Ymax) {
       if (split_rowgemm_pair_smem(g, 256, 3, true) <= 232448) return split_rowgemm_pair_launch<256, 3, true>(g, st);
       if (split_rowgemm_pair_smem(g, 256, 2, true) <= 232448) return split_rowgemm_pair_launch<256, 2, true>(g, st);
@@ -883,8 +882,9 @@ int launch_split_rowgemm(const TcGemm& g, cudaStream_t st) {
       return split_rowgemm_pair_launch<256, 2, false>(g, st);
     }
   }
-  static const bool narrow = getenv("PZ_SPLIT_NCOLS") && atoi(getenv("PZ_SPLIT_NCOLS")) == 128;
-  if (g.Nout % 256 == 0 && !(narrow && !g.Ymax)) return split_rowgemm_launch<256, 2>(g, st);
+  // the one-CTA kernels: rows that tile only by 128 per weight set (pz_group_mlp_maxpool with B*N = 128 mod 256), and
+  // 128-column outputs with a tile-max epilogue
+  if (g.Nout % 256 == 0) return split_rowgemm_launch<256, 2>(g, st);
   return split_rowgemm_launch<128, 3>(g, st);
 }
 
@@ -908,13 +908,14 @@ __device__ __forceinline__ float4 ldg_nc_pinned(const float4* p) {
 // Producers (8 warps): P rows are fp32 in global memory; they are loaded one half-stage ahead into registers (fully
 // coalesced LDG.128, the row ids one TILE ahead), relu(P - Q) is formed in fp32, split into hi / lo and each plane is
 // written with one swizzled st.shared -- the operand is written once and never re-read by the producers.
-// PW: producer warps (8 or 16; 16 = twice the warps per scheduler to hide the latencies of the producer chain)
-template <int ROWS, int NST, int PW>
-__global__ void __launch_bounds__((5 + PW) * 32, 1) split_gather_kernel(const TcGemm g) {
+// (16 producer warps, twice the warps per scheduler to hide the latencies of the producer chain, measured slower: 0.242 vs
+// 0.229 ms)
+template <int ROWS, int NST>
+__global__ void __launch_bounds__(SG_THREADS, 1) split_gather_kernel(const TcGemm g) {
   extern __shared__ __align__(1024) uint8_t sgg_smem_raw[];
   const uint32_t smem_base = (smem_u32(sgg_smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_gen = sgg_smem_raw + (smem_base - smem_u32(sgg_smem_raw));
-  constexpr int EPI = 4, PROD_THREADS = PW * 32, THREADS = (5 + PW) * 32, RP = PW * 4;   // RP: rows per producer pass
+  constexpr int EPI = 4, PW = 8, PROD_THREADS = PW * 32, THREADS = SG_THREADS, RP = PW * 4;   // RP: rows per producer pass
   constexpr uint32_t X_PLANE = ROWS * 128, STAGE = 2 * X_PLANE;
   const int kblocks = g.K / KB;
   const uint32_t w_plane = (uint32_t)kblocks * TILE16K;          // resident: [W hi kblocks tiles][W lo kblocks tiles]
@@ -1402,8 +1403,8 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(SG_THREADS, 1) split
   }
 }
 
-template <int NST>
 static int split_gather_pair_launch(const TcGemm& g, cudaStream_t st) {
+  constexpr int NST = 3;
   const int kblocks = g.K / KB;
   const size_t smem = 2 * (size_t)kblocks * TILE16K + (size_t)NST * 2 * 128 * 128 + 8 * (3 * NST + 4) + 32 +
                       2 * (size_t)4 * 64 * sizeof(float);
@@ -1420,13 +1421,13 @@ static int split_gather_pair_launch(const TcGemm& g, cudaStream_t st) {
   return 0;
 }
 
-template <int ROWS, int NST, int PW>
+template <int ROWS, int NST>
 static int split_gather_launch(const TcGemm& g, cudaStream_t st) {
   const int kblocks = g.K / KB;
   const size_t smem = 1024 + 2 * (size_t)kblocks * TILE16K + (size_t)NST * 2 * ROWS * 128 + 8 * (2 * NST + 4) + 32 +
                       2 * (size_t)(ROWS / 32) * 64 * sizeof(float);
   PZ_REQUIRE(smem <= 232448, PZ_ERR_UNSUPPORTED, "split_gather: needs %zu B of shared memory (K=%d)", smem, g.K);
-  auto kern = split_gather_kernel<ROWS, NST, PW>;
+  auto kern = split_gather_kernel<ROWS, NST>;
   PZ_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int nsets = (g.rows_per_wset > 0 && g.M > g.rows_per_wset) ? 2 : 1;
   const int nparts = nsets * (g.Nout / 128);
@@ -1434,7 +1435,7 @@ static int split_gather_launch(const TcGemm& g, cudaStream_t st) {
   int per = kNumSMs / nparts;
   if (per > tiles_per_part) per = tiles_per_part;
   if (per < 1) per = 1;
-  PZ_CUDA(launch_pdl(kern, dim3(per * nparts), dim3((5 + PW) * 32), smem, st, g));
+  PZ_CUDA(launch_pdl(kern, dim3(per * nparts), dim3(SG_THREADS), smem, st, g));
   PZ_LAUNCH_CHECK();
   return 0;
 }
@@ -1453,17 +1454,15 @@ int launch_split_gather(const TcGemm& g, cudaStream_t st) {
     PZ_REQUIRE(g.W[1] && g.Wlo[1] && g.M == 2 * g.rows_per_wset, PZ_ERR_ARG, "split_gather: two weight sets need M == 2*rows_per_wset");
   if (g.K <= 128) {
     PZ_REQUIRE(g.M % (256 * nsets) == 0, PZ_ERR_UNSUPPORTED, "split_gather: M=%d must be a multiple of %d", g.M, 256 * nsets);
-    static const bool pw16 = getenv("PZ_SG_PW16") != nullptr;   // A/B hook: 16 producer warps (measured slower: 0.242 vs 0.229 ms)
-    // (128-row stages, three or four deep, measured slower as well: 0.258 / 0.262 ms)
-    return pw16 ? split_gather_launch<256, 2, 16>(g, st) : split_gather_launch<256, 2, 8>(g, st);
+    // (128-row stages, three or four deep, measured slower: 0.258 / 0.262 ms)
+    return split_gather_launch<256, 2>(g, st);
   }
   PZ_REQUIRE(g.M % (128 * nsets) == 0, PZ_ERR_UNSUPPORTED, "split_gather: M=%d must be a multiple of %d", g.M, 128 * nsets);
-  // 256 output channels: one CTA pair per tile (cta_group::2), every gathered row formed once for both channel blocks
-  static const bool no_pair = getenv("PZ_SG_NO_PAIR") != nullptr;   // A/B hook
-  static const int pair_nst = getenv("PZ_SG_PAIR_NST") ? atoi(getenv("PZ_SG_PAIR_NST")) : 3;
-  if (g.Nout == 256 && g.M % (256 * nsets) == 0 && !no_pair)
-    return pair_nst == 2 ? split_gather_pair_launch<2>(g, st) : split_gather_pair_launch<3>(g, st);
-  return split_gather_launch<128, 2, 8>(g, st);
+  // 256 output channels on rows that tile by 256 per weight set: one CTA pair per tile (cta_group::2), every gathered row
+  // formed once for both channel blocks
+  if (g.Nout == 256 && g.M % (256 * nsets) == 0) return split_gather_pair_launch(g, st);
+  // any other Nout (C1 = 256 with C2 = 128) or rows that tile only by 128: one CTA per 128-row tile and channel block
+  return split_gather_launch<128, 2>(g, st);
 }
 
 // fp32 [rows, cols] (row stride ldi) -> fp16 hi / lo planes (row stride ldo)

@@ -351,8 +351,10 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const TcGemm g) {
             }
           }
         }
+        // the store epilogue is compiled out of the gather kernels (launch_tc_gemm_gather allows the group max only):
+        // it would cost them registers, and at the 128-register cap a spill
 #pragma unroll 1
-        for (int c32 = c_begin; c32 < ROWS / 32 && g.epi == 0; c32 += c_step) {
+        for (int c32 = c_begin; c32 < ROWS / 32 && !GATHER && g.epi == 0; c32 += c_step) {
           float v[32];
           tmem_ld32(t_addr + c32 * 32, v);
           if (g.epi == 0) {
@@ -382,22 +384,6 @@ __global__ void __launch_bounds__(THREADS, 1) tc_gemm_kernel(const TcGemm g) {
               if (g.Rf || g.Rb) x += res[i];
               v[i] = x;
               tmax = fmaxf(tmax, x);
-            }
-            if (g.YT && (cht * NCHB + chb) * 128 >= g.t_ch_begin) {
-              // transposed bf16 store: this thread's 32 consecutive rows are contiguous in YT
-              __nv_bfloat16* dst = g.YT + ((size_t)rt * (g.Nout - g.t_ch_begin) + (ch - g.t_ch_begin)) * ROWS + c32 * 32;
-#pragma unroll
-              for (int q4 = 0; q4 < 4; ++q4) {
-                uint4 pk;
-                __nv_bfloat162 h0 = __floats2bfloat162_rn(v[q4 * 8 + 0], v[q4 * 8 + 1]);
-                __nv_bfloat162 h1 = __floats2bfloat162_rn(v[q4 * 8 + 2], v[q4 * 8 + 3]);
-                __nv_bfloat162 h2 = __floats2bfloat162_rn(v[q4 * 8 + 4], v[q4 * 8 + 5]);
-                __nv_bfloat162 h3 = __floats2bfloat162_rn(v[q4 * 8 + 6], v[q4 * 8 + 7]);
-                pk.x = *reinterpret_cast<uint32_t*>(&h0); pk.y = *reinterpret_cast<uint32_t*>(&h1);
-                pk.z = *reinterpret_cast<uint32_t*>(&h2); pk.w = *reinterpret_cast<uint32_t*>(&h3);
-                reinterpret_cast<uint4*>(dst)[q4] = pk;
-              }
-              continue;
             }
             if (g.Yf) {
               float* yp = g.Yf + rbase * g.ldyf + ch;
@@ -466,7 +452,7 @@ static int launch_tc_gemm_gather(const TcGemm& g, cudaStream_t st, int nsets) {
 }
 
 int launch_tc_gemm(const TcGemm& g, cudaStream_t st) {
-  PZ_REQUIRE(g.W[0] && g.X && (g.Yf || g.Yb || g.YT), PZ_ERR_ARG, "tc_gemm: null operand");
+  PZ_REQUIRE(g.W[0] && g.X && (g.Yf || g.Yb), PZ_ERR_ARG, "tc_gemm: null operand");
   PZ_REQUIRE(g.M > 0 && g.Nout > 0 && g.K > 0, PZ_ERR_ARG, "tc_gemm: bad shape");
   PZ_REQUIRE(g.K % 64 == 0 && g.Nout % 128 == 0 && g.ldx % 8 == 0 && g.ldw % 8 == 0, PZ_ERR_UNSUPPORTED,
              "tc_gemm: needs K %% 64 == 0, Nout %% 128 == 0 and 16-byte aligned rows (K=%d Nout=%d)", g.K, g.Nout);

@@ -372,10 +372,9 @@ extern "C" int pz_gemm_tf32_batched(int a_mn_major, int b_mn_major, int M, int N
              bias_or_null, relu, mask_or_null, ldmask, accumulate, batch, strideA, strideB, strideC};
   // weights-resident mode: forward / data-gradient GEMMs whose B operand (one 128-column tile, all of K) fits in 128 KB
   // and that have enough row tiles to amortise loading it once per CTA
-  static const bool no_bres = getenv("PZ_TF32_NO_BRES") != nullptr;      // tuning hook: force the streaming kernel
   // (measured: 17 % faster than streaming for the 128-wide layers, 4.7 TB/s on compulsory bytes; for N = 256 the A
   // operand would be read once per column tile, which costs more than the weights it saves)
-  if (!no_bres && batch == 1 && splitk == 1 && N == 128 && M / 128 >= 4 * kNumSMs) {
+  if (batch == 1 && splitk == 1 && N == 128 && M / 128 >= 4 * kNumSMs) {
     if (K <= 128) return tf32_launch<128, 8, true>(g, as_stream(stream));     // 64 KB of weights + 8 x 16 KB of A in flight
     if (K <= 256) return tf32_launch<128, 4, true>(g, as_stream(stream));     // 128 KB + 4 x 16 KB
   }

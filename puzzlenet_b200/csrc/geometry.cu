@@ -288,26 +288,15 @@ static int fps_grid_launch(const float* xyz, int B, int N, const int64_t* start,
 
 int launch_fps(const float* xyz, int B, int N, const int64_t* start, int S, int64_t* out64,
                int* out_rows32, float* new_xyz, cudaStream_t st) {
-  if (const char* e = getenv("PZ_FPS_T")) {   // tuning experiment hook: threads per cloud for N <= 1024
-    const int T = atoi(e);
-    if (N <= 1024) {
-      if (T == 64) return fps_launch_t<16, 64>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
-      if (T == 128) return fps_launch_t<8, 128>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
-      if (T == 512) return fps_launch_t<2, 512>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
-      if (T == 1024) return fps_launch_t<1, 1024>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
-    }
-  }
-  static const bool no_grid = getenv("PZ_FPS_NO_GRID") != nullptr;         // A/B hook
-  if (N > 4096 && N <= 14336 && S <= 8192 && !no_grid) return fps_grid_launch(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
+  if (N > 4096 && N <= 14336 && S <= 8192) return fps_grid_launch(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
   // large clouds, few enough of them that two CTAs per cloud still run in one wave: the 2-CTA cluster variant
-  static const bool no_cluster = getenv("PZ_FPS_NO_CLUSTER") != nullptr;   // A/B hook
-  if (N > 4096 && 4 * B <= kNumSMs && !no_cluster) {     // a handful of large clouds (assembly, dataset): 4 CTAs per cloud
+  if (N > 4096 && 4 * B <= kNumSMs) {     // a handful of large clouds (assembly, dataset): 4 CTAs per cloud
     const int part = (N + 3) / 4;
     if (part <= 2 * 1024) return fps_launch_cluster<2, 4>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
     if (part <= 3 * 1024) return fps_launch_cluster<3, 4>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
     if (part <= 4 * 1024) return fps_launch_cluster<4, 4>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
   }
-  if (N > 4096 && 2 * B <= kNumSMs && !no_cluster) {
+  if (N > 4096 && 2 * B <= kNumSMs) {
     const int part = (N + 1) / 2;
     if (part <= 3 * 1024) return fps_launch_cluster<3, 2>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
     if (part <= 4 * 1024) return fps_launch_cluster<4, 2>(xyz, B, N, start, S, out64, out_rows32, new_xyz, st);
@@ -1154,8 +1143,7 @@ int launch_knn(const float* query, const float* xyz, int B, int S, int N, int K,
   PZ_REQUIRE(K >= 1 && K <= 32, PZ_ERR_UNSUPPORTED, "pz_knn: K=%d not in [1,32]", K);
   PZ_REQUIRE(N >= K, PZ_ERR_UNSUPPORTED, "pz_knn: N=%d < K=%d", N, K);
   PZ_REQUIRE(B <= 65535, PZ_ERR_UNSUPPORTED, "pz_knn: B=%d > 65535", B);
-  static const bool brute = getenv("PZ_KNN_BRUTE") != nullptr;   // A/B hook: the exhaustive scan for every N
-  if (!brute && N > KNN_CHUNK && N <= KG_MAXN && S >= 64) {        // large clouds (the dataset shape): block pruning
+  if (N > KNN_CHUNK && N <= KG_MAXN && S >= 64) {        // large clouds (the dataset shape): block pruning
     const int nblk = (N + KG_BLK - 1) / KG_BLK, npad = nblk * KG_BLK;
     const size_t smem = (size_t)3 * (npad + 4) * sizeof(float) + (size_t)npad * sizeof(unsigned short) + (size_t)6 * nblk * sizeof(float) +
                         KG_CELLS * sizeof(int) + KG_WARPS * 6 * sizeof(unsigned) + (size_t)KG_WARPS * 64 * sizeof(uint2);

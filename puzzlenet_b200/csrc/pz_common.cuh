@@ -40,7 +40,7 @@ int fail(int code, const char* fmt, ...);
 // fetches overlap the predecessor's tail); every such kernel calls pdl_enter() BEFORE its first access to global memory:
 // it blocks until the predecessor grid has completed and its writes are visible, and only then lets the successor in, so
 // at most two grids of the chain are in flight and a resident CTA never runs ahead of anything but its direct predecessor.
-// Only kernels that call pdl_enter() may be launched with launch_pdl().  PZ_NO_PDL=1: plain launches (A/B hook).
+// Only kernels that call pdl_enter() may be launched with launch_pdl().
 // Measured (B=64 split forward, 1 B200): eager launches on one stream 1.59 -> 1.51 ms per forward.  NOT used under stream
 // capture: in the 4-stream graph schedule the early-resident CTAs of one stream's next kernel hold SMs that another
 // stream's ready kernel would have used (1.37 -> 1.52 ms per step), nor with the stage recorder on (an event record between
@@ -53,8 +53,7 @@ __device__ __forceinline__ void pdl_enter() {
   pdl_trigger();
 }
 #endif
-bool pdl_enabled();                   // capi.cu: not disabled by PZ_NO_PDL
-bool pdl_for_stream(cudaStream_t st);   // capi.cu: pdl_enabled(), the stage recorder is off and `st` is not capturing
+bool pdl_for_stream(cudaStream_t st);   // capi.cu: the stage recorder is off and `st` is not capturing
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
@@ -182,8 +181,7 @@ struct TcGemm {
   int rb_rows = 0, rb_ld = 0;
   float* Ymax = nullptr;                           // epi 0: also Ymax[tile * ldmax + ch] = max over the tile's rows
   int ldmax = 0;
-  __nv_bfloat16* YT = nullptr;                     // epi 0: channels >= t_ch_begin are stored TRANSPOSED per row tile:
-  int t_ch_begin = 0;                              //   YT[(tile*(Nout-t_ch_begin) + ch-t_ch_begin)*ROWS + row_in_tile]
+  __nv_bfloat16* YT = nullptr;                     // split row GEMM: output stored TRANSPOSED per block of t_rows rows
   const float* xyz = nullptr;                      // epi 0 only: y += W1x[ch,0:3] . xyz[row]  (layer 1 of a grouped MLP)
   const float* W1x[2] = {nullptr, nullptr};
   int ldw1x = 0;
@@ -247,9 +245,6 @@ int launch_seg_pairs_split(const HeadMlp3& pre_f, const HeadMlp3& pre_r, const H
                            bool reuse_images, void* img, const float* local_fpc, const float* tilemax_mrpc,
                            const int64_t* pairs, int n, float* de_fpcb, cudaStream_t st);
 int launch_tc_rowgemm(const TcGemm& g, cudaStream_t st);   // gemm_tc_rows.cu: same struct, row-major store epilogue
-// attention_tc.cu: per cloud  r = x - softmax(q k^T / sqrt(64)) v   on tcgen05 (L == 256, d_k == 64, C == 256)
-int launch_attention_tc(const __nv_bfloat16* qk, const __nv_bfloat16* vT, const __nv_bfloat16* x, int ldx, int clouds,
-                        __nv_bfloat16* r, float* attn, int attn_mode, cudaStream_t st);
 // attention_layer_tc.cu: a stack of 1-4 offset-attention layers per cloud in ONE launch (per layer: projections, softmax,
 // P v, out-proj, residuals); layer l + 1 reads the output of layer l
 struct AttnLayerTc {
@@ -268,7 +263,8 @@ struct AttnLayerTc {
   float* yf = nullptr;                    // optional fp32 copy, layer l at yf + l * yf_layer_stride
   int ldyf = 0;
   size_t yf_layer_stride = 0;
-  float* attn = nullptr;                  // attention map accumulation (see attention_tc_kernel), mode per layer
+  float* attn = nullptr;                  // attention map accumulation, mode per layer: 0 none, 1 store, 2 add,
+                                          // 3 (sum + map) / 4 (the mean of the four layers' maps)
   int attn_mode[4] = {0, 0, 0, 0};
   long long* prof = nullptr;              // pz_profile_attention_timeline
 };

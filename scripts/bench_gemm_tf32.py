@@ -1,5 +1,5 @@
 """Microbenchmark of pz_gemm_tf32 / pz_sgemm on the GEMM shapes of one training step (64 pairs per GPU).
-    python scripts/bench_gemm_tf32.py         (PZ_TF32_NO_BRES=1 forces the streaming kernel)"""
+    python scripts/bench_gemm_tf32.py"""
 import json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -47,7 +47,7 @@ def main():
         rows.append({"gemm": name, "tf32_ms": round(ms, 4), "tf32_tflops": round(2.0 * M * N * K / ms / 1e9, 1),
                      "compulsory_GBps": round(gb / ms * 1e3, 1), "sgemm_fp32_ms": round(ms32, 4)})
         del A, B, C
-    print(json.dumps({"bres_disabled": os.environ.get("PZ_TF32_NO_BRES") is not None, "rows": rows}, indent=1))
+    print(json.dumps({"rows": rows}, indent=1))
 
 
 if __name__ == "__main__":

@@ -2,11 +2,8 @@
 block against the CPU oracle, at the fp32 tolerance of north_star (1e-4 relative; measured ~1e-6).  The kernels:
 split_rowgemm_pair_kernel / split_gather_kernel / split_gather_pair_kernel (gemm_split.cu: CTA pairs, TMA),
 attention_split_kernel (attention_split.cu), head_*_split_kernel (heads_split.cu), stem_tc_kernel<true> (encoder.cu); the
-one-CTA fallbacks (split_rowgemm_kernel, the 128-row split_gather_kernel, the FFMA stem) through their A/B hooks.
+one-CTA kernels (split_rowgemm_kernel, the 128-row split_gather_kernel) through the group-MLP shapes that reach them.
 End to end at B=64: tests/test_gpu_b64_parity.py."""
-import os
-import subprocess
-import sys
 import numpy as np
 import pytest
 import torch
@@ -40,24 +37,42 @@ def test_layer_attention_split(state_dict, B):
     np.testing.assert_allclose(a.sum(-1).cpu().numpy(), 1.0, atol=1e-5)
 
 
-@pytest.mark.parametrize("stage", [1, 2])
-def test_group_mlp_maxpool_split(state_dict, stage):
+_STAGE1, _STAGE2 = ("Encoder.mlp3", "Encoder.mlp4"), ("Encoder2.mlp5", "Encoder2.mlp6")
+
+
+@pytest.mark.parametrize("layers, B, N, S, seed", [
+    pytest.param(_STAGE1, 2, 1024, 128, 3, id="1"),
+    pytest.param(_STAGE2, 2, 512, 64, 4, id="2"),
+    # B*N = 384 rows tile by 128 but not by 256: the one-CTA row GEMMs split_rowgemm_kernel<128,3> (C1 = 128) and
+    # split_rowgemm_kernel<256,2> (C1 = 256)
+    pytest.param(_STAGE1, 3, 128, 32, 5, id="1-rows128"),
+    pytest.param(_STAGE2, 3, 128, 32, 6, id="2-rows128"),
+    # C1 = 256 with C2 = 128 (no encoder layer has it, so seeded random weights): the 128-row split_gather_kernel
+    pytest.param(None, 2, 512, 64, 7, id="c1_256-c2_128"),
+])
+def test_group_mlp_maxpool_split(state_dict, layers, B, N, S, seed):
     """Layer 1 over source points (row GEMM, fp32 P), fp32 Q, gathered relu(P - Q) formed in registers, three-MMA layer 2,
-    max over the 32 neighbours: both stage shapes of the encoder (67->128->128 on 1024 points, 131->256->256 on 512)."""
+    max over the 32 neighbours: both stage shapes of the encoder (67->128->128 on 1024 points, 131->256->256 on 512) and
+    the shapes that reach the one-CTA kernels."""
     from puzzlenet_b200 import pointnet_util as pu
-    g = torch.Generator().manual_seed(2 + stage)
-    N, D, S = (1024, 64, 128) if stage == 1 else (512, 128, 64)
-    la, lb = ("Encoder.mlp3", "Encoder.mlp4") if stage == 1 else ("Encoder2.mlp5", "Encoder2.mlp6")
-    xyz = torch.rand(2, N, 3, generator=g) - 0.5
-    feat = torch.randn(2, N, D, generator=g)
+    g = torch.Generator().manual_seed(seed)
+    sd = state_dict
+    if layers is None:
+        sd = {"a.weight": torch.randn(256, 3 + 64, generator=g) / 67 ** 0.5, "a.bias": torch.randn(256, generator=g) / 67 ** 0.5,
+              "b.weight": torch.randn(128, 256, generator=g) / 16, "b.bias": torch.randn(128, generator=g) / 16}
+        layers = ("a", "b")
+    la, lb = layers
+    D = sd[la + ".weight"].shape[1] - 3
+    xyz = torch.rand(B, N, 3, generator=g) - 0.5
+    feat = torch.randn(B, N, D, generator=g)
     torch.manual_seed(8)
     nx, npts, _, _, idx = po.sample_and_group(S, 0, 32, xyz, feat, knn=True, return_idx=True)
-    ref = torch.relu(po._lin(state_dict, lb, torch.relu(po._lin(state_dict, la, npts)))).max(-2).values
+    ref = torch.relu(po._lin(sd, lb, torch.relu(po._lin(sd, la, npts)))).max(-2).values
     got = pu.group_mlp_maxpool(xyz.to(DEV), feat.to(DEV), nx.to(DEV), idx.to(DEV),
-                               state_dict[la + ".weight"].to(DEV), state_dict[la + ".bias"].to(DEV),
-                               state_dict[lb + ".weight"].to(DEV), state_dict[lb + ".bias"].to(DEV), precision=2)
+                               sd[la + ".weight"].to(DEV), sd[la + ".bias"].to(DEV),
+                               sd[lb + ".weight"].to(DEV), sd[lb + ".bias"].to(DEV), precision=2)
     errs = dict(rel=parity.rel(got, ref), elem=parity.rel_elem(got, ref))
-    print(f"split group MLP stage {stage}:", errs)
+    print(f"split group MLP {la} B={B} N={N}:", errs)
     assert got.shape == ref.shape and max(errs.values()) < TOL, errs
 
 
@@ -128,45 +143,3 @@ def test_split_chain_is_race_free_at_b64(cuda_model):
     finally:
         cuda_model.precision = "fp32"
     assert not torch.equal(first["a"][0], first["b"][0])
-
-
-_FALLBACK_SNIPPET = r"""
-import sys, types, torch
-sys.path.insert(0, %r)
-from oracle import parity, puzzle_oracle as po
-from puzzlenet_b200.model5_b import TouchedRegraster
-from puzzlenet_b200.weights import make_batch, synthetic_pairs, synthetic_state_dict
-sd = synthetic_state_dict(0)
-m = TouchedRegraster(types.SimpleNamespace(dataset="vase")); m.load_state_dict(sd, strict=True); m.to("cuda:0").eval()
-m.precision = "split"
-fpc, mrpc = synthetic_pairs(2, seed=64)
-other = synthetic_pairs(2, seed=65)
-torch.manual_seed(1234)
-ref = po.predict5(sd, fpc, mrpc)
-for graphs in (False, True):     # eager launches (programmatic dependent launch), then CUDA-graph replay
-    m.cuda_graphs = graphs
-    for i in range(3):           # back-to-back calls on one workspace: the last one is checked
-        pair = (fpc, mrpc) if i == 2 else other
-        torch.manual_seed(1234)
-        out, _, de_f, de_m = m.predict5(make_batch(pair[0].cuda(), pair[1].cuda()), 0)
-    torch.cuda.synchronize()
-    errs = [parity.rel(out, ref["out"]), parity.rel(de_f, ref["de_fpcb"]), parity.rel(de_m, ref["de_mrpcb"])]
-    rot, trans = parity.pose_errors(out, ref["out"])
-    print("FALLBACK", graphs, max(errs), rot, trans)
-    assert max(errs) < 1e-4 and rot < 0.01 and trans < 1e-4, (graphs, errs, rot, trans)
-"""
-
-
-@pytest.mark.parametrize("env", [{"PZ_SG_NO_PAIR": "1", "PZ_RG_NO_PAIR": "1", "PZ_STEM_FFMA": "1", "PZ_ATTN_NO_FUSE": "1"},
-                                 {"PZ_SG_PAIR_NST": "2", "PZ_SG_PW16": "1", "PZ_ATTN_NO_CHAIN": "1"},
-                                 {"PZ_NO_PDL": "1"}, {"PZ_SIDE_STREAM": "1", "PZ_ATTN_NO_PDL": "1"}, {"PZ_PDL_IN_GRAPHS": "1"}])
-def test_split_fallback_kernels(env):
-    """The A/B hooks select the one-CTA kernels (cp.async row GEMM, two-pass gather GEMM, FFMA stem) / the alternative
-    pipeline depths / plain launches instead of programmatic dependent launch / the geometry on a side stream / programmatic
-    edges inside captured graphs; they are read once per process, so the forward runs in a child process (three calls back to
-    back on one workspace, eager and as graph replays).  Same bounds as the default."""
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    r = subprocess.run([sys.executable, "-c", _FALLBACK_SNIPPET % root], env={**os.environ, **env}, capture_output=True,
-                       text=True, timeout=600)
-    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
-    assert "FALLBACK" in r.stdout
