@@ -132,7 +132,7 @@ int pz_plane_split(const float* pts, const int32_t* sizes_or_null, int P, int n_
 /* sample_and_group's grouping + the shared MLP + neighbourhood max-pool in one pass, never
  * materialising [B,S,K,3+D]: model5_b.py:449-454 / :456-461 with pointnet_util.py:123-130.
  *   out[b,s,:] = max_k relu(W2 relu(W1 [xyz[j]-new_xyz[b,s] ; feat[j]] + b1) + b2),  j = knn[b,s,k]
- * W1 [C1,3+D], W2 [C2,C1] row-major (nn.Linear layout), K must be 32.
+ * W1 [C1,3+D], W2 [C2,C1] row-major (nn.Linear layout), K must be 32; B*S*K and B*N at most INT_MAX.
  * workspace: pz_group_mlp_workspace_bytes(B,N,D,S,K,C1,C2). */
 size_t pz_group_mlp_workspace_bytes(int B, int N, int D, int S, int K, int C1, int C2);
 int pz_group_mlp_maxpool(const float* xyz, const float* feat, const float* new_xyz,
@@ -207,9 +207,15 @@ typedef struct PzEncoderOutputs {
   float* att_cat;   /* [E*B,256,1280]  cat(att1..att4, f2f) (model5_b.py:467,472) */
 } PzEncoderOutputs;
 
+/* Clouds per pz_encoder_forward call (E*B) and per pz_predict5 call (2B), in every precision: the kNN launches and the
+ * fp32 attention put one cloud per grid row.  The test suite runs calls of up to 8190 clouds (pz_encode_pieces with
+ * PZ_MAX_PIECES pieces, whose front half is pz_predict5's with B = P) and pz_predict5 up to B = 256. */
+#define PZ_MAX_CLOUDS 65535
+
 /* E encoders (different weight sets) over E*B clouds in one pass: cloud c uses weights[c / B].
  * xyz [E*B,1024,3]; start1 [E*B], start2 [E*B] = FPS start indices of stage 1 (in [0,1024)) and
- * stage 2 (in [0,512)).  Eval-mode BatchNorm (running statistics).  E in {1,2}. */
+ * stage 2 (in [0,512)).  Eval-mode BatchNorm (running statistics).  E in {1,2}.
+ * Supported: 1 <= E*B <= PZ_MAX_CLOUDS (PZ_ERR_UNSUPPORTED otherwise, before any launch). */
 size_t pz_encoder_workspace_bytes(int E, int B);
 int pz_encoder_forward(const PzEncoderWeights* weights_host, int E, int B, const float* xyz,
                        const int64_t* start1, const int64_t* start2, int precision,
@@ -230,7 +236,8 @@ typedef struct PzHeadWeights {
  * (Encoder stage 1, Encoder stage 2, Encoder2 stage 1, Encoder2 stage 2; SURVEY.md App. A).
  * out6 [B,6]; de_fpcb, de_mrpcb [B,2,1024].  flags & PZ_FLAG_NEED additionally fills x2_* [B,256,3] and
  * attention_* [B,256,256] (may be null otherwise).  Reproduces the reference's use of the mrpc
- * global feature for both boundary heads (model5_b.py:741-744). */
+ * global feature for both boundary heads (model5_b.py:741-744).
+ * Supported: 1 <= B <= PZ_MAX_CLOUDS / 2 = 32767 (PZ_ERR_UNSUPPORTED otherwise, before any launch). */
 size_t pz_predict5_workspace_bytes(int B);
 int pz_predict5(const PzEncoderWeights* enc_host /*[2]*/, const PzHeadWeights* heads_host,
                 const float* fpc, const float* mrpc, int B, const int64_t* starts, int precision,

@@ -6,6 +6,7 @@
 // every launch covers 128 clouds at B=64 instead of 64 -- FPS, the latency-bound stage, then
 // occupies 128 of the 148 SMs.
 
+#include <climits>
 #include <functional>
 
 #include <cuda_fp16.h>
@@ -1286,6 +1287,8 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
                                 bool reuse_pack, cudaStream_t st) {
   PZ_REQUIRE(E == 1 || E == 2, PZ_ERR_ARG, "encoder: E must be 1 or 2 (got %d)", E);
   PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "encoder: B must be >= 1");
+  PZ_REQUIRE((long long)E * B <= PZ_MAX_CLOUDS, PZ_ERR_UNSUPPORTED, "encoder: E*B = %lld clouds > %d", (long long)E * B,
+             PZ_MAX_CLOUDS);
   PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
              "encoder: unknown precision %d", precision);
   for (int e = 0; e < E; ++e)
@@ -1588,6 +1591,7 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
   PZ_REQUIRE(enc_host && heads_host && fpc && mrpc && starts && out6 && de_fpcb && de_mrpcb, PZ_ERR_ARG,
              "pz_predict5: null pointer");
   PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "pz_predict5: B must be >= 1");
+  PZ_REQUIRE(B <= PZ_MAX_CLOUDS / 2, PZ_ERR_UNSUPPORTED, "pz_predict5: B = %d > %d (2B clouds)", B, PZ_MAX_CLOUDS / 2);
   const int need = flags & PZ_FLAG_NEED;
   const bool reuse_pack = (flags & PZ_FLAG_REUSE_PACKS) != 0;
   if (need)
@@ -1932,6 +1936,10 @@ extern "C" int pz_group_mlp_maxpool(const float* xyz, const float* feat, const f
   PZ_REQUIRE(K == 32, PZ_ERR_UNSUPPORTED, "pz_group_mlp_maxpool: K must be 32 (got %d)", K);
   PZ_REQUIRE(C1 <= 256, PZ_ERR_UNSUPPORTED, "pz_group_mlp_maxpool: C1 must be <= 256 (got %d)", C1);
   PZ_REQUIRE(((size_t)B * S * K) % 128 == 0, PZ_ERR_UNSUPPORTED, "pz_group_mlp_maxpool: B*S must be a multiple of 4");
+  // grouped rows (GEMM M) and source-point row ids (B*N) are 32-bit ints on the device
+  PZ_REQUIRE((size_t)B * S * K <= INT_MAX && (size_t)B * N <= INT_MAX, PZ_ERR_UNSUPPORTED,
+             "pz_group_mlp_maxpool: B*S*K = %zu and B*N = %zu must not exceed %d", (size_t)B * S * K, (size_t)B * N,
+             INT_MAX);
   PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
              "pz_group_mlp_maxpool: unknown precision %d", precision);
   cudaStream_t st = as_stream(stream);

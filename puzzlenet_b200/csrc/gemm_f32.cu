@@ -41,7 +41,10 @@ __global__ void __launch_bounds__(GT, 2) gemm_f32_kernel(GemmF32 g) {
 
   const int t = threadIdx.x;
   const int tx = t & 15, ty = t >> 4;
-  const int m0 = blockIdx.y * BM, n0 = blockIdx.x * BN;
+  // (row tile, column tile) on the 1-D grid, column tile fastest: neighbouring CTAs share the rows of A in L2
+  const int ntn = (g.N + BN - 1) / BN;
+  const int mt = blockIdx.x / ntn;
+  const int m0 = mt * BM, n0 = (blockIdx.x - mt * ntn) * BN;
   const int wset = g.rows_per_wset > 0 ? m0 / g.rows_per_wset : 0;
   // split-K: CTA z handles k in [z*ksplit, (z+1)*ksplit) and stores raw partial sums to Y + z*M*ldy
   const int kbeg = g.ksplit > 0 ? blockIdx.z * g.ksplit : 0;
@@ -257,7 +260,8 @@ static int gemm_dispatch_vec(const GemmF32& g, cudaStream_t st) {
   const bool vec_a = (g.K % 8 == 0) && (g.lda % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.A) & 15) == 0);
   bool vec_w = (g.K % 8 == 0) && (g.ldw % 4 == 0) && ((reinterpret_cast<uintptr_t>(g.W[0]) & 15) == 0);
   if (g.W[1]) vec_w = vec_w && ((reinterpret_cast<uintptr_t>(g.W[1]) & 15) == 0);
-  dim3 grid((g.N + BN - 1) / BN, (g.M + BM - 1) / BM, g.ksplit > 0 ? (g.K + g.ksplit - 1) / g.ksplit : 1);
+  const long long tiles = ((long long)g.M + BM - 1) / BM * ((g.N + BN - 1) / BN);   // <= 2^31 - 1: launch_gemm_f32
+  dim3 grid((unsigned)tiles, 1, g.ksplit > 0 ? (g.K + g.ksplit - 1) / g.ksplit : 1);
   if (vec_a && vec_w)
     gemm_f32_kernel<BN, AMODE, EPI, true, true><<<grid, GT, 0, st>>>(g);
   else if (vec_a)
@@ -273,7 +277,9 @@ static int gemm_dispatch_vec(const GemmF32& g, cudaStream_t st) {
 int launch_gemm_f32(const GemmF32& g, cudaStream_t st) {
   PZ_REQUIRE(g.A && g.W[0] && g.Y, PZ_ERR_ARG, "gemm_f32: null operand");
   PZ_REQUIRE(g.M > 0 && g.N > 0 && g.K > 0, PZ_ERR_ARG, "gemm_f32: bad shape %dx%dx%d", g.M, g.N, g.K);
-  PZ_REQUIRE((g.M + BM - 1) / BM <= 65535, PZ_ERR_UNSUPPORTED, "gemm_f32: M=%d too large", g.M);
+  const int bn = g.N > 64 ? 128 : 64;
+  PZ_REQUIRE(((long long)g.M + BM - 1) / BM * ((g.N + bn - 1) / bn) <= 0x7fffffff, PZ_ERR_UNSUPPORTED,
+             "gemm_f32: M=%d N=%d needs more than 2^31 - 1 tiles", g.M, g.N);
   if (g.rows_per_wset > 0)
     PZ_REQUIRE(g.rows_per_wset % BM == 0 && g.W[(g.M - 1) / g.rows_per_wset] != nullptr, PZ_ERR_ARG,
                "gemm_f32: weight sets must cover whole %d-row tiles", BM);
@@ -288,7 +294,7 @@ int launch_gemm_f32(const GemmF32& g, cudaStream_t st) {
   if (gather)
     PZ_REQUIRE(g.K <= 256 && g.xyz && g.centers && g.W1[0] && g.b1[0] && g.M % 32 == 0, PZ_ERR_ARG,
                "gemm_f32: gathered A needs K <= 256 and xyz/centers/W1/b1");
-  const bool wide = g.N > 64;
+  const bool wide = bn == 128;
   if (gather) {
     if (gmax) return wide ? gemm_dispatch_vec<128, A_GATHER, EPI_GROUPMAX>(g, st) : gemm_dispatch_vec<64, A_GATHER, EPI_GROUPMAX>(g, st);
     return wide ? gemm_dispatch_vec<128, A_GATHER, EPI_STORE>(g, st) : gemm_dispatch_vec<64, A_GATHER, EPI_STORE>(g, st);

@@ -38,7 +38,7 @@ def _assert_equal_and_within(got, ref, precision):
 
 
 @pytest.mark.parametrize("precision", PRECISIONS)
-@pytest.mark.parametrize("P", [5, 64])
+@pytest.mark.parametrize("P", [1, 5, 64])
 def test_diagonal_pairs_equal_predict5_bitwise(model, precision, P):
     from puzzlenet_b200.weights import make_batch
     model.precision = precision
