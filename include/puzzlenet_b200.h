@@ -42,7 +42,7 @@ typedef void* pz_stream_t; /* cudaStream_t */
 #define PZ_PREC_SPLIT 2 /* every operand as an fp16 hi/lo pair, three tcgen05 MMAs per product (hi*hi + hi*lo + lo*hi),
                          * fp32 accumulate: the tensor-core path that meets the fp32 tolerances (1e-4, 0.01 deg) */
 
-#define PZ_ABI_VERSION 6
+#define PZ_ABI_VERSION 7
 
 /* pz_predict5 flags */
 #define PZ_FLAG_NEED 1          /* also return x2 / attention of both clouds (predict5 need=True) */
@@ -286,6 +286,9 @@ int pz_predict_pairs(const PzHeadWeights* heads_host, const PzPieceEmbeddings* e
 
 /* se3.exp(x) -- se_math/se3.py:57-80.  twist [B,6] (omega, v) -> g [B,4,4]. */
 int pz_se3_exp(const float* twist, int B, float* g, pz_stream_t stream);
+/* Its backward: dtwist [B,6] = sum_e dg[b,e] * d g[b,e] / d twist[b,:] over the 12 non-constant entries (rows 0..2)
+ * of g; dg [B,4,4].  Same formulas as pz_se3_exp, Taylor branch for |omega| < 0.01 included.  B >= 1. */
+int pz_se3_exp_backward(const float* twist, const float* dg, int B, float* dtwist, pz_stream_t stream);
 
 /* ------------------------------------------------- losses / post-forward epilogue */
 
@@ -302,6 +305,8 @@ int pz_chamfer_grad(const float* x, const float* y, int B, int n, int m, const i
 
 /* TouchedRegraster.comp(g, igt) -- model5_b.py:1512-1519: mse(g.igt, I)*16 -> loss [1]. */
 int pz_comp(const float* g, const float* igt, int B, float* loss, pz_stream_t stream);
+/* Its backward: dg [B,4,4] = dloss[0] * d comp / d g (dloss is a device scalar).  B >= 1. */
+int pz_comp_backward(const float* g, const float* igt, int B, const float* dloss, float* dg, pz_stream_t stream);
 
 /* se3.transform(g, a) -- se_math/se3.py:110-120 for points stored [B,n,3]: out = R p + t. */
 int pz_se3_transform(const float* g, const float* pts, int B, int n, float* out, pz_stream_t stream);

@@ -16,7 +16,7 @@ LIB_PATH = os.path.join(_HERE, "lib", "libpuzzlenet_sm100.so")
 PZ_PREC_FP32 = 0
 PZ_PREC_BF16 = 1
 PZ_PREC_SPLIT = 2
-ABI_VERSION = 6
+ABI_VERSION = 7
 PZ_SCORE_COLS = 12
 PZ_FLAG_NEED = 1
 PZ_FLAG_REUSE_PACKS = 2
@@ -90,10 +90,12 @@ SIGNATURES = {
     "pz_predict_pairs": (C.c_int, [C.POINTER(PzHeadWeights), C.POINTER(PzPieceEmbeddings), C.c_int, c_i64p, C.c_int,
                                    C.c_int, C.c_int, c_f32p, c_f32p, c_f32p, C.c_void_p, C.c_size_t, c_stream]),
     "pz_se3_exp": (C.c_int, [c_f32p, C.c_int, c_f32p, c_stream]),
+    "pz_se3_exp_backward": (C.c_int, [c_f32p, c_f32p, C.c_int, c_f32p, c_stream]),
     "pz_chamfer": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, c_f32p, c_f32p, C.c_void_p, C.c_void_p, c_stream]),
     "pz_chamfer_grad": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, c_f32p, c_f32p,
                                   c_f32p, c_f32p, c_stream]),
     "pz_comp": (C.c_int, [c_f32p, c_f32p, C.c_int, c_f32p, c_stream]),
+    "pz_comp_backward": (C.c_int, [c_f32p, c_f32p, C.c_int, c_f32p, c_f32p, c_stream]),
     "pz_se3_transform": (C.c_int, [c_f32p, c_f32p, C.c_int, C.c_int, c_f32p, c_stream]),
     "pz_boundary_topk": (C.c_int, [c_f32p, C.c_int, C.c_int, C.c_int, c_i64p, c_f32p, c_stream]),
     "pz_topk": (C.c_int, [c_f32p, C.c_int, C.c_int, C.c_int, C.c_int, c_i64p, c_f32p, c_stream]),

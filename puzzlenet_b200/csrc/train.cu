@@ -10,6 +10,7 @@
 //   * pz_softmax_bwd    backward of scaled_dot_production's softmax (model5_b.py:67-75)
 //   * pz_cross_entropy  F.cross_entropy(logits [B,2,N], target [B,N]) forward + backward (model5_b.py:1063-1064)
 //   * pz_pose_grad      d loss / d twist through se3.exp + se3.transform (+ comp) (model5_b.py:947-967)
+//   * pz_se3_exp_backward, pz_comp_backward   the autograd backward of se3.exp and of comp on their own
 //   * pz_adam_step      torch.optim.Adam on one flat parameter buffer (model5_b.py:1453-1457)
 #include <math.h>
 
@@ -646,6 +647,43 @@ __global__ void __launch_bounds__(256) pose_grad_kernel(const float* __restrict_
   }
 }
 
+// se3.exp backward on its own (autograd of se3.exp): dtwist[b,:] = sum_e dg[b,e] dg_e/dtwist over the 12 entries of
+// rows 0..2 of g [B,4,4] (row 3 is constant).  One thread per item.
+__global__ void __launch_bounds__(128) se3_exp_bwd_kernel(const float* __restrict__ twist, const float* __restrict__ dg,
+                                                          int B, float* __restrict__ dtwist) {
+  const int b = blockIdx.x * 128 + threadIdx.x;
+  if (b >= B) return;
+  Dual g[12];
+  se3_exp_dual(twist + (size_t)b * 6, g);
+  const float* d = dg + (size_t)b * 16;
+  for (int i = 0; i < 6; ++i) {
+    float s = 0.f;
+    for (int e = 0; e < 12; ++e) s = fmaf(d[e], g[e].d[i], s);
+    dtwist[(size_t)b * 6 + i] = s;
+  }
+}
+
+// comp backward (the comp term of pose_grad_kernel on a [B,4,4] g): L = sum_{b,r,c} (A - I)^2 / B with A = g igt,
+// dg[b,r,k] = dloss * 2/B * sum_c (A - I)[r,c] igt[b,k,c].  One thread per entry of dg.
+__global__ void __launch_bounds__(256) comp_bwd_kernel(const float* __restrict__ g, const float* __restrict__ igt, int B,
+                                                       const float* __restrict__ dloss, float* __restrict__ dg) {
+  const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+  if (e >= 16LL * B) return;
+  const long long b = e >> 4;
+  const int r = (int)(e >> 2) & 3, k = (int)e & 3;
+  const float* G = g + b * 16 + r * 4;
+  const float* H = igt + b * 16;
+  float s = 0.f;
+  for (int c = 0; c < 4; ++c) {
+    float a = G[0] * H[c];
+    a = fmaf(G[1], H[4 + c], a);
+    a = fmaf(G[2], H[8 + c], a);
+    a = fmaf(G[3], H[12 + c], a);
+    s = fmaf(a - (r == c ? 1.f : 0.f), H[k * 4 + c], s);
+  }
+  dg[e] = 2.f * dloss[0] / (float)B * s;
+}
+
 // =============================================================================== Adam (torch.optim.Adam semantics)
 __global__ void __launch_bounds__(256) adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                                    float* __restrict__ v, long long n, float lr, float b1, float b2,
@@ -907,6 +945,23 @@ extern "C" int pz_pose_grad(const float* out6, const float* pts_or_null, const f
   PZ_REQUIRE((pts_or_null == nullptr) == (dpts_or_null == nullptr), PZ_ERR_ARG, "pz_pose_grad: pts and dpts go together");
   pose_grad_kernel<<<B, 256, 0, as_stream(stream)>>>(out6, pts_or_null, dpts_or_null, n, igt_or_null, comp_scale, B, beta,
                                                      dout6);
+  PZ_LAUNCH_CHECK();
+  return PZ_OK;
+}
+
+extern "C" int pz_se3_exp_backward(const float* twist, const float* dg, int B, float* dtwist, pz_stream_t stream) {
+  PZ_REQUIRE(twist && dg && dtwist, PZ_ERR_ARG, "pz_se3_exp_backward: null pointer");
+  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "pz_se3_exp_backward: B must be >= 1");
+  se3_exp_bwd_kernel<<<(unsigned)((B + 127) / 128), 128, 0, as_stream(stream)>>>(twist, dg, B, dtwist);
+  PZ_LAUNCH_CHECK();
+  return PZ_OK;
+}
+
+extern "C" int pz_comp_backward(const float* g, const float* igt, int B, const float* dloss, float* dg,
+                                pz_stream_t stream) {
+  PZ_REQUIRE(g && igt && dloss && dg, PZ_ERR_ARG, "pz_comp_backward: null pointer");
+  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "pz_comp_backward: B must be >= 1");
+  comp_bwd_kernel<<<(unsigned)((16LL * B + 255) / 256), 256, 0, as_stream(stream)>>>(g, igt, B, dloss, dg);
   PZ_LAUNCH_CHECK();
   return PZ_OK;
 }

@@ -1,8 +1,7 @@
 """Loss-side and post-forward operators of the reference model, on the CUDA library.
 
 * :func:`chamfer_loss`     -- ``TouchedRegraster.chamfer_loss`` model5_b.py:1495-1505 (differentiable)
-* :func:`comp`             -- ``TouchedRegraster.comp`` model5_b.py:1512-1519 (forward only here; training uses
-  the fused loss kernels of :mod:`puzzlenet_b200.training`)
+* :func:`comp`             -- ``TouchedRegraster.comp`` model5_b.py:1512-1519 (differentiable)
 * :func:`boundary_topk`    -- ``torch.topk(torch.softmax(l, 1)[:, 1, :], 128, 1)[1]`` model5_b.py:1323-1330
 * :func:`transform_points` -- ``se3.transform`` (se_math/se3.py:110-120) for ``[B,n,3]`` points
 * :func:`pair_score`       -- the whole post-forward part of ``test_step`` (model5_b.py:1314-1358) in one launch
@@ -72,14 +71,40 @@ def chamfer_loss(a: torch.Tensor, b: torch.Tensor):
     return d_x, d_y
 
 
-def comp(g: torch.Tensor, igt: torch.Tensor) -> torch.Tensor:
-    """model5_b.py:1512-1519: ``mse(g.matmul(igt), I) * 16`` -> 0-d tensor."""
-    g_, h_ = _f32(g).view(-1, 4, 4), _f32(igt).view(-1, 4, 4)
-    assert g_.shape == h_.shape
+def _comp_raw(g_, h_):
     loss = torch.empty(1, device=g_.device, dtype=torch.float32)
     with torch.cuda.device(g_.device):
         _lib.call("pz_comp", g_.data_ptr(), h_.data_ptr(), g_.shape[0], loss.data_ptr(), _lib.stream_ptr())
     return loss[0]
+
+
+class _CompFunction(torch.autograd.Function):
+    """gradient w.r.t. g only: igt is the ground truth (the reference's loss never differentiates it)"""
+
+    @staticmethod
+    def forward(ctx, g_, h_):
+        ctx.save_for_backward(g_, h_)
+        return _comp_raw(g_, h_)
+
+    @staticmethod
+    def backward(ctx, dloss):
+        g_, h_ = ctx.saved_tensors
+        dg = torch.empty_like(g_)
+        dloss = dloss.contiguous().float()
+        with torch.cuda.device(g_.device):
+            _lib.call("pz_comp_backward", g_.data_ptr(), h_.data_ptr(), g_.shape[0], dloss.data_ptr(), dg.data_ptr(),
+                      _lib.stream_ptr())
+        return dg, None
+
+
+def comp(g: torch.Tensor, igt: torch.Tensor) -> torch.Tensor:
+    """model5_b.py:1512-1519: ``mse(g.matmul(igt), I) * 16`` -> 0-d tensor; differentiable w.r.t. ``g`` when it
+    requires grad (``pz_comp_backward``)."""
+    g_, h_ = _f32(g).view(-1, 4, 4), _f32(igt).view(-1, 4, 4)
+    assert g_.shape == h_.shape
+    if g_.requires_grad:
+        return _CompFunction.apply(g_, h_)
+    return _comp_raw(g_, h_)
 
 
 def boundary_topk(logits: torch.Tensor, k: int = 128, return_prob: bool = False):

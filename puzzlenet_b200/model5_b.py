@@ -18,10 +18,12 @@ through ``libpuzzlenet_sm100.so`` (hand-written sm_100a kernels, C ABI in
 Deviations from the reference, all documented in DESIGN.md:
 * ``TouchedRegraster.forward`` delegates to ``predict5`` (the reference's ``forward`` calls the
   broken ``predict4``, SURVEY.md D2).
-* Training has no autograd graph: ``training_step`` runs forward, losses, the hand-written backward, the
-  gradient all-reduce and Adam itself (``puzzlenet_b200/training.py``; Lightning: manual optimization).
-  ``predict5(training=True)`` is the train-mode forward only; the ``predict6`` pretraining branch trains through
-  ``training_step(pretrain=True)`` (or ``current_epoch < C.pretrain_epochs`` under Lightning).
+* ``training_step`` runs forward, losses, the hand-written backward, the gradient all-reduce and Adam itself
+  (``puzzlenet_b200/training.py``; Lightning: manual optimization).  By default ``predict5(training=True)`` is the
+  train-mode forward without an autograd graph and ``predict6(training=True)`` raises; with the opt-in
+  ``differentiable = True`` both record a graph whose backward runs the same hand-written kernels
+  (``puzzlenet_b200/autograd.py``), so a custom loss trains with ``loss.backward()`` and any ``torch.optim``
+  optimizer.
 * The class derives from ``nn.Module`` when ``pytorch_lightning`` is not installed.
 """
 from __future__ import annotations
@@ -353,6 +355,7 @@ class TouchedRegraster(_Base):
         self._trainer_state = None
         self._weights_generation = 0  # bumped whenever the weights change behind torch's back (see _weights_key)
         self.cuda_graphs = False      # opt-in: replay one captured CUDA graph per forward (see _graph_replay)
+        self.differentiable = False   # opt-in: training=True forwards record an autograd graph (puzzlenet_b200/autograd.py)
         self.graph_static_outputs = False   # True: return the graph's own output buffers (overwritten by the next replay)
         self.max_graphs = 16          # captured graphs kept (one per batch size, need, precision, device, stream); LRU
 
@@ -497,25 +500,47 @@ class TouchedRegraster(_Base):
     def predict5(self, batch, batch_indic, need=False, training=False, starts=None):
         """model5_b.py:672-759.  ``starts`` (optional, not in the reference): int64 [4,B] FPS start
         indices in the reference's draw order; when omitted the four ``torch.randint`` draws are taken
-        from the CPU generator exactly as the reference does (SURVEY.md Appendix A)."""
+        from the CPU generator exactly as the reference does (SURVEY.md Appendix A).  ``training=True`` runs the
+        train-mode forward in the Trainer's precision; with ``differentiable`` set and grad mode on, its outputs
+        (``x2_*`` / ``attention_*`` too) are connected to autograd: the parameters and, when they require grad, the
+        clouds receive gradients."""
         if training:
-            # train-mode forward (model5_b.py:684-690: batch-statistics BatchNorm, running stats updated); fp32 only
+            # train-mode forward (model5_b.py:684-690: batch-statistics BatchNorm, running stats updated)
             _lib.require_cuda(batch[0], batch[1])
-            for mod in (self.Encoder, self.Encoder2, self.tfMLP, self.fpc_decoder, self.rpc_decoder):
-                mod.train()
-            r = self.trainer_state().predict5_train(batch[0], batch[1], starts)
+            self._train_mode()
+            if self.differentiable and torch.is_grad_enabled():
+                from .autograd import train_forward
+                out6, de_f, de_m, x2f, af, x2m, am = train_forward(self.trainer_state(), batch[0], batch[1], starts,
+                                                                   need)
+                r = (out6, [0], x2f, af, x2m, am, de_f, de_m)
+            else:
+                r = self.trainer_state().predict5_train(batch[0], batch[1], starts)
             return r if need else (r[0], r[0], r[6], r[7])
         return self._predict(batch, need, starts, shared=False)
+
+    def _train_mode(self):
+        for mod in (self.Encoder, self.Encoder2, self.tfMLP, self.fpc_decoder, self.rpc_decoder):
+            mod.train()
 
     def predict6(self, batch, batch_indic, need=False, training=False, pretrain=False, starts=None):
         """model5_b.py:612-668 -- the pretraining forward: BOTH clouds go through ``self.Encoder`` and only the pose
         is predicted.  ``pretrain=False`` reaches ``self.Decoder`` / ``self.mrpcbDecoder`` in the reference, which
-        its constructor does not create (AttributeError there); it raises here as well."""
-        if training:
-            raise NotImplementedError("puzzlenet_b200.predict6 is inference-only, like predict5")
+        its constructor does not create (AttributeError there); it raises here as well.  ``training=True`` needs
+        ``differentiable`` (the train-mode forward with an autograd graph, as in predict5; ``Encoder`` is applied
+        twice and its gradients from the two passes add)."""
+        if training and not self.differentiable:
+            raise NotImplementedError("puzzlenet_b200.predict6(training=True) needs model.differentiable = True; "
+                                      "otherwise the pretraining branch trains through training_step(pretrain=True)")
         if not pretrain:
             raise AttributeError("'TouchedRegraster' object has no attribute 'Decoder' (model5_b.py:661: predict6 "
                                  "only works with pretrain=True)")
+        if training:
+            _lib.require_cuda(batch[0], batch[1])
+            self._train_mode()
+            from .autograd import train_forward
+            out6, _, _, x2f, af, x2m, am = train_forward(self.trainer_state(), batch[0], batch[1], starts, need,
+                                                         pretrain=True)
+            return (out6, [0], x2f, af, x2m, am) if need else out6
         r = self._predict(batch, need, starts, shared=True)
         if not need:
             return r[0]

@@ -7,13 +7,37 @@ import torch
 from . import _lib
 
 
+def _exp_raw(x_: torch.Tensor) -> torch.Tensor:
+    g = torch.empty(x_.shape[0], 4, 4, device=x_.device, dtype=torch.float32)
+    with torch.cuda.device(x_.device):
+        _lib.call("pz_se3_exp", x_.data_ptr(), x_.shape[0], g.data_ptr(), _lib.stream_ptr())
+    return g
+
+
+class _ExpFunction(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x_):
+        ctx.save_for_backward(x_)
+        return _exp_raw(x_)
+
+    @staticmethod
+    def backward(ctx, dg):
+        x_, = ctx.saved_tensors
+        dx = torch.zeros_like(x_)
+        if x_.shape[0]:
+            dg = dg.contiguous().float()
+            with torch.cuda.device(x_.device):
+                _lib.call("pz_se3_exp_backward", x_.data_ptr(), dg.data_ptr(), x_.shape[0], dx.data_ptr(),
+                          _lib.stream_ptr())
+        return dx
+
+
 def exp(x: torch.Tensor) -> torch.Tensor:
-    """twist [*, 6] (omega first, v last) -> [*, 4, 4] on the GPU (one tiny kernel)."""
+    """twist [*, 6] (omega first, v last) -> [*, 4, 4] on the GPU (one tiny kernel); differentiable when ``x``
+    requires grad (``pz_se3_exp_backward``)."""
     _lib.require_cuda(x)
     x_ = x.reshape(-1, 6).contiguous().float()
-    g = torch.empty(x_.shape[0], 4, 4, device=x.device, dtype=torch.float32)
-    with torch.cuda.device(x.device):
-        _lib.call("pz_se3_exp", x_.data_ptr(), x_.shape[0], g.data_ptr(), _lib.stream_ptr())
+    g = _ExpFunction.apply(x_) if x_.requires_grad else _exp_raw(x_)
     return g.view(*x.shape[:-1], 4, 4)
 
 

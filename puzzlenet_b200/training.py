@@ -12,6 +12,7 @@ torch is used for memory, streams and the collective only -- no autograd, no tor
 """
 from __future__ import annotations
 
+import contextlib
 import math
 from typing import Dict, Optional
 
@@ -139,7 +140,8 @@ class _Flat:
         self.grads = torch.zeros(n_total, device=dev, dtype=torch.float32)
         self.exp_avg = torch.zeros(n_total, device=dev, dtype=torch.float32)
         self.exp_avg_sq = torch.zeros(n_total, device=dev, dtype=torch.float32)
-        self.grad_of: Dict[int, torch.Tensor] = {}
+        self.live = [p for _, p in live]
+        self.offsets = []
         self.segments: Dict[str, list] = {}          # gradient buckets: "Encoder", "Encoder2", "heads" -> [lo, hi)
         off = 0
         with torch.no_grad():
@@ -151,9 +153,14 @@ class _Flat:
                 lo_hi[1] = off + pad(n)
                 self.params[off:off + n].copy_(p.reshape(-1))
                 p.data = self.params[off:off + n].view_as(p)
-                self.grad_of[id(p)] = self.grads[off:off + n].view_as(p)
+                self.offsets.append(off)
                 off += pad(n)
         self.n = n_total
+        self.grad_of: Dict[int, torch.Tensor] = self.views(self.grads)
+
+    def views(self, grads: torch.Tensor) -> Dict[int, torch.Tensor]:
+        """id(parameter) -> its gradient as a view of the flat buffer ``grads`` (laid out like ``self.grads``)"""
+        return {id(p): grads[off:off + p.numel()].view_as(p) for p, off in zip(self.live, self.offsets)}
 
     def g(self, p):
         return self.grad_of[id(p)]
@@ -205,6 +212,7 @@ class Trainer:
         self._pending, self._reduced = [], set()
         self.dev = self.flat.params.device
         self._buf: Dict[str, torch.Tensor] = {}
+        self._grad_of = self.flat.grad_of          # where the backward writes parameter gradients (see _scope)
         self.sync_replicas()
 
     def sync_replicas(self, src: int = 0):
@@ -244,6 +252,22 @@ class Trainer:
             self._buf[name] = t
         return t
 
+    @contextlib.contextmanager
+    def _scope(self, store: Optional[Dict[str, torch.Tensor]] = None, grad_of: Optional[Dict[int, torch.Tensor]] = None):
+        """Run the forward / backward methods on another buffer namespace (``store``: a graph's own activations, which
+        later calls on this Trainer must not overwrite) and / or into other parameter-gradient views (``grad_of``, as
+        returned by ``_Flat.views``)."""
+        saved = self._buf, self._grad_of
+        self._buf = saved[0] if store is None else store
+        self._grad_of = saved[1] if grad_of is None else grad_of
+        try:
+            yield
+        finally:
+            self._buf, self._grad_of = saved
+
+    def _g(self, p):
+        return self._grad_of[id(p)]
+
     # -------------------------------------------------------------------------------------------- grouped layer 1
     def _group_layer1_forward(self, tag, lin, xyz, feat, D, centres, idx, B, N, S, out):
         """relu(lin([xyz_j - c_s ; feat_j])) for every (group, neighbour) WITHOUT the [B,S,K,3+D] tensor:
@@ -262,10 +286,11 @@ class Trainer:
         _lib.call("pz_gather_sub_relu", _p(P), _p(Q), _p(idx), B * S, KNN, S, N, C1, _p(out), _st())
         return dict(lin=lin, lin_f=lin_f, wx=wx, xyz=xyz, feat=feat, D=D, centres=centres, idx=idx, N=N, S=S, C1=C1)
 
-    def _group_layer1_backward(self, tag, st, B, d_pre, dfeat):
+    def _group_layer1_backward(self, tag, st, B, d_pre, dfeat, dxyz=None, dcentres=None):
         """d_pre [B*S*K, C1] = gradient w.r.t. the layer's pre-activation (ReLU-gated).  Adds the weight / bias
-        gradients of ``lin`` and accumulates d loss / d feat into ``dfeat`` [B*N, D]."""
-        G, lin, C1, D, N, S = self.flat.g, st["lin"], st["C1"], st["D"], st["N"], st["S"]
+        gradients of ``lin`` and accumulates d loss / d feat into ``dfeat`` [B*N, D]; with ``dxyz`` [B*N, 3] and
+        ``dcentres`` [B*S, 3] also d loss / d xyz_j and d loss / d c_s (accumulated into)."""
+        G, lin, C1, D, N, S = self._g, st["lin"], st["C1"], st["D"], st["N"], st["S"]
         dP, dQ = self.buf(tag + ".dP", B * N, C1), self.buf(tag + ".dQ", B * S, C1)
         dP.zero_()
         _lib.call("pz_group_scatter_grad", _p(d_pre), _p(st["idx"]), B * S, KNN, S, N, C1, _p(dP), _p(dQ), _st())
@@ -279,6 +304,9 @@ class Trainer:
         gw = G(lin.weight)                                                            # [C1, 3 + D]: add both column blocks
         axpby(C1, 3, 1.0, gwx, 3, 1.0, gw, 3 + D, gw, 3 + D)
         axpby(C1, D, 1.0, gwf, D, 1.0, gw[:, 3:], 3 + D, gw[:, 3:], 3 + D)
+        if dxyz is not None:                                                          # dxyz += dP W_x ; dc += dQ W_x
+            gemm(dP, st["wx"], dxyz, B * N, 3, C1, lda=C1, ldb=3, ldc=3, beta=1.0)
+            gemm(dQ, st["wx"], dcentres, B * S, 3, C1, lda=C1, ldb=3, ldc=3, beta=1.0)
 
     # -------------------------------------------------------------------------------------------- encoder
     def _encoder_forward(self, tag, enc, xyz, start1, start2):
@@ -350,10 +378,13 @@ class Trainer:
         _lib.call("pz_maxpool_forward", _p(c.out), B, S2, 1024, _p(c.fg), _p(c.argo), _st())
         return c
 
-    def _encoder_backward(self, c, dfg, dxf, accumulate=False):
+    def _encoder_backward(self, c, dfg, dxf, accumulate=False, dattn=None, dxyz=None, dx2=None):
         """dfg [B,1024] = d loss / d f_global; dxf [B*1024,64] = d loss / d x_feature from the boundary heads
-        (accumulated into, then consumed).  Writes every parameter gradient of the encoder."""
-        enc, B, tag, G = c.enc, c.B, c.tag, self.flat.g
+        (accumulated into, then consumed).  Writes every parameter gradient of the encoder.  Optional gradients of
+        the other outputs: ``dattn`` [B,256,256] of the mean attention map, ``dx2`` [B*256,3] of the stage-2 centres.
+        ``dxyz`` [B*1024,3] (zeroed by the caller) receives d loss / d xyz through the stem, both grouping stages and
+        the centres (FPS and kNN indices are constants)."""
+        enc, B, tag, G = c.enc, c.B, c.tag, self._g
         b = lambda n, *s, **k: self.buf(f"{tag}.{n}", *s, **k)  # noqa: E731
         T, R1, R2, R0 = B * S2, B * S1 * KNN, B * S2 * KNN, B * NPTS
         dout = b("dout", T, 1024)
@@ -385,6 +416,8 @@ class Trainer:
                      sc=S2 * 256)
                 gemm(dr, v, dA, S2, S2, 256, tb=True, lda=256, ldb=256, ldc=S2, alpha=-1.0, batch=B, sa=S2 * 256,
                      sb=S2 * 256, sc=LL)
+            if dattn is not None:                    # attention = mean of the four maps (model5_b.py:468-469)
+                axpby(B * S2, S2, 0.25, dattn, S2, 1.0, dA, S2, dA, S2)
             _lib.call("pz_softmax_backward", _p(A), _p(dA), B * S2, S2, 1.0 / math.sqrt(64.0), _p(dS), _st())
             # S = q k^T :  dq = dS k ; dk = dS^T q
             if self.tf32:
@@ -411,7 +444,17 @@ class Trainer:
                    tf32=self.tf32, bias_grad=False)
         df1f = b("df1f", B * S1, 128)
         df1f.zero_()
-        self._group_layer1_backward(tag + ".sg2", c.sg2, B, db1, df1f)
+        dx1 = dxc2 = None
+        if dxyz is not None:
+            dx1, dxc2 = b("dx1", B * S1, 3), b("dxc2", B * S2, 3)
+            dx1.zero_()
+            if dx2 is None:
+                dxc2.zero_()
+            else:
+                axpby(B * S2, 3, 1.0, dx2, 3, 0.0, None, 0, dxc2, 3)
+        self._group_layer1_backward(tag + ".sg2", c.sg2, B, db1, df1f, dx1, dxc2)
+        if dxyz is not None:                         # x2 = x1[fps2]
+            _lib.call("pz_scatter_add_rows", _p(dxc2), 3, 0, 3, _p(c.fps2), B * S2, S2, S1, _p(dx1), 3, _st())
         # sg1
         da2, da1 = b("da2", R1, 128), b("da1", R1, 128)
         _lib.call("pz_maxpool_backward", _p(df1f), _p(c.f1f), _p(c.arg1), B * S1, KNN, 128, 1, _p(da2), _st())
@@ -420,7 +463,9 @@ class Trainer:
         _lib.call("pz_colsum", _p(gated1), 128, B * S1, 128, 1.0, _p(G(enc.mlp4.bias)), _st())
         linear_bwd(da2, 128, c.a1, 128, R1, enc.mlp4, G(enc.mlp4.weight), G(enc.mlp4.bias), da1, 128, mask=c.a1, ldmask=128,
                    tf32=self.tf32, bias_grad=False)
-        self._group_layer1_backward(tag + ".sg1", c.sg1, B, da1, dxf)
+        self._group_layer1_backward(tag + ".sg1", c.sg1, B, da1, dxf, dxyz, dx1)
+        if dxyz is not None:                         # x1 = xyz[fps1]
+            _lib.call("pz_scatter_add_rows", _p(dx1), 3, 0, 3, _p(c.fps1), B * S1, S1, NPTS, _p(dxyz), 3, _st())
         # stem
         dh2, dy1, dh1 = b("dh2", R0, 64), b("dy1", R0, 64), b("dh1", R0, 64)
         _lib.call("pz_bn_point_train_backward", _p(c.h2), _p(c.xf), _p(dxf), B, NPTS, 64, _p(enc.bn2.weight), _p(c.bn[2]),
@@ -428,7 +473,8 @@ class Trainer:
         linear_bwd(dh2, 64, c.y1, 64, R0, enc.mlp2, G(enc.mlp2.weight), G(enc.mlp2.bias), dy1, 64, tf32=self.tf32)
         _lib.call("pz_bn_point_train_backward", _p(c.h1), _p(c.y1), _p(dy1), B, NPTS, 64, _p(enc.bn1.weight), _p(c.bn[0]),
                   _p(c.bn[1]), 1, int(accumulate), _p(dh1), _p(G(enc.bn1.weight)), _p(G(enc.bn1.bias)), _st())
-        linear_bwd(dh1, 64, c.xyz, 3, R0, enc.mlp1, G(enc.mlp1.weight), G(enc.mlp1.bias), tf32=self.tf32)
+        linear_bwd(dh1, 64, c.xyz, 3, R0, enc.mlp1, G(enc.mlp1.weight), G(enc.mlp1.bias), dxyz, 3, beta=1.0,
+                   tf32=self.tf32)
 
     # -------------------------------------------------------------------------------------------- MLP stacks
     def _mlp_forward(self, tag, seq, x, ldx, M):
@@ -445,7 +491,7 @@ class Trainer:
 
     def _mlp_backward(self, tag, lins, acts, x, ldx, M, dy, dx, lddx):
         """dy = gradient of the last (linear) output; returns nothing, fills dx [M, in] (may be None)."""
-        G = self.flat.g
+        G = self._g
         for i in range(len(lins) - 1, -1, -1):
             lin = lins[i]
             xin, ldin = (acts[i - 1], lins[i - 1].weight.shape[0]) if i > 0 else (x, ldx)
@@ -500,9 +546,17 @@ class Trainer:
         ``(out, [0], x2_fpc, attention_fpc, x2_mrpc, attention_mrpc, de_fpcb, de_mrpcb)``."""
         fpc, mrpc = fpc.contiguous().float(), mrpc.contiguous().float()
         _lib.require_cuda(fpc, mrpc)
-        B = fpc.shape[0]
         with torch.cuda.device(self.dev):
             fw = self._forward(fpc, mrpc, starts)
+            out6, de_f, de_m, x2f, af, x2m, am = self._outputs(fw, fpc.shape[0], need=True)
+        self._invalidate_inference_state()            # the BatchNorm running statistics were updated in place
+        return out6, [0], x2f, af, x2m, am, de_f, de_m
+
+    def _outputs(self, fw, B, need):
+        """The train-mode forward's outputs as fresh tensors: ``(out6, de_fpcb, de_mrpcb, x2_fpc, attention_fpc,
+        x2_mrpc, attention_mrpc)``; ``de_*`` are None after predict6's forward, the last four None without ``need``."""
+        res = [None] * 4
+        if need:
             res = []
             for e in (fw["ef"], fw["em"]):
                 att = torch.empty(B, S2, S2, device=self.dev)
@@ -511,10 +565,11 @@ class Trainer:
                 axpby(n, S2, 0.25, e.A[2], S2, 1.0, att, S2, att, S2)
                 axpby(n, S2, 0.25, e.A[3], S2, 1.0, att, S2, att, S2)
                 res += [e.x2.clone(), att]
-        de_f = fw["logit_f"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
-        de_m = fw["logit_m"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
-        self._invalidate_inference_state()            # the BatchNorm running statistics were updated in place
-        return fw["out6"].clone(), [0], res[0], res[1], res[2], res[3], de_f, de_m
+        de_f = de_m = None
+        if "logit_f" in fw:
+            de_f = fw["logit_f"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
+            de_m = fw["logit_m"].view(B, NPTS, 2).permute(0, 2, 1).contiguous()
+        return (fw["out6"].clone(), de_f, de_m, *res)
 
     def _pose_losses(self, out6, mrpc, rpc, igt, B):
         """The pose part of training_step (model5_b.py:947-1029): mat = se3.exp(out), de_mrpc = mat . mrpc,
@@ -590,16 +645,7 @@ class Trainer:
             fw = self._forward(fpc, mrpc, starts, pretrain=True)
             out6 = fw["out6"]
             vals, mat, de_mrpc, dout6, (w_re, w_g, w_emd) = self._pose_losses(out6, mrpc, rpc, igt, B)
-            df = self.buf("df", B, 2048)
-            self._mlp_backward("tf", fw["tf_l"], fw["tf_a"], fw["f"], 2048, B, dout6, df, 2048)
-            dfg_f, dfg_m = self.buf("dfg_f", B, 1024), self.buf("dfg_m", B, 1024)
-            axpby(B, 1024, 1.0, df, 2048, 0.0, None, 0, dfg_f, 1024)
-            axpby(B, 1024, 1.0, df[:, 1024:], 2048, 0.0, None, 0, dfg_m, 1024)
-            dxf = self.buf("dxf_f", B * NPTS, 64)
-            dxf.zero_()
-            self._encoder_backward(fw["ef"], dfg_f, dxf, accumulate=False)
-            dxf.zero_()
-            self._encoder_backward(fw["em"], dfg_m, dxf, accumulate=True)
+            self._backward(fw, B, dout6)
             if self.use_emd2 or self.use_cd2:
                 self._attention_peak_terms(fw["ef"], fw["em"], B, vals)
             v = vals.cpu().tolist()
@@ -618,14 +664,10 @@ class Trainer:
         fpc, mrpc, igt, rpc, fpcb, rpcb, fpc_idx, rpc_idx = [t.contiguous().float() for t in batch[:8]]
         _lib.require_cuda(fpc, mrpc, igt, rpc, fpcb, rpcb, fpc_idx, rpc_idx)
         B = fpc.shape[0]
-        G = self.flat.g
         self.flat.grads.zero_()
         with torch.cuda.device(self.dev):
             fw = self._forward(fpc, mrpc, starts)
-            ef, em, f, tf_l, tf_a, out6 = fw["ef"], fw["em"], fw["f"], fw["tf_l"], fw["tf_a"], fw["out6"]
-            lf_l, lf_a, lm_l, lm_a, gmax, garg = fw["lf_l"], fw["lf_a"], fw["lm_l"], fw["lm_a"], fw["gmax"], fw["garg"]
-            seg_f, seg_m, sf_l, sf_a, sm_l, sm_a = fw["seg_f"], fw["seg_m"], fw["sf_l"], fw["sf_a"], fw["sm_l"], fw["sm_a"]
-            logit_f, logit_m = fw["logit_f"], fw["logit_m"]
+            ef, em, out6, logit_f, logit_m = fw["ef"], fw["em"], fw["out6"], fw["logit_f"], fw["logit_m"]
             R0 = B * NPTS
             # ---- losses
             vals, mat, de_mrpc, dout6, (w_re, w_g, w_emd) = self._pose_losses(out6, mrpc, rpc, igt, B)
@@ -661,34 +703,7 @@ class Trainer:
                 g1b, _ = emd_cuda.matchcost_backward(gcb, inv_bnd, rpcb, match_m)
                 axpby(B * 128, 3, 1.0, gbx, 3, 1.0, g1b, 3, gbx, 3)
             _lib.call("pz_pose_grad", _p(out6), _p(bnd_m), _p(gbx), 128, None, 0.0, B, 1.0, _p(dout6), _st())
-
-            # ---- backward: pose head
-            df = self.buf("df", B, 2048)
-            self._mlp_backward("tf", tf_l, tf_a, f, 2048, B, dout6, df, 2048)
-            dfg_f, dfg_m = self.buf("dfg_f", B, 1024), self.buf("dfg_m", B, 1024)
-            axpby(B, 1024, 1.0, df, 2048, 0.0, None, 0, dfg_f, 1024)
-            axpby(B, 1024, 1.0, df[:, 1024:], 2048, 0.0, None, 0, dfg_m, 1024)
-            # ---- backward: boundary heads
-            dseg_f, dseg_m = self.buf("dseg_f", R0, 128), self.buf("dseg_m", R0, 128)
-            self._mlp_backward("sf", sf_l, sf_a, seg_f, 128, R0, dlf, dseg_f, 128)
-            self._mlp_backward("sm", sm_l, sm_a, seg_m, 128, R0, dlm, dseg_m, 128)
-            dg_f, dg_m = self.buf("dg_f", B, 64), self.buf("dg_m", B, 64)
-            _lib.call("pz_group_sum", _p(dseg_f), 128, B, NPTS, 64, _p(dg_f), _st())
-            _lib.call("pz_group_sum", _p(dseg_m), 128, B, NPTS, 64, _p(dg_m), _st())
-            axpby(B, 64, 1.0, dg_f, 64, 1.0, dg_m, 64, dg_f, 64)
-            dloc_m, dloc_f = self.buf("dloc_m", R0, 64), self.buf("dloc_f", R0, 64)
-            _lib.call("pz_maxpool_backward", _p(dg_f), _p(gmax), _p(garg), B, NPTS, 64, 0, _p(dloc_m), _st())
-            axpby(R0, 64, 1.0, dloc_m, 64, 1.0, dseg_m[:, 64:], 128, dloc_m, 64)
-            axpby(R0, 64, 1.0, dseg_f[:, 64:], 128, 0.0, None, 0, dloc_f, 64)
-            dxf_f, dxf_m = self.buf("dxf_f", R0, 64), self.buf("dxf_m", R0, 64)
-            self._mlp_backward("lf", lf_l, lf_a, ef.xf, 64, R0, dloc_f, dxf_f, 64)
-            self._mlp_backward("lm", lm_l, lm_a, em.xf, 64, R0, dloc_m, dxf_m, 64)
-            self._bucket_ready("heads")
-            # ---- backward: encoders
-            self._encoder_backward(ef, dfg_f, dxf_f)
-            self._bucket_ready("Encoder")
-            self._encoder_backward(em, dfg_m, dxf_m)
-            self._bucket_ready("Encoder2")
+            self._backward(fw, B, dout6, dlf, dlm, overlap_allreduce=True)
             if self.use_emd2 or self.use_cd2:
                 self._attention_peak_terms(ef, em, B, vals)
             v = vals.cpu().tolist()
@@ -706,6 +721,54 @@ class Trainer:
             loss += (terms["emd2"] if self.use_emd2 else 0.0) + (terms["loss_cd2"] if self.use_cd2 else 0.0)
         terms["loss"] = loss
         return terms
+
+    def _backward(self, fw, B, dout6, dlf=None, dlm=None, dattn=(None, None), dx2=(None, None), dxyz=(None, None),
+                  overlap_allreduce=False):
+        """Backward of the train-mode forward ``fw`` (``_forward``) from gradients of its outputs, added into the
+        parameter gradients (zeroed by the caller): ``dout6`` [B,6] of the pose; ``dlf`` / ``dlm`` [B*1024,2] of the
+        point-major logits of the two boundary heads (predict5 only; both or neither); per cloud (fpc, mrpc) optional
+        ``dattn`` [B,256,256] of the mean attention map and ``dx2`` [B*256,3] of the stage-2 centres; ``dxyz``
+        [B*1024,3] per cloud (zeroed by the caller) receive d loss / d cloud.  With ``fw`` from predict6 both clouds
+        went through ``Encoder`` and its gradients from the two passes add.  ``overlap_allreduce``: start each
+        gradient bucket's all-reduce as soon as it is final."""
+        R0 = B * NPTS
+        pretrain = "logit_f" not in fw
+        # ---- pose head
+        df = self.buf("df", B, 2048)
+        self._mlp_backward("tf", fw["tf_l"], fw["tf_a"], fw["f"], 2048, B, dout6, df, 2048)
+        dfg_f, dfg_m = self.buf("dfg_f", B, 1024), self.buf("dfg_m", B, 1024)
+        axpby(B, 1024, 1.0, df, 2048, 0.0, None, 0, dfg_f, 1024)
+        axpby(B, 1024, 1.0, df[:, 1024:], 2048, 0.0, None, 0, dfg_m, 1024)
+        if pretrain:                # no boundary heads: nothing reaches x_feature from above
+            dxf_f = dxf_m = self.buf("dxf_f", R0, 64)
+            dxf_f.zero_()
+        else:
+            # ---- boundary heads
+            dseg_f, dseg_m = self.buf("dseg_f", R0, 128), self.buf("dseg_m", R0, 128)
+            self._mlp_backward("sf", fw["sf_l"], fw["sf_a"], fw["seg_f"], 128, R0, dlf, dseg_f, 128)
+            self._mlp_backward("sm", fw["sm_l"], fw["sm_a"], fw["seg_m"], 128, R0, dlm, dseg_m, 128)
+            dg_f, dg_m = self.buf("dg_f", B, 64), self.buf("dg_m", B, 64)
+            _lib.call("pz_group_sum", _p(dseg_f), 128, B, NPTS, 64, _p(dg_f), _st())
+            _lib.call("pz_group_sum", _p(dseg_m), 128, B, NPTS, 64, _p(dg_m), _st())
+            axpby(B, 64, 1.0, dg_f, 64, 1.0, dg_m, 64, dg_f, 64)
+            dloc_m, dloc_f = self.buf("dloc_m", R0, 64), self.buf("dloc_f", R0, 64)
+            _lib.call("pz_maxpool_backward", _p(dg_f), _p(fw["gmax"]), _p(fw["garg"]), B, NPTS, 64, 0, _p(dloc_m), _st())
+            axpby(R0, 64, 1.0, dloc_m, 64, 1.0, dseg_m[:, 64:], 128, dloc_m, 64)
+            axpby(R0, 64, 1.0, dseg_f[:, 64:], 128, 0.0, None, 0, dloc_f, 64)
+            dxf_f, dxf_m = self.buf("dxf_f", R0, 64), self.buf("dxf_m", R0, 64)
+            self._mlp_backward("lf", fw["lf_l"], fw["lf_a"], fw["ef"].xf, 64, R0, dloc_f, dxf_f, 64)
+            self._mlp_backward("lm", fw["lm_l"], fw["lm_a"], fw["em"].xf, 64, R0, dloc_m, dxf_m, 64)
+            if overlap_allreduce:
+                self._bucket_ready("heads")
+        # ---- encoders
+        self._encoder_backward(fw["ef"], dfg_f, dxf_f, dattn=dattn[0], dxyz=dxyz[0], dx2=dx2[0])
+        if overlap_allreduce and not pretrain:
+            self._bucket_ready("Encoder")
+        if pretrain:
+            dxf_m.zero_()
+        self._encoder_backward(fw["em"], dfg_m, dxf_m, accumulate=pretrain, dattn=dattn[1], dxyz=dxyz[1], dx2=dx2[1])
+        if overlap_allreduce and not pretrain:
+            self._bucket_ready("Encoder2")
 
     def _bucket_ready(self, name):
         """Called by the backward pass as soon as a gradient bucket is final: start its all-reduce so that it
