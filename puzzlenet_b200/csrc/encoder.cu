@@ -6,6 +6,7 @@
 // every launch covers 128 clouds at B=64 instead of 64 -- FPS, the latency-bound stage, then
 // occupies 128 of the 148 SMs.
 
+#include <algorithm>
 #include <climits>
 #include <functional>
 
@@ -472,20 +473,6 @@ __global__ void __launch_bounds__(256) idx64_to_rows32_kernel(const int64_t* __r
     rows[e] = (int)(e / per_cloud) * N + (int)idx[e];
 }
 
-// sum split-K partials, add bias, optional relu
-__global__ void __launch_bounds__(256) splitk_finish_kernel(const float* __restrict__ part, int splits, int M,
-                                                            int N, const float* __restrict__ bias, int relu,
-                                                            float* __restrict__ y, int ldy) {
-  const int e = blockIdx.x * 256 + threadIdx.x;
-  if (e >= M * N) return;
-  const int m = e / N, n = e - m * N;
-  float s = 0.f;
-  for (int z = 0; z < splits; ++z) s += part[(size_t)z * M * N + e];
-  if (bias) s += bias[n];
-  if (relu) s = fmaxf(s, 0.f);
-  y[(size_t)m * ldy + n] = s;
-}
-
 // Y[M,N] = act(X[M,K] W[N,K]^T + b) for skinny M (the pose MLP, model5_b.py:561-571 / :723-725: M = B <= 64 rows per
 // row block).  One CTA per SK_COLS output columns and 64 rows over the WHOLE K: grid = N / 8 CTAs (128 for the first
 // layer), so every layer is ONE launch with no split-K partials and no finishing pass.  X and the 8 weight rows stream
@@ -574,8 +561,7 @@ __global__ void __launch_bounds__(256) skinny_linear_kernel(const float* __restr
 // Pose-MLP layer: one launch of skinny_linear_kernel (K % 128 == 0, 16-byte aligned rows); anything else through the
 // tiled fp32 GEMM.
 static int skinny_linear(const float* A, int lda, const float* W, const float* bias, int M, int N, int K,
-                         int relu, float* Y, int ldy, float* partial, size_t partial_floats, cudaStream_t st) {
-  (void)partial; (void)partial_floats;
+                         int relu, float* Y, int ldy, cudaStream_t st) {
   if (K % SK_KC == 0 && lda % 4 == 0 && (((uintptr_t)A | (uintptr_t)W) & 15) == 0) {
     PZ_CUDA(cudaFuncSetAttribute(skinny_linear_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SK_SMEM));
     dim3 grid((N + SK_COLS - 1) / SK_COLS, (M + SK_ROWS - 1) / SK_ROWS);
@@ -771,21 +757,10 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(const PackJobs jobs) 
 }
 
 // Q[s, k] = W1[k, 0:3] . centre[s]  -- the centroid half of layer 1 of a grouped MLP (the per-neighbour
-// half, P, comes out of the layer-1 GEMM):  relu(W1 [xyz_j - c_s ; f_j] + b1) = relu(P_j - Q_s).
-__global__ void __launch_bounds__(256) centre_proj_kernel(const float* __restrict__ centres, const float* w1a,
-                                                          const float* w1b, int ldw1, int rows_per_set, int rows,
-                                                          int C1, __nv_bfloat16* __restrict__ Q) {
-  const size_t e = (size_t)blockIdx.x * 256 + threadIdx.x;
-  if (e >= (size_t)rows * C1) return;
-  const int s = (int)(e / C1), k = (int)(e - (size_t)s * C1);
-  const float* w = (s / rows_per_set == 0 ? w1a : w1b) + (size_t)k * ldw1;
-  const float* c = centres + (size_t)s * 3;
-  Q[e] = __float2bfloat16_rn(fmaf(w[0], c[0], fmaf(w[1], c[1], w[2] * c[2])));
-}
-
-// the same in fp32 for the split path: Q [rows, C1].  The three xyz weights of every channel (both weight sets) are
-// staged in shared memory once per block (they sit 3 + D floats apart in the weight matrix); a thread then walks
-// consecutive (row, channel) elements, so the Q stores are coalesced and the centre is a broadcast read.
+// half, P, comes out of the layer-1 GEMM):  relu(W1 [xyz_j - c_s ; f_j] + b1) = relu(P_j - Q_s).  fp32 Q [rows, C1] for
+// the split path.  The three xyz weights of every channel (both weight sets) are staged in shared memory once per block
+// (they sit 3 + D floats apart in the weight matrix); a thread then walks consecutive (row, channel) elements, so the Q
+// stores are coalesced and the centre is a broadcast read.
 __global__ void __launch_bounds__(256) centre_proj_f32_kernel(const float* __restrict__ centres, const float* w1a,
                                                               const float* w1b, int ldw1, int rows_per_set, int rows,
                                                               int C1, float* __restrict__ Q) {
@@ -836,13 +811,32 @@ static bool encoder_weights_ok(const PzEncoderWeights& w) {
   return true;
 }
 
-struct EncoderScratch {
-  float *xfeat, *F1, *nx1, *f1f, *F2, *nx2, *att_cat, *q, *k, *v, *r, *tailp, *fglob;
-  int *knn1r, *knn2r;
-  // bf16 path
-  __nv_bfloat16 *xfeat_b, *P1, *f1f_b, *P2, *att_cat_b, *r_b, *wpack, *qk_b, *vT_b, *Q1, *Q2;
-  float *bqkv;
-};
+// ---- the encoder's workspace: a common part, then the layout of the precision that runs (encoder_forward_impl).
+// Common: tensors of every precision; xfeat, nx2 and fglob are replaced by the caller's outputs where it asked for them.
+struct EncoderCommon { float *xfeat, *nx1, *nx2, *fglob; int *knn1r, *knn2r; };
+static void carve(int C, Arena& a, EncoderCommon& s) {
+  s.xfeat = a.take<float>((size_t)C * NPTS * D0);
+  s.nx1 = a.take<float>((size_t)C * S1 * 3);
+  s.knn1r = a.take<int>((size_t)C * S1 * KNN);
+  s.nx2 = a.take<float>((size_t)C * S2 * 3);
+  s.knn2r = a.take<int>((size_t)C * S2 * KNN);
+  s.fglob = a.take<float>((size_t)C * 1024);
+}
+
+// fp32 path: F1 / F2 = the feature half of layer 1 of each grouped MLP, f1f and att_cat where the caller keeps no copy,
+// q / k / v / r of one attention layer, the tail's 128-row tile maxima
+struct Fp32Scratch { float *F1, *f1f, *F2, *att_cat, *q, *k, *v, *r, *tilemax; };
+static void carve(int C, Arena& a, Fp32Scratch& s) {
+  s.F1 = a.take<float>((size_t)C * NPTS * C1A);
+  s.f1f = a.take<float>((size_t)C * S1 * C1B);
+  s.F2 = a.take<float>((size_t)C * S1 * C2A);
+  s.att_cat = a.take<float>((size_t)C * LATT * 1280);
+  s.q = a.take<float>((size_t)C * LATT * 64);
+  s.k = a.take<float>((size_t)C * LATT * 64);
+  s.v = a.take<float>((size_t)C * LATT * CATT);
+  s.r = a.take<float>((size_t)C * LATT * CATT);
+  s.tilemax = a.take<float>((size_t)C * (LATT / 128) * 1024);
+}
 
 // bf16 weight pack of ONE encoder (elements): W3f[128,64] W4[128,128] W5f[256,128] W6[256,256]
 // Wout[1024,1280]  4 x (20 tile images of Wqkv|Wo for the fused attention layer)
@@ -850,41 +844,57 @@ constexpr size_t WP_W3F = 0, WP_W4 = WP_W3F + 128 * 64, WP_W5F = WP_W4 + 128 * 1
                  WP_WOUT = WP_W6 + 256 * 256, WP_ATTIMG = WP_WOUT + 1024 * 1280, WP_STEM = WP_ATTIMG + 4 * ATTN_WIMG_ELEMS,
                  WP_TOTAL = WP_STEM + 2 * 64 * STEM_WS;   // stem: W2 hi, lo as [64, STEM_WS] images
 
+// bf16 path: x_feature, P1 / P2 (layer 1 of each grouped MLP over the source points), f1f and att_cat in bf16; the weight
+// packs of both encoders and their q|k|v biases
+struct Bf16Scratch { __nv_bfloat16 *xfeat, *P1, *f1f, *P2, *att_cat, *wpack; float* bqkv; };
+static void carve(int C, Arena& a, Bf16Scratch& s) {
+  s.xfeat = a.take<__nv_bfloat16>((size_t)C * NPTS * D0);
+  s.P1 = a.take<__nv_bfloat16>((size_t)C * NPTS * C1A);
+  s.f1f = a.take<__nv_bfloat16>((size_t)C * S1 * C1B);
+  s.P2 = a.take<__nv_bfloat16>((size_t)C * S1 * C2A);
+  s.att_cat = a.take<__nv_bfloat16>((size_t)C * LATT * 1280);
+  s.wpack = a.take<__nv_bfloat16>(2 * WP_TOTAL);
+  s.bqkv = a.take<float>(2 * 4 * 384);
+}
+
 // split path: fp16 planes of ONE encoder (elements per plane): W3f[128,64] W4[128,128] W5f[256,128] W6[256,256]
 // 4 x (Wqk[128,256] Wv[256,256] Wo[256,256]) Wout[1024,1280]; planes at wpack + ((e * 2 + plane) * WS_TOTAL)
 constexpr size_t WS_W3F = 0, WS_W4 = WS_W3F + 128 * 64, WS_W5F = WS_W4 + 128 * 128, WS_W6 = WS_W5F + 256 * 128,
                  WS_ATT = WS_W6 + 256 * 256, WS_ATT_STRIDE = 128 * 256 + 2 * 256 * 256, WS_WOUT = WS_ATT + 4 * WS_ATT_STRIDE,
                  WS_TOTAL = WS_WOUT + 1024 * 1280;
 
-static size_t encoder_scratch_layout(int C, Arena& a, EncoderScratch& s) {
-  s.xfeat = a.take<float>((size_t)C * NPTS * D0);
-  s.F1 = a.take<float>((size_t)C * NPTS * C1A);
-  s.nx1 = a.take<float>((size_t)C * S1 * 3);
-  s.knn1r = a.take<int>((size_t)C * S1 * KNN);
-  s.f1f = a.take<float>((size_t)C * S1 * C1B);
-  s.F2 = a.take<float>((size_t)C * S1 * C2A);
-  s.nx2 = a.take<float>((size_t)C * S2 * 3);
-  s.knn2r = a.take<int>((size_t)C * S2 * KNN);
-  s.att_cat = a.take<float>((size_t)C * LATT * 1280);
-  s.q = a.take<float>((size_t)C * LATT * 64);
-  s.k = a.take<float>((size_t)C * LATT * 64);
-  s.v = a.take<float>((size_t)C * LATT * CATT);
-  s.r = a.take<float>((size_t)C * LATT * CATT);
-  s.tailp = a.take<float>((size_t)C * 2 * 1024);
-  s.fglob = a.take<float>((size_t)C * 1024);
-  s.xfeat_b = a.take<__nv_bfloat16>((size_t)C * NPTS * D0);
-  s.P1 = a.take<__nv_bfloat16>((size_t)C * NPTS * C1A);
-  s.Q1 = a.take<__nv_bfloat16>((size_t)C * S1 * C1A);
-  s.f1f_b = a.take<__nv_bfloat16>((size_t)C * S1 * C1B);
-  s.P2 = a.take<__nv_bfloat16>((size_t)C * S1 * C2A);
-  s.Q2 = a.take<__nv_bfloat16>((size_t)C * S2 * C2A);
-  s.att_cat_b = a.take<__nv_bfloat16>((size_t)C * LATT * 1280);
-  s.qk_b = a.take<__nv_bfloat16>((size_t)C * LATT * 128);
-  s.vT_b = a.take<__nv_bfloat16>((size_t)C * LATT * CATT);
-  s.r_b = a.take<__nv_bfloat16>((size_t)C * LATT * CATT);
-  s.wpack = a.take<__nv_bfloat16>(2 * WP_TOTAL > 4 * WS_TOTAL ? 2 * WP_TOTAL : 4 * WS_TOTAL);   // bf16 packs OR split planes
+// split path: every 16-bit tensor is a pair of same-shaped fp16 planes [hi, lo], stored as the raw 16-bit type TcGemm and
+// AttnSplit take.  P (layer 1 over the source points) and Q = W1[:,0:3] c of each grouped MLP stay fp32.  The chained
+// attention launches read one q|k / v^T set while they write the next layer's into the other; r stays on chip (fused
+// out-projection) and has no buffer.
+typedef __nv_bfloat16 h16;
+struct SplitScratch {
+  h16 *xfeat[2], *f1f[2], *att_cat[2];   // [plane]
+  h16 *qk[2][2], *vT[2][2];              // [set][plane]: q|k [C*256, 128], v^T [C][256 ch][256 tokens]
+  float *P1, *Q1, *P2, *Q2;
+  int* flags;                            // [3][C] hand-over counters of the chained attention launches
+  float* tilemax;                        // [C*2, 1024] the tail's 128-row tile maxima
+  h16* wpack;
+  float* bqkv;
+};
+static void carve(int C, Arena& a, SplitScratch& s) {
+  for (int pl = 0; pl < 2; ++pl) {
+    s.xfeat[pl] = a.take<h16>((size_t)C * NPTS * D0);
+    s.f1f[pl] = a.take<h16>((size_t)C * S1 * C1B);
+    s.att_cat[pl] = a.take<h16>((size_t)C * LATT * 1280);
+    for (int set = 0; set < 2; ++set) {
+      s.qk[set][pl] = a.take<h16>((size_t)C * LATT * 128);
+      s.vT[set][pl] = a.take<h16>((size_t)C * LATT * CATT);
+    }
+  }
+  s.P1 = a.take<float>((size_t)C * NPTS * C1A);
+  s.Q1 = a.take<float>((size_t)C * S1 * C1A);
+  s.P2 = a.take<float>((size_t)C * S1 * C2A);
+  s.Q2 = a.take<float>((size_t)C * S2 * C2A);
+  s.flags = a.take<int>((size_t)3 * C);
+  s.tilemax = a.take<float>((size_t)C * (LATT / 128) * 1024);
+  s.wpack = a.take<h16>(4 * WS_TOTAL);
   s.bqkv = a.take<float>(2 * 4 * 384);
-  return a.used;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -899,14 +909,11 @@ static size_t encoder_scratch_layout(int C, Arena& a, EncoderScratch& s) {
 using AfterStem = std::function<int(const float* xfeat)>;
 
 static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
-                                const int64_t* start2, const PzEncoderOutputs& o, EncoderScratch& s, float* fglob_pair,
-                                const float** xfeat_out, const AfterStem* after_stem, bool reuse_pack, cudaStream_t st) {
+                                const int64_t* start2, const PzEncoderOutputs& o, const EncoderCommon& c,
+                                const Bf16Scratch& s, const AfterStem* after_stem, bool reuse_pack, cudaStream_t st) {
   const int C = E * B;
   const PzEncoderWeights& wa = w[0];
   const PzEncoderWeights& wb = w[E - 1];
-  float* xfeat = o.x_feature ? o.x_feature : s.xfeat;
-  float* nx2 = o.x2 ? o.x2 : s.nx2;
-  if (xfeat_out) *xfeat_out = xfeat;
 
   // ---- weights -> bf16 packs (one launch, ~8 MB read).  The pack lives in the caller's workspace; a caller that
   // knows the weights are unchanged since its previous call may say so (PZ_FLAG_REUSE_PACKS) and skip it.
@@ -958,56 +965,56 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
   PZ_CUDA(cudaEventRecord(ss->fork, st));
   PZ_CUDA(cudaStreamWaitEvent(sg, ss->fork, 0));
   prof_mark("_side_begin", sg, gl);
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, sg));
+  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, sg));
   prof_mark("fps1", sg, gl);
-  PZ_TRY(launch_knn(s.nx1, xyz, C, S1, NPTS, KNN, o.knn1, s.knn1r, nullptr, sg));
+  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, sg));
   prof_mark("knn1", sg, gl);
   PZ_CUDA(cudaEventRecord(ss->join_a, sg));
-  PZ_TRY(launch_fps(s.nx1, C, S1, start2, S2, o.fps2, nullptr, nx2, sg));
+  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, sg));
   prof_mark("fps2", sg, gl);
-  PZ_TRY(launch_knn(nx2, s.nx1, C, S2, S1, KNN, o.knn2, s.knn2r, nullptr, sg));
+  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, sg));
   prof_mark("knn2", sg, gl);
   PZ_CUDA(cudaEventRecord(ss->join_b, sg));
 
   PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
   stem_tc_kernel<false><<<C * NPTS / (128 * HD_REPS), 128, STEM_TC_SMEM, st>>>(xyz, stem_of(wa), stem_of(wb), wpa + WP_STEM,
-                                                                          wpb + WP_STEM, B, HD_REPS, xfeat, s.xfeat_b, nullptr);
+                                                                          wpb + WP_STEM, B, HD_REPS, c.xfeat, s.xfeat, nullptr);
   PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
   {
     TcGemm g;  // P1 = x_feature W3[:,3:]^T + b3 + W3[:,0:3] xyz
-    g.X = s.xfeat_b; g.ldx = D0; g.W[0] = wpa + WP_W3F; g.W[1] = wpb + WP_W3F; g.ldw = D0;
+    g.X = s.xfeat; g.ldx = D0; g.W[0] = wpa + WP_W3F; g.W[1] = wpb + WP_W3F; g.ldw = D0;
     g.bias[0] = wa.mlp3_b; g.bias[1] = wb.mlp3_b; g.rows_per_wset = B * NPTS; g.M = C * NPTS; g.Nout = C1A; g.K = D0;
     g.Yb = s.P1; g.ldyb = C1A; g.xyz = xyz; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0;
     PZ_TRY(launch_tc_rowgemm(g, st));
     prof_mark("sg1_layer1", st);
   }
-  if (after_stem) PZ_TRY((*after_stem)(xfeat));
+  if (after_stem) PZ_TRY((*after_stem)(c.xfeat));
   PZ_CUDA(cudaStreamWaitEvent(st, ss->join_a, 0));   // kNN of stage 1 (and FPS 1, Q1) are done
   prof_mark("_wait_geometry1", st);
   {
     TcGemm g;  // f1f = max_k relu(W4 relu(P1[j] - Q1[s]) + b4)
-    g.X = s.P1; g.ldx = C1A; g.rows = s.knn1r; g.centers = s.nx1; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0; g.W[0] = wpa + WP_W4; g.W[1] = wpb + WP_W4; g.ldw = C1A;
+    g.X = s.P1; g.ldx = C1A; g.rows = c.knn1r; g.centers = c.nx1; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0; g.W[0] = wpa + WP_W4; g.W[1] = wpb + WP_W4; g.ldw = C1A;
     g.bias[0] = wa.mlp4_b; g.bias[1] = wb.mlp4_b; g.rows_per_wset = B * S1 * KNN; g.M = C * S1 * KNN; g.Nout = C1B;
-    g.K = C1A; g.epi = 1; g.relu = 1; g.Yf = o.f1f; g.ldyf = C1B; g.Yb = s.f1f_b; g.ldyb = C1B;
+    g.K = C1A; g.epi = 1; g.relu = 1; g.Yf = o.f1f; g.ldyf = C1B; g.Yb = s.f1f; g.ldyb = C1B;
     PZ_TRY(launch_tc_gemm(g, st));
     prof_mark("sg1_gather_layer2_maxpool", st);
   }
   {
     TcGemm g;  // P2 = f1f W5[:,3:]^T + b5 + W5[:,0:3] x1
-    g.X = s.f1f_b; g.ldx = C1B; g.W[0] = wpa + WP_W5F; g.W[1] = wpb + WP_W5F; g.ldw = C1B;
+    g.X = s.f1f; g.ldx = C1B; g.W[0] = wpa + WP_W5F; g.W[1] = wpb + WP_W5F; g.ldw = C1B;
     g.bias[0] = wa.mlp5_b; g.bias[1] = wb.mlp5_b; g.rows_per_wset = B * S1; g.M = C * S1; g.Nout = C2A; g.K = C1B;
-    g.Yb = s.P2; g.ldyb = C2A; g.xyz = s.nx1; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B;
+    g.Yb = s.P2; g.ldyb = C2A; g.xyz = c.nx1; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B;
     PZ_TRY(launch_tc_rowgemm(g, st));
     prof_mark("sg2_layer1", st);
   }
   PZ_CUDA(cudaStreamWaitEvent(st, ss->join_b, 0));   // stage-2 geometry is done (side stream joined)
   prof_mark("_wait_geometry2", st);
-  __nv_bfloat16* cat_b = s.att_cat_b;           // [C*256, 1280] bf16: cat(att1..att4, f2f)
+  __nv_bfloat16* cat_b = s.att_cat;             // [C*256, 1280] bf16: cat(att1..att4, f2f)
   float* cat_f = o.att_cat;                     // fp32 copy only when the caller asks for it
   {
     TcGemm g;
-    g.X = s.P2; g.ldx = C2A; g.rows = s.knn2r; g.centers = nx2; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B; g.W[0] = wpa + WP_W6; g.W[1] = wpb + WP_W6; g.ldw = C2A;
+    g.X = s.P2; g.ldx = C2A; g.rows = c.knn2r; g.centers = c.nx2; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B; g.W[0] = wpa + WP_W6; g.W[1] = wpb + WP_W6; g.ldw = C2A;
     g.bias[0] = wa.mlp6_b; g.bias[1] = wb.mlp6_b; g.rows_per_wset = B * S2 * KNN; g.M = C * S2 * KNN; g.Nout = C2B;
     g.K = C2A; g.epi = 1; g.relu = 1; g.Yb = cat_b + 4 * CATT; g.ldyb = 1280;
     if (cat_f) { g.Yf = cat_f + 4 * CATT; g.ldyf = 1280; }
@@ -1015,9 +1022,6 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     PZ_TRY(launch_tc_gemm(g, st));
     prof_mark("sg2_gather_layer2_maxpool", st);
   }
-  if (o.f2f && cat_f)
-    PZ_CUDA(cudaMemcpy2DAsync(o.f2f, CATT * sizeof(float), cat_f + 4 * CATT, 1280 * sizeof(float), CATT * sizeof(float),
-                              (size_t)C * LATT, cudaMemcpyDeviceToDevice, st));
 
   // ---- 4 x offset attention
   const int rows = C * LATT;
@@ -1038,29 +1042,20 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     prof_mark("attn_layer_fused", st);
   }
   // ---- tail
-  {
-    float* fg = o.f_global ? o.f_global : s.fglob;
-    TcGemm g;
-    g.X = cat_b; g.ldx = 1280; g.W[0] = wpa + WP_WOUT; g.W[1] = wpb + WP_WOUT; g.ldw = 1280;
-    g.bias[0] = wa.out_b; g.bias[1] = wb.out_b; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = 1024; g.K = 1280;
-    if (o.out) {
-      g.Yf = o.out; g.ldyf = 1024;
-      PZ_TRY(launch_tc_gemm(g, st));
-      prof_mark("tail_linear", st);
-      rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(o.out, 1024, LATT, 1024, C, C, 0, fg, 1024);
-      PZ_LAUNCH_CHECK();
-      prof_mark("tail_point_max", st);
-    } else {
-      g.epi = 2; g.Yf = fg; g.ldyf = 1024;      // one 256-row tile == one cloud: max over its rows in the epilogue
-      PZ_TRY(launch_tc_gemm(g, st));
-      prof_mark("tail_linear_maxpool", st);
-    }
-    if (fglob_pair)
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair, (size_t)E * 1024 * sizeof(float), fg, 1024 * sizeof(float),
-                                1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
-    if (fglob_pair && E == 2)
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair + 1024, (size_t)E * 1024 * sizeof(float), fg + (size_t)B * 1024,
-                                1024 * sizeof(float), 1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
+  TcGemm g;
+  g.X = cat_b; g.ldx = 1280; g.W[0] = wpa + WP_WOUT; g.W[1] = wpb + WP_WOUT; g.ldw = 1280;
+  g.bias[0] = wa.out_b; g.bias[1] = wb.out_b; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = 1024; g.K = 1280;
+  if (o.out) {
+    g.Yf = o.out; g.ldyf = 1024;
+    PZ_TRY(launch_tc_gemm(g, st));
+    prof_mark("tail_linear", st);
+    rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(o.out, 1024, LATT, 1024, C, C, 0, c.fglob, 1024);
+    PZ_LAUNCH_CHECK();
+    prof_mark("tail_point_max", st);
+  } else {
+    g.epi = 2; g.Yf = c.fglob; g.ldyf = 1024;   // one 256-row tile == one cloud: max over its rows in the epilogue
+    PZ_TRY(launch_tc_gemm(g, st));
+    prof_mark("tail_linear_maxpool", st);
   }
   return 0;
 }
@@ -1070,30 +1065,14 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
 // split path (PZ_PREC_SPLIT): the bf16 path's dataflow with every tensor-core operand as fp16 hi / lo planes and
 // every product as three MMAs (gemm_split.cu, attention_split.cu) -- the fp32 tolerances at tensor-core speed.
 // P = layer 1 over the source points and Q = W1[:,0:3] c stay fp32 in HBM; the gather GEMM forms relu(P_j - Q_s) in
-// fp32 registers before splitting it.  Scratch is the bf16 / fp32 paths' scratch re-used (the planes of a tensor live
-// in two same-sized buffers that are idle in this precision).
+// fp32 registers before splitting it.
 // ---------------------------------------------------------------------------------------------
 static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
-                                 const int64_t* start2, const PzEncoderOutputs& o, EncoderScratch& s, float* fglob_pair,
-                                 const float** xfeat_out, const AfterStem* after_stem, bool reuse_pack, cudaStream_t st) {
+                                 const int64_t* start2, const PzEncoderOutputs& o, const EncoderCommon& c,
+                                 const SplitScratch& s, const AfterStem* after_stem, bool reuse_pack, cudaStream_t st) {
   const int C = E * B;
   const PzEncoderWeights& wa = w[0];
   const PzEncoderWeights& wb = w[E - 1];
-  float* xfeat = o.x_feature ? o.x_feature : s.xfeat;
-  float* nx2 = o.x2 ? o.x2 : s.nx2;
-  if (xfeat_out) *xfeat_out = xfeat;
-  typedef __nv_bfloat16 h16;   // raw 16-bit storage; the split kernels read it as fp16
-  // plane pairs (hi, lo) carved out of buffers that are idle in this precision
-  h16* xfeat_h[2] = {s.P1, s.P1 + (size_t)C * NPTS * D0};
-  float* P1 = s.F1;                                      // [C*1024, 128] fp32
-  float* P2 = s.F2;                                      // [C*512, 256] fp32
-  float* Q1 = s.v;                                       // [C*512, 128] fp32
-  float* Q2 = s.r;                                       // [C*256, 256] fp32
-  h16* f1f_h[2] = {s.f1f_b, s.Q1};
-  h16* cat_h[2] = {s.att_cat_b, reinterpret_cast<h16*>(s.att_cat)};   // [C*256, 1280]
-  h16* qk_h[2] = {s.qk_b, reinterpret_cast<h16*>(s.q)};               // [C*256, 128]
-  h16* vT_h[2] = {s.vT_b, s.P2};                                      // [C][256 ch][256 tok]
-  h16* r_h[2] = {s.r_b, s.Q2};                                        // [C*256, 256]
 
   if (!reuse_pack) {
     PackJobs jobs;
@@ -1141,7 +1120,7 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
 
   // the attention launches' hand-over counters (see the attention block): zeroed here, where no kernel-to-kernel link of the
   // programmatic launch chain is broken by the memset node
-  PZ_CUDA(cudaMemsetAsync(s.tailp, 0, (size_t)3 * C * sizeof(int), st));
+  PZ_CUDA(cudaMemsetAsync(s.flags, 0, (size_t)3 * C * sizeof(int), st));
 
   // ---- geometry (FPS -> centre projection -> kNN, both stages): ahead of the feature chain on the caller's stream.
   // ONE chain: every GEMM CTA of this path fills an SM (shared memory), so a geometry kernel on a second stream does not
@@ -1149,49 +1128,49 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
   // forward 1.70 ms with a side stream, 1.59 without, 1.51 with programmatic dependent launch on the one chain; the
   // 4-stream graph schedule 1.39 vs 1.37 ms per step).
   prof_mark("_side_begin", st);
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, st));
+  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, st));
   prof_mark("fps1", st);
-  PZ_TRY(launch_knn(s.nx1, xyz, C, S1, NPTS, KNN, o.knn1, s.knn1r, nullptr, st));
+  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, st));
   prof_mark("knn1", st);
-  PZ_TRY(launch_centre_proj_f32(s.nx1, wa.mlp3_w, wb.mlp3_w, 3 + D0, B * S1, C * S1, C1A, Q1, st));
-  PZ_TRY(launch_fps(s.nx1, C, S1, start2, S2, o.fps2, nullptr, nx2, st));
+  PZ_TRY(launch_centre_proj_f32(c.nx1, wa.mlp3_w, wb.mlp3_w, 3 + D0, B * S1, C * S1, C1A, s.Q1, st));
+  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, st));
   prof_mark("fps2", st);
-  PZ_TRY(launch_knn(nx2, s.nx1, C, S2, S1, KNN, o.knn2, s.knn2r, nullptr, st));
+  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, st));
   prof_mark("knn2", st);
-  PZ_TRY(launch_centre_proj_f32(nx2, wa.mlp5_w, wb.mlp5_w, 3 + C1B, B * S2, C * S2, C2A, Q2, st));
+  PZ_TRY(launch_centre_proj_f32(c.nx2, wa.mlp5_w, wb.mlp5_w, 3 + C1B, B * S2, C * S2, C2A, s.Q2, st));
 
   // ---- feature chain
   // stem: layer 2 as a split-fp16 mma.sync product (x_feature within ~1e-6 of the fp32 stem), the fp16 hi / lo planes of
   // x_feature written by the same kernel (C * 1024 points always tile by 128 * HD_REPS)
   PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
   PZ_CUDA(launch_pdl(stem_tc_kernel<true>, dim3(C * NPTS / (128 * HD_REPS)), dim3(128), STEM_TC_SMEM, st, xyz, stem_of(wa),
-                     stem_of(wb), (const __nv_bfloat16*)nullptr, (const __nv_bfloat16*)nullptr, B, HD_REPS, xfeat,
-                     reinterpret_cast<__nv_bfloat16*>(xfeat_h[0]), reinterpret_cast<__half*>(xfeat_h[1])));
+                     stem_of(wb), (const __nv_bfloat16*)nullptr, (const __nv_bfloat16*)nullptr, B, HD_REPS, c.xfeat,
+                     s.xfeat[0], reinterpret_cast<__half*>(s.xfeat[1])));
   PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
   {
     TcGemm g;  // P1 = x_feature W3[:,3:]^T + b3 + W3[:,0:3] xyz   (fp32 out)
-    g.X = xfeat_h[0]; g.Xlo = xfeat_h[1]; g.ldx = D0; set_w(g, WS_W3F); g.ldw = D0;
+    g.X = s.xfeat[0]; g.Xlo = s.xfeat[1]; g.ldx = D0; set_w(g, WS_W3F); g.ldw = D0;
     g.bias[0] = wa.mlp3_b; g.bias[1] = wb.mlp3_b; g.rows_per_wset = B * NPTS; g.M = C * NPTS; g.Nout = C1A; g.K = D0;
-    g.Yf = P1; g.ldyf = C1A; g.xyz = xyz; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0;
+    g.Yf = s.P1; g.ldyf = C1A; g.xyz = xyz; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0;
     PZ_TRY(launch_split_rowgemm(g, st));
     prof_mark("sg1_layer1", st);
   }
-  if (after_stem) PZ_TRY((*after_stem)(xfeat));
+  if (after_stem) PZ_TRY((*after_stem)(c.xfeat));
   prof_mark("_wait_geometry1", st);
   {
     TcGemm g;  // f1f = max_k relu(W4 relu(P1[j] - Q1[s]) + b4)
-    g.Xf = P1; g.ldx = C1A; g.Qf = Q1; g.rows = s.knn1r; set_w(g, WS_W4); g.ldw = C1A;
+    g.Xf = s.P1; g.ldx = C1A; g.Qf = s.Q1; g.rows = c.knn1r; set_w(g, WS_W4); g.ldw = C1A;
     g.bias[0] = wa.mlp4_b; g.bias[1] = wb.mlp4_b; g.rows_per_wset = B * S1 * KNN; g.M = C * S1 * KNN; g.Nout = C1B;
-    g.K = C1A; g.epi = 1; g.relu = 1; g.Yf = o.f1f; g.ldyf = C1B; g.Yb = f1f_h[0]; g.Yblo = f1f_h[1]; g.ldyb = C1B;
+    g.K = C1A; g.epi = 1; g.relu = 1; g.Yf = o.f1f; g.ldyf = C1B; g.Yb = s.f1f[0]; g.Yblo = s.f1f[1]; g.ldyb = C1B;
     PZ_TRY(launch_split_gather(g, st));
     prof_mark("sg1_gather_layer2_maxpool", st);
   }
   {
     TcGemm g;  // P2 = f1f W5[:,3:]^T + b5 + W5[:,0:3] x1
-    g.X = f1f_h[0]; g.Xlo = f1f_h[1]; g.ldx = C1B; set_w(g, WS_W5F); g.ldw = C1B;
+    g.X = s.f1f[0]; g.Xlo = s.f1f[1]; g.ldx = C1B; set_w(g, WS_W5F); g.ldw = C1B;
     g.bias[0] = wa.mlp5_b; g.bias[1] = wb.mlp5_b; g.rows_per_wset = B * S1; g.M = C * S1; g.Nout = C2A; g.K = C1B;
-    g.Yf = P2; g.ldyf = C2A; g.xyz = s.nx1; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B;
+    g.Yf = s.P2; g.ldyf = C2A; g.xyz = c.nx1; g.W1x[0] = wa.mlp5_w; g.W1x[1] = wb.mlp5_w; g.ldw1x = 3 + C1B;
     PZ_TRY(launch_split_rowgemm(g, st));
     prof_mark("sg2_layer1", st);
   }
@@ -1199,138 +1178,103 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
   float* cat_f = o.att_cat;
   {
     TcGemm g;
-    g.Xf = P2; g.ldx = C2A; g.Qf = Q2; g.rows = s.knn2r; set_w(g, WS_W6); g.ldw = C2A;
+    g.Xf = s.P2; g.ldx = C2A; g.Qf = s.Q2; g.rows = c.knn2r; set_w(g, WS_W6); g.ldw = C2A;
     g.bias[0] = wa.mlp6_b; g.bias[1] = wb.mlp6_b; g.rows_per_wset = B * S2 * KNN; g.M = C * S2 * KNN; g.Nout = C2B;
-    g.K = C2A; g.epi = 1; g.relu = 1; g.Yb = cat_h[0] + 4 * CATT; g.Yblo = cat_h[1] + 4 * CATT; g.ldyb = 1280;
+    g.K = C2A; g.epi = 1; g.relu = 1; g.Yb = s.att_cat[0] + 4 * CATT; g.Yblo = s.att_cat[1] + 4 * CATT; g.ldyb = 1280;
     if (cat_f) { g.Yf = cat_f + 4 * CATT; g.ldyf = 1280; }
     else if (o.f2f) { g.Yf = o.f2f; g.ldyf = CATT; }
     PZ_TRY(launch_split_gather(g, st));
     prof_mark("sg2_gather_layer2_maxpool", st);
   }
-  if (o.f2f && cat_f)
-    PZ_CUDA(cudaMemcpy2DAsync(o.f2f, CATT * sizeof(float), cat_f + 4 * CATT, 1280 * sizeof(float), CATT * sizeof(float),
-                              (size_t)C * LATT, cudaMemcpyDeviceToDevice, st));
 
   // ---- 4 x offset attention
   const int rows = C * LATT;
   // the out-projection  out = x + relu(Wo r + bo)  runs inside the attention kernel (r never leaves the SM: 67 MB of HBM
   // traffic and one launch per layer less), and so do the NEXT layer's q|k|v projections of the same rows (chained: two
   // more launches per layer less); q|k and v^T planes then alternate between two buffer sets, because the CTAs of a launch
-  // still read the current ones.
-  // chained launches hand over per cloud (AttnSplit::dep_flags): 3 x C counters in the tail's scratch, idle until the tail
-  int* aflags = reinterpret_cast<int*>(s.tailp);
-  h16* qk_set[2][2] = {{qk_h[0], qk_h[1]}, {s.xfeat_b, reinterpret_cast<h16*>(s.k)}};   // second set: idle buffers of equal size
-  h16* vT_set[2][2] = {{vT_h[0], vT_h[1]}, {r_h[0], r_h[1]}};                           // (r is not materialised)
+  // still read the current ones.  Chained launches hand over per cloud (AttnSplit::dep_flags, 3 x C counters).
   for (int l = 0; l < 4; ++l) {
     const size_t xoff = l == 0 ? 4 * CATT : (size_t)(l - 1) * CATT;
     const size_t wl = WS_ATT + (size_t)l * WS_ATT_STRIDE;
     const int cur = l & 1;
     if (l == 0) {
       TcGemm gq;  // [q | k] = x Wqk^T + b
-      gq.X = cat_h[0] + xoff; gq.Xlo = cat_h[1] + xoff; gq.ldx = 1280; set_w(gq, wl); gq.ldw = CATT;
+      gq.X = s.att_cat[0] + xoff; gq.Xlo = s.att_cat[1] + xoff; gq.ldx = 1280; set_w(gq, wl); gq.ldw = CATT;
       gq.bias[0] = s.bqkv + (size_t)l * 384; gq.bias[1] = s.bqkv + ((size_t)(E - 1) * 4 + l) * 384;
-      gq.rows_per_wset = B * LATT; gq.M = rows; gq.Nout = 128; gq.K = CATT; gq.Yb = qk_set[cur][0]; gq.Yblo = qk_set[cur][1]; gq.ldyb = 128;
+      gq.rows_per_wset = B * LATT; gq.M = rows; gq.Nout = 128; gq.K = CATT; gq.Yb = s.qk[cur][0]; gq.Yblo = s.qk[cur][1]; gq.ldyb = 128;
       PZ_TRY(launch_split_rowgemm(gq, st));
       TcGemm gv = gq;  // v^T per cloud (K-major operand of P v)
       set_w(gv, wl + 128 * CATT); gv.bias[0] = gq.bias[0] + 128; gv.bias[1] = gq.bias[1] + 128;
-      gv.Nout = CATT; gv.Yb = nullptr; gv.Yblo = nullptr; gv.YT = vT_set[cur][0]; gv.YTlo = vT_set[cur][1]; gv.t_rows = LATT;
+      gv.Nout = CATT; gv.Yb = nullptr; gv.Yblo = nullptr; gv.YT = s.vT[cur][0]; gv.YTlo = s.vT[cur][1]; gv.t_rows = LATT;
       PZ_TRY(launch_split_rowgemm(gv, st));
       prof_mark("attn_qkv_proj", st);
     }
     AttnSplit ap;
-    ap.qk_hi = qk_set[cur][0]; ap.qk_lo = qk_set[cur][1]; ap.vT_hi = vT_set[cur][0]; ap.vT_lo = vT_set[cur][1];
-    ap.x_hi = cat_h[0] + xoff; ap.x_lo = cat_h[1] + xoff; ap.ldx = 1280; ap.r_hi = r_h[0]; ap.r_lo = r_h[1];
+    ap.qk_hi = s.qk[cur][0]; ap.qk_lo = s.qk[cur][1]; ap.vT_hi = s.vT[cur][0]; ap.vT_lo = s.vT[cur][1];
+    ap.x_hi = s.att_cat[0] + xoff; ap.x_lo = s.att_cat[1] + xoff; ap.ldx = 1280;
     ap.attn = o.attention; ap.attn_mode = o.attention ? (l == 0 ? 1 : (l == 3 ? 3 : 2)) : 0;
     ap.wo_hi[0] = wp_[0][0] + wl + 384 * CATT; ap.wo_lo[0] = wp_[0][1] + wl + 384 * CATT;
     ap.wo_hi[1] = wp_[1][0] + wl + 384 * CATT; ap.wo_lo[1] = wp_[1][1] + wl + 384 * CATT;
     ap.bo[0] = wa.o_b[l]; ap.bo[1] = wb.o_b[l]; ap.clouds_per_set = B;
-    ap.y_hi = cat_h[0] + (size_t)l * CATT; ap.y_lo = cat_h[1] + (size_t)l * CATT; ap.ldy = 1280;
+    ap.y_hi = s.att_cat[0] + (size_t)l * CATT; ap.y_lo = s.att_cat[1] + (size_t)l * CATT; ap.ldy = 1280;
     if (cat_f) { ap.yf = cat_f + (size_t)l * CATT; ap.ldyf = 1280; }
     if (l < 3) {   // the next layer's projections of these rows
       const size_t wn = WS_ATT + (size_t)(l + 1) * WS_ATT_STRIDE;
       ap.wqkv_hi[0] = wp_[0][0] + wn; ap.wqkv_lo[0] = wp_[0][1] + wn; ap.wqkv_hi[1] = wp_[1][0] + wn; ap.wqkv_lo[1] = wp_[1][1] + wn;
       ap.bqkv[0] = s.bqkv + (size_t)(l + 1) * 384; ap.bqkv[1] = s.bqkv + ((size_t)(E - 1) * 4 + l + 1) * 384;
-      ap.qk2_hi = qk_set[cur ^ 1][0]; ap.qk2_lo = qk_set[cur ^ 1][1]; ap.vT2_hi = vT_set[cur ^ 1][0]; ap.vT2_lo = vT_set[cur ^ 1][1];
-      ap.sig_flags = aflags + (size_t)l * C;
+      ap.qk2_hi = s.qk[cur ^ 1][0]; ap.qk2_lo = s.qk[cur ^ 1][1]; ap.vT2_hi = s.vT[cur ^ 1][0]; ap.vT2_lo = s.vT[cur ^ 1][1];
+      ap.sig_flags = s.flags + (size_t)l * C;
     }
-    if (l > 0) ap.dep_flags = aflags + (size_t)(l - 1) * C;
+    if (l > 0) ap.dep_flags = s.flags + (size_t)(l - 1) * C;
     PZ_TRY(launch_attention_split(ap, C, st));
     prof_mark("attn_softmax_av", st);
   }
   // ---- tail: Linear(1280, 1024), then the max over the 256 points of a cloud
-  {
-    float* fg = o.f_global ? o.f_global : s.fglob;
-    TcGemm g;
-    g.X = cat_h[0]; g.Xlo = cat_h[1]; g.ldx = 1280; set_w(g, WS_WOUT); g.ldw = 1280;
-    g.bias[0] = wa.out_b; g.bias[1] = wb.out_b; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = 1024; g.K = 1280;
-    if (o.out) { g.Yf = o.out; g.ldyf = 1024; }
-    g.Ymax = s.tailp; g.ldmax = 1024;            // per 128-row tile column maxima: two tiles per cloud
-    PZ_TRY(launch_split_rowgemm(g, st));
-    prof_mark("tail_linear_maxpool", st);
-    PZ_CUDA(launch_pdl(rowblock_max_kernel, dim3(4, C), dim3(256), 0, st, (const float*)s.tailp, 1024, LATT / 128, 1024, C, C, 0, fg, 1024));
-    PZ_LAUNCH_CHECK();
-    prof_mark("tail_point_max", st);
-    if (fglob_pair)
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair, (size_t)E * 1024 * sizeof(float), fg, 1024 * sizeof(float),
-                                1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
-    if (fglob_pair && E == 2)
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair + 1024, (size_t)E * 1024 * sizeof(float), fg + (size_t)B * 1024,
-                                1024 * sizeof(float), 1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
-  }
+  TcGemm g;
+  g.X = s.att_cat[0]; g.Xlo = s.att_cat[1]; g.ldx = 1280; set_w(g, WS_WOUT); g.ldw = 1280;
+  g.bias[0] = wa.out_b; g.bias[1] = wb.out_b; g.rows_per_wset = B * LATT; g.M = rows; g.Nout = 1024; g.K = 1280;
+  if (o.out) { g.Yf = o.out; g.ldyf = 1024; }
+  g.Ymax = s.tilemax; g.ldmax = 1024;           // per 128-row tile column maxima: two tiles per cloud
+  PZ_TRY(launch_split_rowgemm(g, st));
+  prof_mark("tail_linear_maxpool", st);
+  PZ_CUDA(launch_pdl(rowblock_max_kernel, dim3(4, C), dim3(256), 0, st, (const float*)s.tilemax, 1024, LATT / 128, 1024, C, C, 0,
+                     c.fglob, 1024));
+  PZ_LAUNCH_CHECK();
+  prof_mark("tail_point_max", st);
   return 0;
 }
 
-// fglob_pair: optional [B, E*1024] destination laid out for the pose MLP's concat (model5_b.py:723)
-static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
-                                const int64_t* start2, int precision, const PzEncoderOutputs& o, void* ws,
-                                size_t ws_bytes, float* fglob_pair, const float** xfeat_out, const AfterStem* after_stem,
-                                bool reuse_pack, cudaStream_t st) {
-  PZ_REQUIRE(E == 1 || E == 2, PZ_ERR_ARG, "encoder: E must be 1 or 2 (got %d)", E);
-  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "encoder: B must be >= 1");
-  PZ_REQUIRE((long long)E * B <= PZ_MAX_CLOUDS, PZ_ERR_UNSUPPORTED, "encoder: E*B = %lld clouds > %d", (long long)E * B,
-             PZ_MAX_CLOUDS);
-  PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
-             "encoder: unknown precision %d", precision);
-  for (int e = 0; e < E; ++e)
-    PZ_REQUIRE(encoder_weights_ok(w[e]), PZ_ERR_ARG, "encoder: weight set %d has a null pointer", e);
+// fp32 path (PZ_PREC_FP32): every tensor and product in fp32 on the CUDA cores (stem_kernel, gemm_f32.cu)
+static int encoder_forward_fp32(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
+                                const int64_t* start2, const PzEncoderOutputs& o, const EncoderCommon& c,
+                                const Fp32Scratch& s, const AfterStem* after_stem, cudaStream_t st) {
   const int C = E * B;
-  Arena arena(ws, ws_bytes);
-  EncoderScratch s;
-  encoder_scratch_layout(C, arena, s);
-  PZ_REQUIRE(ws && arena.ok(), PZ_ERR_WORKSPACE, "encoder: workspace %zu B < required %zu B", ws_bytes, arena.used);
-  if (precision == PZ_PREC_BF16)
-    return encoder_forward_bf16(w, E, B, xyz, start1, start2, o, s, fglob_pair, xfeat_out, after_stem, reuse_pack, st);
-  if (precision == PZ_PREC_SPLIT)
-    return encoder_forward_split(w, E, B, xyz, start1, start2, o, s, fglob_pair, xfeat_out, after_stem, reuse_pack, st);
   const PzEncoderWeights& wa = w[0];
   const PzEncoderWeights& wb = w[E - 1];
-  float* xfeat = o.x_feature ? o.x_feature : s.xfeat;
   float* f1f = o.f1f ? o.f1f : s.f1f;
   float* att_cat = o.att_cat ? o.att_cat : s.att_cat;
-  float* nx2 = o.x2 ? o.x2 : s.nx2;
-  if (xfeat_out) *xfeat_out = xfeat;
 
   // stem: Linear(3,64)+BN+ReLU, Linear(64,64)+BN+ReLU -> x_feature [C,1024,64]
-  stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, xfeat);
+  stem_kernel<<<C * NPTS / 128, 128, 0, st>>>(xyz, stem_of(wa), stem_of(wb), B, c.xfeat);
   PZ_LAUNCH_CHECK();
   prof_mark("stem", st);
-  if (after_stem) PZ_TRY((*after_stem)(xfeat));
+  if (after_stem) PZ_TRY((*after_stem)(c.xfeat));
 
   // ---- stage 1: FPS 1024->512, kNN 32, grouped MLP 67->128->128, max over K
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, s.nx1, st));
+  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, st));
   prof_mark("fps1", st);
-  PZ_TRY(launch_knn(s.nx1, xyz, C, S1, NPTS, KNN, o.knn1, s.knn1r, nullptr, st));
+  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, st));
   prof_mark("knn1", st);
   {
     GemmF32 g;  // F1 = x_feature * mlp3.weight[:, 3:]^T   (bias + xyz part are added per neighbour)
-    g.A = xfeat; g.lda = D0; g.W[0] = wa.mlp3_w + 3; g.W[1] = wb.mlp3_w + 3; g.ldw = 3 + D0;
+    g.A = c.xfeat; g.lda = D0; g.W[0] = wa.mlp3_w + 3; g.W[1] = wb.mlp3_w + 3; g.ldw = 3 + D0;
     g.rows_per_wset = B * NPTS; g.Y = s.F1; g.ldy = C1A; g.M = C * NPTS; g.N = C1A; g.K = D0;
     PZ_TRY(launch_gemm_f32(g, st));
     prof_mark("sg1_layer1", st);
   }
   {
     GemmF32 g;
-    g.A = s.F1; g.lda = C1A; g.rows = s.knn1r; g.xyz = xyz; g.centers = s.nx1;
+    g.A = s.F1; g.lda = C1A; g.rows = c.knn1r; g.xyz = xyz; g.centers = c.nx1;
     g.W1[0] = wa.mlp3_w; g.W1[1] = wb.mlp3_w; g.b1[0] = wa.mlp3_b; g.b1[1] = wb.mlp3_b; g.ldw1 = 3 + D0;
     g.W[0] = wa.mlp4_w; g.W[1] = wb.mlp4_w; g.bias[0] = wa.mlp4_b; g.bias[1] = wb.mlp4_b; g.ldw = C1A;
     g.rows_per_wset = B * S1 * KNN; g.Y = f1f; g.ldy = C1B; g.M = C * S1 * KNN; g.N = C1B; g.K = C1A;
@@ -1339,9 +1283,9 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
     prof_mark("sg1_gather_layer2_maxpool", st);
   }
   // ---- stage 2: FPS 512->256 on the stage-1 centroids, kNN 32, grouped MLP 131->256->256
-  PZ_TRY(launch_fps(s.nx1, C, S1, start2, S2, o.fps2, nullptr, nx2, st));
+  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, st));
   prof_mark("fps2", st);
-  PZ_TRY(launch_knn(nx2, s.nx1, C, S2, S1, KNN, o.knn2, s.knn2r, nullptr, st));
+  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, st));
   prof_mark("knn2", st);
   {
     GemmF32 g;
@@ -1353,7 +1297,7 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
   float* f2f_slot = att_cat + 4 * CATT;  // cat([att1..att4, f2f]) (model5_b.py:467,472): f2f is columns 1024..1279
   {
     GemmF32 g;
-    g.A = s.F2; g.lda = C2A; g.rows = s.knn2r; g.xyz = s.nx1; g.centers = nx2;
+    g.A = s.F2; g.lda = C2A; g.rows = c.knn2r; g.xyz = c.nx1; g.centers = c.nx2;
     g.W1[0] = wa.mlp5_w; g.W1[1] = wb.mlp5_w; g.b1[0] = wa.mlp5_b; g.b1[1] = wb.mlp5_b; g.ldw1 = 3 + C1B;
     g.W[0] = wa.mlp6_w; g.W[1] = wb.mlp6_w; g.bias[0] = wa.mlp6_b; g.bias[1] = wb.mlp6_b; g.ldw = C2A;
     g.rows_per_wset = B * S2 * KNN; g.Y = f2f_slot; g.ldy = 1280; g.M = C * S2 * KNN; g.N = C2B; g.K = C2A;
@@ -1361,9 +1305,6 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
     PZ_TRY(launch_gemm_f32(g, st));
     prof_mark("sg2_gather_layer2_maxpool", st);
   }
-  if (o.f2f)
-    PZ_CUDA(cudaMemcpy2DAsync(o.f2f, CATT * sizeof(float), f2f_slot, 1280 * sizeof(float), CATT * sizeof(float),
-                              (size_t)C * LATT, cudaMemcpyDeviceToDevice, st));
 
   // ---- 4 x offset attention (model5_b.py:92-101); layer i writes att_cat[:, i*256:(i+1)*256]
   const int rows = C * LATT;
@@ -1391,31 +1332,65 @@ static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const f
   }
 
   // ---- tail: Linear(1280,1024) then max over the 256 points (model5_b.py:472-475)
-  {
-    GemmF32 g;
-    g.A = att_cat; g.lda = 1280; g.W[0] = wa.out_w; g.W[1] = wb.out_w; g.bias[0] = wa.out_b; g.bias[1] = wb.out_b;
-    g.ldw = 1280; g.rows_per_wset = B * LATT; g.M = rows; g.N = 1024; g.K = 1280;
-    float* fg = o.f_global ? o.f_global : s.fglob;
-    if (o.out) {
-      g.Y = o.out; g.ldy = 1024;
-      PZ_TRY(launch_gemm_f32(g, st));
-      prof_mark("tail_linear", st);
-      rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(o.out, 1024, LATT, 1024, C, C, 0, fg, 1024);
-    } else {
-      g.Y = s.tailp; g.ldy = 1024; g.group = 128;
-      PZ_TRY(launch_gemm_f32(g, st));
-      prof_mark("tail_linear_maxpool", st);
-      rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(s.tailp, 1024, LATT / 128, 1024, C, C, 0, fg, 1024);
-    }
-    PZ_LAUNCH_CHECK();
-    prof_mark("tail_point_max", st);
-    if (fglob_pair)  // [B, E*1024]: pair b = [f_global(cloud b), f_global(cloud B+b)]
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair, (size_t)E * 1024 * sizeof(float), fg, 1024 * sizeof(float),
-                                1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
-    if (fglob_pair && E == 2)
-      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair + 1024, (size_t)E * 1024 * sizeof(float), fg + (size_t)B * 1024,
-                                1024 * sizeof(float), 1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
+  GemmF32 g;
+  g.A = att_cat; g.lda = 1280; g.W[0] = wa.out_w; g.W[1] = wb.out_w; g.bias[0] = wa.out_b; g.bias[1] = wb.out_b;
+  g.ldw = 1280; g.rows_per_wset = B * LATT; g.M = rows; g.N = 1024; g.K = 1280;
+  if (o.out) {
+    g.Y = o.out; g.ldy = 1024;
+    PZ_TRY(launch_gemm_f32(g, st));
+    prof_mark("tail_linear", st);
+    rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(o.out, 1024, LATT, 1024, C, C, 0, c.fglob, 1024);
+  } else {
+    g.Y = s.tilemax; g.ldy = 1024; g.group = 128;
+    PZ_TRY(launch_gemm_f32(g, st));
+    prof_mark("tail_linear_maxpool", st);
+    rowblock_max_kernel<<<dim3(4, C), 256, 0, st>>>(s.tilemax, 1024, LATT / 128, 1024, C, C, 0, c.fglob, 1024);
   }
+  PZ_LAUNCH_CHECK();
+  prof_mark("tail_point_max", st);
+  return 0;
+}
+
+// fglob_pair: optional [B, E*1024] destination laid out for the pose MLP's concat (model5_b.py:723)
+static int encoder_forward_impl(const PzEncoderWeights* w, int E, int B, const float* xyz, const int64_t* start1,
+                                const int64_t* start2, int precision, const PzEncoderOutputs& o, void* ws,
+                                size_t ws_bytes, float* fglob_pair, const AfterStem* after_stem, bool reuse_pack,
+                                cudaStream_t st) {
+  PZ_REQUIRE(E == 1 || E == 2, PZ_ERR_ARG, "encoder: E must be 1 or 2 (got %d)", E);
+  PZ_REQUIRE(B >= 1, PZ_ERR_ARG, "encoder: B must be >= 1");
+  PZ_REQUIRE((long long)E * B <= PZ_MAX_CLOUDS, PZ_ERR_UNSUPPORTED, "encoder: E*B = %lld clouds > %d", (long long)E * B,
+             PZ_MAX_CLOUDS);
+  PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
+             "encoder: unknown precision %d", precision);
+  for (int e = 0; e < E; ++e)
+    PZ_REQUIRE(encoder_weights_ok(w[e]), PZ_ERR_ARG, "encoder: weight set %d has a null pointer", e);
+  const int C = E * B;
+  Arena arena(ws, ws_bytes);
+  EncoderCommon c;
+  Fp32Scratch f = {}; Bf16Scratch b = {}; SplitScratch x = {};
+  carve(C, arena, c);
+  if (precision == PZ_PREC_FP32) carve(C, arena, f);
+  else if (precision == PZ_PREC_BF16) carve(C, arena, b);
+  else carve(C, arena, x);
+  PZ_REQUIRE(ws && arena.ok(), PZ_ERR_WORKSPACE, "encoder: workspace %zu B < required %zu B", ws_bytes, arena.used);
+  if (o.x_feature) c.xfeat = o.x_feature;
+  if (o.x2) c.nx2 = o.x2;
+  if (o.f_global) c.fglob = o.f_global;
+
+  if (precision == PZ_PREC_FP32) PZ_TRY(encoder_forward_fp32(w, E, B, xyz, start1, start2, o, c, f, after_stem, st));
+  else if (precision == PZ_PREC_BF16) PZ_TRY(encoder_forward_bf16(w, E, B, xyz, start1, start2, o, c, b, after_stem, reuse_pack, st));
+  else PZ_TRY(encoder_forward_split(w, E, B, xyz, start1, start2, o, c, x, after_stem, reuse_pack, st));
+
+  // f2f = att_cat[:, 1024:1280].  The fp32 path always assembles an fp32 att_cat; without one the tensor-core paths' stage-2
+  // GEMM has written f2f directly.
+  const float* cat = o.att_cat ? o.att_cat : precision == PZ_PREC_FP32 ? f.att_cat : nullptr;
+  if (o.f2f && cat)
+    PZ_CUDA(cudaMemcpy2DAsync(o.f2f, CATT * sizeof(float), cat + 4 * CATT, 1280 * sizeof(float), CATT * sizeof(float),
+                              (size_t)C * LATT, cudaMemcpyDeviceToDevice, st));
+  if (fglob_pair)  // [B, E*1024]: pair b = [f_global(cloud b), f_global(cloud B+b)]
+    for (int e = 0; e < E; ++e)
+      PZ_CUDA(cudaMemcpy2DAsync(fglob_pair + (size_t)e * 1024, (size_t)E * 1024 * sizeof(float), c.fglob + (size_t)e * B * 1024,
+                                1024 * sizeof(float), 1024 * sizeof(float), B, cudaMemcpyDeviceToDevice, st));
   return 0;
 }
 
@@ -1434,9 +1409,14 @@ using namespace pz;
 // ------------------------------------------------------------------------------ C ABI
 extern "C" size_t pz_encoder_workspace_bytes(int E, int B) {
   if (E < 1 || B < 1) return 0;
-  Arena a(nullptr, 0);
-  EncoderScratch s;
-  return align_up(encoder_scratch_layout(E * B, a, s), 256);
+  auto bytes = [&](auto&& s) {   // the common part, then one precision's layout
+    Arena a(nullptr, 0);
+    EncoderCommon c;
+    carve(E * B, a, c);
+    carve(E * B, a, s);
+    return a.used;
+  };
+  return align_up(std::max({bytes(Fp32Scratch()), bytes(Bf16Scratch()), bytes(SplitScratch())}), 256);
 }
 
 extern "C" int pz_encoder_forward(const PzEncoderWeights* weights_host, int E, int B, const float* xyz,
@@ -1446,16 +1426,17 @@ extern "C" int pz_encoder_forward(const PzEncoderWeights* weights_host, int E, i
   PZ_REQUIRE(weights_host && xyz && start1 && start2 && outputs_host, PZ_ERR_ARG, "pz_encoder_forward: null pointer");
   prof_begin(as_stream(stream));
   return encoder_forward_impl(weights_host, E, B, xyz, start1, start2, precision, *outputs_host, workspace,
-                              workspace_bytes, nullptr, nullptr, nullptr, false, as_stream(stream));
+                              workspace_bytes, nullptr, nullptr, false, as_stream(stream));
 }
 
 namespace {
 struct PredictScratch {
-  float *xyz, *fpair, *h0, *h1, *partial, *local, *gmax, *gbias, *tilemax;
+  float *xyz, *fpair, *h0, *h1, *local, *gmax, *gbias, *tilemax;
+  float *x2_all, *attn_all;   // need mode: the encoder's [2B,256,3] / [2B,256,256] outputs, copied out per half
   __nv_bfloat16* himg_split;
   int64_t *st1, *st2;
   void* enc;
-  size_t enc_bytes, partial_floats;
+  size_t enc_bytes;
 };
 size_t predict_layout(int B, Arena& a, PredictScratch& s) {
   s.xyz = a.take<float>((size_t)2 * B * NPTS * 3);
@@ -1464,12 +1445,12 @@ size_t predict_layout(int B, Arena& a, PredictScratch& s) {
   s.fpair = a.take<float>((size_t)B * 2048);
   s.h0 = a.take<float>((size_t)B * 1024);
   s.h1 = a.take<float>((size_t)B * 1024);
-  s.partial_floats = (size_t)16 * B * 1024;
-  s.partial = a.take<float>(s.partial_floats);
   s.local = a.take<float>((size_t)2 * B * NPTS * 64);
   s.gmax = a.take<float>((size_t)B * 64);
   s.gbias = a.take<float>((size_t)2 * B * 64);
   s.tilemax = a.take<float>((size_t)2 * B * 8 * 128);
+  s.x2_all = a.take<float>((size_t)2 * B * S2 * 3);
+  s.attn_all = a.take<float>((size_t)2 * B * LATT * LATT);
   s.himg_split = a.take<__nv_bfloat16>(2 * HEAD_SPLIT_IMG_SET);
   s.enc_bytes = pz_encoder_workspace_bytes(2, B);
   s.enc = a.take<char>(s.enc_bytes);
@@ -1561,7 +1542,7 @@ int predict_front(const PzEncoderWeights* enc_host, const PzHeadWeights& h, cons
   };
 
   return encoder_forward_impl(enc_host, 2, B, s.xyz, s.st1, s.st2, precision, eo, s.enc, s.enc_bytes, fglob_pair,
-                              nullptr, &heads_fn, reuse_pack, st);
+                              &heads_fn, reuse_pack, st);
 }
 
 // null-pointer check of every head weight
@@ -1574,11 +1555,11 @@ int check_heads(const PzHeadWeights* heads_host, const char* who) {
 
 // pose MLP on rows of cat(ffpc, fmrpc) (model5_b.py:723-725): 2048-1024-512-512-256-6, fp32 in every precision
 int pose_mlp(const PzHeadWeights& h, const float* fpair, int n, float* h0, float* h1, float* out6, cudaStream_t st) {
-  PZ_TRY(skinny_linear(fpair, 2048, h.tf_w[0], h.tf_b[0], n, 1024, 2048, 1, h0, 1024, nullptr, 0, st));
-  PZ_TRY(skinny_linear(h0, 1024, h.tf_w[1], h.tf_b[1], n, 512, 1024, 1, h1, 512, nullptr, 0, st));
-  PZ_TRY(skinny_linear(h1, 512, h.tf_w[2], h.tf_b[2], n, 512, 512, 1, h0, 512, nullptr, 0, st));
-  PZ_TRY(skinny_linear(h0, 512, h.tf_w[3], h.tf_b[3], n, 256, 512, 1, h1, 256, nullptr, 0, st));
-  PZ_TRY(skinny_linear(h1, 256, h.tf_w[4], h.tf_b[4], n, 6, 256, 0, out6, 6, nullptr, 0, st));
+  PZ_TRY(skinny_linear(fpair, 2048, h.tf_w[0], h.tf_b[0], n, 1024, 2048, 1, h0, 1024, st));
+  PZ_TRY(skinny_linear(h0, 1024, h.tf_w[1], h.tf_b[1], n, 512, 1024, 1, h1, 512, st));
+  PZ_TRY(skinny_linear(h1, 512, h.tf_w[2], h.tf_b[2], n, 512, 512, 1, h0, 512, st));
+  PZ_TRY(skinny_linear(h0, 512, h.tf_w[3], h.tf_b[3], n, 256, 512, 1, h1, 256, st));
+  PZ_TRY(skinny_linear(h1, 256, h.tf_w[4], h.tf_b[4], n, 6, 256, 0, out6, 6, st));
   prof_mark("pose_mlp", st);
   return 0;
 }
@@ -1606,26 +1587,19 @@ extern "C" int pz_predict5(const PzEncoderWeights* enc_host, const PzHeadWeights
              workspace_bytes, arena.used);
   prof_begin(st);
   PzEncoderOutputs eo = {};
-  float* x2_all = nullptr;
-  float* attn_all = nullptr;
-  // need=True: the encoder writes contiguous [2B,..] tensors but the caller's four outputs are
-  // separate, so attention [2B,256,256] and x2 [2B,256,3] go through scratch that is free until
-  // the heads run (`local`, `partial`) and are copied out per half.
-  if (need) {
-    attn_all = s.local;                                    // 2B*65536 floats == 2B*1024*64
-    x2_all = s.partial;                                    // 2B*768 floats  <= 16*B*1024
-    eo.attention = attn_all;
-    eo.x2 = x2_all;
+  if (need) {   // the encoder writes contiguous [2B,..] tensors; the caller's four outputs are separate
+    eo.attention = s.attn_all;
+    eo.x2 = s.x2_all;
   }
   const PzHeadWeights& h = *heads_host;
   PZ_TRY(predict_front(enc_host, h, fpc, mrpc, B, starts, precision, reuse_pack, s, eo, s.fpair, s.local, s.tilemax,
                        de_fpcb, de_mrpcb, st));
   if (need) {
     const size_t ab = (size_t)B * LATT * LATT * sizeof(float), xb = (size_t)B * S2 * 3 * sizeof(float);
-    PZ_CUDA(cudaMemcpyAsync(attention_fpc, attn_all, ab, cudaMemcpyDeviceToDevice, st));
-    PZ_CUDA(cudaMemcpyAsync(attention_mrpc, attn_all + (size_t)B * LATT * LATT, ab, cudaMemcpyDeviceToDevice, st));
-    PZ_CUDA(cudaMemcpyAsync(x2_fpc, x2_all, xb, cudaMemcpyDeviceToDevice, st));
-    PZ_CUDA(cudaMemcpyAsync(x2_mrpc, x2_all + (size_t)B * S2 * 3, xb, cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(attention_fpc, s.attn_all, ab, cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(attention_mrpc, s.attn_all + (size_t)B * LATT * LATT, ab, cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(x2_fpc, s.x2_all, xb, cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(x2_mrpc, s.x2_all + (size_t)B * S2 * 3, xb, cudaMemcpyDeviceToDevice, st));
   }
   return pose_mlp(h, s.fpair, B, s.h0, s.h1, out6, st);
 }
@@ -1800,17 +1774,45 @@ extern "C" int pz_linear(const float* x, int ldx, const float* W, const float* b
   return launch_gemm_f32(g, as_stream(stream));
 }
 
+namespace {
+// pz_offset_attention's workspace: one layout per precision over rows = B * L rows of C channels
+struct OffsetAttnFp32 { float *q, *k, *v, *r; };
+size_t layout(Arena& a, size_t rows, int C, OffsetAttnFp32& s) {
+  s.q = a.take<float>(rows * (C / 4));
+  s.k = a.take<float>(rows * (C / 4));
+  s.v = a.take<float>(rows * C);
+  s.r = a.take<float>(rows * C);
+  return a.used;
+}
+// bf16: x and out, one layer's weight tile images, the q|k|v bias
+struct OffsetAttnBf16 { __nv_bfloat16 *x, *y, *wimg; float* bqkv; };
+size_t layout(Arena& a, size_t rows, int C, OffsetAttnBf16& s) {
+  s.x = a.take<__nv_bfloat16>(rows * C);
+  s.y = a.take<__nv_bfloat16>(rows * C);
+  s.wimg = a.take<__nv_bfloat16>(ATTN_WIMG_ELEMS);
+  s.bqkv = a.take<float>(384);
+  return a.used;
+}
+// split, [plane]: x, q|k, v^T, r, the four weights (rows: q 0-63, k 64-127, v 128-383, o 384-639), the q|k|v bias
+struct OffsetAttnSplit { h16 *x[2], *qk[2], *vT[2], *r[2], *w[2]; float* bqkv; };
+size_t layout(Arena& a, size_t rows, int C, OffsetAttnSplit& s) {
+  s.x[0] = a.take<h16>(rows * C); s.x[1] = a.take<h16>(rows * C);
+  s.qk[0] = a.take<h16>(rows * 128); s.qk[1] = a.take<h16>(rows * 128);
+  s.vT[0] = a.take<h16>(rows * C); s.vT[1] = a.take<h16>(rows * C);
+  s.r[0] = a.take<h16>(rows * C); s.r[1] = a.take<h16>(rows * C);
+  s.w[0] = a.take<h16>((size_t)640 * C); s.w[1] = a.take<h16>((size_t)640 * C);
+  s.bqkv = a.take<float>(384);
+  return a.used;
+}
+}  // namespace
+
 extern "C" size_t pz_offset_attention_workspace_bytes(int B, int L, int C) {
   if (B < 1 || L < 1 || C < 4) return 0;
-  const size_t rows = (size_t)B * L;
-  // fp32 path: q, k, v, r;  bf16 path (L == 256): x and out as bf16, one layer's weight tile images, the q|k|v bias
-  const size_t fp32_path = align_up(rows * (C / 4) * sizeof(float), 256) * 2 + align_up(rows * C * sizeof(float), 256) * 2;
-  const size_t bf16_path = align_up(rows * C * 2, 256) * 2 + align_up(ATTN_WIMG_ELEMS * 2, 256) + align_up(384 * 4, 256);
-  // split path: planes of x, q|k, v^T, r, the four weights, the q|k|v bias
-  const size_t split_path = align_up(rows * C * 2, 256) * 6 + align_up(rows * 128 * 2, 256) * 2 + align_up((size_t)640 * C * 2, 256) * 2 +
-                            align_up(384 * 4, 256);
-  const size_t m = fp32_path > bf16_path ? fp32_path : bf16_path;
-  return (m > split_path ? m : split_path) + 256;
+  auto bytes = [&](auto&& s) {
+    Arena a(nullptr, 0);
+    return layout(a, (size_t)B * L, C, s);
+  };
+  return align_up(std::max({bytes(OffsetAttnFp32()), bytes(OffsetAttnBf16()), bytes(OffsetAttnSplit())}), 256);
 }
 
 extern "C" int pz_offset_attention(const float* x, const float* Wq, const float* bq, const float* Wk, const float* bk,
@@ -1823,107 +1825,115 @@ extern "C" int pz_offset_attention(const float* x, const float* Wq, const float*
              "pz_offset_attention: unknown precision %d", precision);
   cudaStream_t st = as_stream(stream);
   Arena a(workspace, workspace_bytes);
+  PZ_REQUIRE(precision == PZ_PREC_FP32 || L == 256, PZ_ERR_UNSUPPORTED, "pz_offset_attention(%s): L must be 256 (got %d)",
+             precision == PZ_PREC_SPLIT ? "split" : "bf16", L);
   const size_t rows = (size_t)B * L;
+  OffsetAttnFp32 f = {}; OffsetAttnBf16 b = {}; OffsetAttnSplit s = {};
+  if (precision == PZ_PREC_SPLIT) layout(a, rows, C, s);
+  else if (precision == PZ_PREC_BF16) layout(a, rows, C, b);
+  else layout(a, rows, C, f);
+  PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_offset_attention: workspace %zu B < required %zu B",
+             workspace_bytes, a.used);
   if (precision == PZ_PREC_SPLIT) {   // the split path's layer: row GEMMs + attention_split_kernel (gemm_split.cu, attention_split.cu)
-    PZ_REQUIRE(L == 256, PZ_ERR_UNSUPPORTED, "pz_offset_attention(split): L must be 256 (got %d)", L);
-    typedef __nv_bfloat16 h16;
-    h16* xh = a.take<h16>(rows * C); h16* xl = a.take<h16>(rows * C);
-    h16* qkh = a.take<h16>(rows * 128); h16* qkl = a.take<h16>(rows * 128);
-    h16* vth = a.take<h16>(rows * C); h16* vtl = a.take<h16>(rows * C);
-    h16* rh = a.take<h16>(rows * C); h16* rl = a.take<h16>(rows * C);
-    h16* wh = a.take<h16>((size_t)640 * C); h16* wl = a.take<h16>((size_t)640 * C);   // rows: q 0-63, k 64-127, v 128-383, o 384-639
-    float* bqkv = a.take<float>(384);
-    PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_offset_attention: workspace %zu B < required %zu B",
-               workspace_bytes, a.used);
     PackJobs jobs;
     int n = 0;
     for (int pl = 0; pl < 2; ++pl) {
-      h16* w = pl == 0 ? wh : wl;
+      h16* w = s.w[pl];
       jobs.j[n++] = PackJob{Wq, w, C, 64, C, C, 4 + pl};
       jobs.j[n++] = PackJob{Wk, w + 64 * C, C, 64, C, C, 4 + pl};
       jobs.j[n++] = PackJob{Wv, w + 128 * C, C, C, C, C, 4 + pl};
       jobs.j[n++] = PackJob{Wo, w + 384 * C, C, C, C, C, 4 + pl};
     }
-    jobs.j[n++] = PackJob{bq, bqkv, 64, 1, 64, 64, 0};
-    jobs.j[n++] = PackJob{bk, bqkv + 64, 64, 1, 64, 64, 0};
-    jobs.j[n++] = PackJob{bv, bqkv + 128, C, 1, C, C, 0};
+    jobs.j[n++] = PackJob{bq, s.bqkv, 64, 1, 64, 64, 0};
+    jobs.j[n++] = PackJob{bk, s.bqkv + 64, 64, 1, 64, 64, 0};
+    jobs.j[n++] = PackJob{bv, s.bqkv + 128, C, 1, C, C, 0};
     jobs.n = n;
     pack_weights_kernel<<<dim3(16, n), 256, 0, st>>>(jobs);
     PZ_LAUNCH_CHECK();
-    PZ_TRY(launch_split_planes(x, C, rows, C, xh, xl, C, st));
+    PZ_TRY(launch_split_planes(x, C, rows, C, s.x[0], s.x[1], C, st));
     TcGemm gq;
-    gq.X = xh; gq.Xlo = xl; gq.ldx = C; gq.W[0] = wh; gq.Wlo[0] = wl; gq.ldw = C; gq.bias[0] = bqkv;
-    gq.M = (int)rows; gq.Nout = 128; gq.K = C; gq.Yb = qkh; gq.Yblo = qkl; gq.ldyb = 128;
+    gq.X = s.x[0]; gq.Xlo = s.x[1]; gq.ldx = C; gq.W[0] = s.w[0]; gq.Wlo[0] = s.w[1]; gq.ldw = C; gq.bias[0] = s.bqkv;
+    gq.M = (int)rows; gq.Nout = 128; gq.K = C; gq.Yb = s.qk[0]; gq.Yblo = s.qk[1]; gq.ldyb = 128;
     PZ_TRY(launch_split_rowgemm(gq, st));
     TcGemm gv = gq;
-    gv.W[0] = wh + 128 * C; gv.Wlo[0] = wl + 128 * C; gv.bias[0] = bqkv + 128; gv.Nout = C; gv.Yb = nullptr; gv.Yblo = nullptr;
-    gv.YT = vth; gv.YTlo = vtl; gv.t_rows = L;
+    gv.W[0] = s.w[0] + 128 * C; gv.Wlo[0] = s.w[1] + 128 * C; gv.bias[0] = s.bqkv + 128; gv.Nout = C; gv.Yb = nullptr; gv.Yblo = nullptr;
+    gv.YT = s.vT[0]; gv.YTlo = s.vT[1]; gv.t_rows = L;
     PZ_TRY(launch_split_rowgemm(gv, st));
     AttnSplit ap;
-    ap.qk_hi = qkh; ap.qk_lo = qkl; ap.vT_hi = vth; ap.vT_lo = vtl; ap.x_hi = xh; ap.x_lo = xl; ap.ldx = C; ap.r_hi = rh; ap.r_lo = rl;
+    ap.qk_hi = s.qk[0]; ap.qk_lo = s.qk[1]; ap.vT_hi = s.vT[0]; ap.vT_lo = s.vT[1]; ap.x_hi = s.x[0]; ap.x_lo = s.x[1]; ap.ldx = C;
+    ap.r_hi = s.r[0]; ap.r_lo = s.r[1];
     ap.attn = attention_or_null; ap.attn_mode = attention_or_null ? 1 : 0;
     PZ_TRY(launch_attention_split(ap, B, st));
     TcGemm go;
-    go.X = rh; go.Xlo = rl; go.ldx = C; go.W[0] = wh + 384 * C; go.Wlo[0] = wl + 384 * C; go.ldw = C; go.bias[0] = bo;
+    go.X = s.r[0]; go.Xlo = s.r[1]; go.ldx = C; go.W[0] = s.w[0] + 384 * C; go.Wlo[0] = s.w[1] + 384 * C; go.ldw = C; go.bias[0] = bo;
     go.M = (int)rows; go.Nout = C; go.K = C; go.relu = 1; go.Rf = x; go.ldrf = C; go.Yf = out; go.ldyf = C;
     return launch_split_rowgemm(go, st);
   }
   if (precision == PZ_PREC_BF16) {   // the fused tcgen05 layer kernel predict5 uses (attention_layer_tc.cu)
-    PZ_REQUIRE(L == 256, PZ_ERR_UNSUPPORTED, "pz_offset_attention(bf16): L must be 256 (got %d)", L);
-    __nv_bfloat16* xb = a.take<__nv_bfloat16>(rows * C);
-    __nv_bfloat16* yb = a.take<__nv_bfloat16>(rows * C);
-    __nv_bfloat16* wimg = a.take<__nv_bfloat16>(ATTN_WIMG_ELEMS);
-    float* bqkv = a.take<float>(384);
-    PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_offset_attention: workspace %zu B < required %zu B",
-               workspace_bytes, a.used);
-    PZ_TRY(launch_cvt_bf16(x, C, (int)rows, C, xb, C, st));
-    PZ_TRY(launch_attn_weight_image(Wq, 64, 0, wimg, st));
-    PZ_TRY(launch_attn_weight_image(Wk, 64, 64, wimg, st));
-    PZ_TRY(launch_attn_weight_image(Wv, C, 128, wimg, st));
-    PZ_TRY(launch_attn_weight_image(Wo, C, 384, wimg, st));
-    PZ_CUDA(cudaMemcpyAsync(bqkv, bq, 64 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    PZ_CUDA(cudaMemcpyAsync(bqkv + 64, bk, 64 * sizeof(float), cudaMemcpyDeviceToDevice, st));
-    PZ_CUDA(cudaMemcpyAsync(bqkv + 128, bv, C * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    PZ_TRY(launch_cvt_bf16(x, C, (int)rows, C, b.x, C, st));
+    PZ_TRY(launch_attn_weight_image(Wq, 64, 0, b.wimg, st));
+    PZ_TRY(launch_attn_weight_image(Wk, 64, 64, b.wimg, st));
+    PZ_TRY(launch_attn_weight_image(Wv, C, 128, b.wimg, st));
+    PZ_TRY(launch_attn_weight_image(Wo, C, 384, b.wimg, st));
+    PZ_CUDA(cudaMemcpyAsync(b.bqkv, bq, 64 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(b.bqkv + 64, bk, 64 * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    PZ_CUDA(cudaMemcpyAsync(b.bqkv + 128, bv, C * sizeof(float), cudaMemcpyDeviceToDevice, st));
     AttnLayerTc p;
     p.nlayers = 1;
-    p.x = xb; p.ldx = C; p.wimg[0] = p.wimg[1] = wimg; p.bqkv[0] = p.bqkv[1] = bqkv; p.bo[0][0] = p.bo[1][0] = bo;
-    p.clouds_per_set = B; p.yb = yb; p.ldyb = C; p.yf = out; p.ldyf = C;
+    p.x = b.x; p.ldx = C; p.wimg[0] = p.wimg[1] = b.wimg; p.bqkv[0] = p.bqkv[1] = b.bqkv; p.bo[0][0] = p.bo[1][0] = bo;
+    p.clouds_per_set = B; p.yb = b.y; p.ldyb = C; p.yf = out; p.ldyf = C;
     p.attn = attention_or_null; p.attn_mode[0] = attention_or_null ? 1 : 0;
     return launch_attention_layer_tc(p, B, st);
   }
-  float* q = a.take<float>(rows * (C / 4));
-  float* k = a.take<float>(rows * (C / 4));
-  float* v = a.take<float>(rows * C);
-  float* r = a.take<float>(rows * C);
-  PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_offset_attention: workspace %zu B < required %zu B",
-             workspace_bytes, a.used);
   auto lin = [&](const float* in, const float* W, const float* b, int N, float* y, int relu, const float* R) {
     GemmF32 g;
     g.A = in; g.lda = C; g.W[0] = W; g.bias[0] = b; g.ldw = C; g.Y = y; g.ldy = N; g.M = (int)rows; g.N = N; g.K = C;
     g.relu = relu; g.R = R; g.ldr = C;
     return launch_gemm_f32(g, st);
   };
-  PZ_TRY(lin(x, Wq, bq, C / 4, q, 0, nullptr));
-  PZ_TRY(lin(x, Wk, bk, C / 4, k, 0, nullptr));
-  PZ_TRY(lin(x, Wv, bv, C, v, 0, nullptr));
-  PZ_TRY(launch_attention(q, C / 4, k, C / 4, v, C, B, L, C / 4, C, x, C, r, C, attention_or_null,
+  PZ_TRY(lin(x, Wq, bq, C / 4, f.q, 0, nullptr));
+  PZ_TRY(lin(x, Wk, bk, C / 4, f.k, 0, nullptr));
+  PZ_TRY(lin(x, Wv, bv, C, f.v, 0, nullptr));
+  PZ_TRY(launch_attention(f.q, C / 4, f.k, C / 4, f.v, C, B, L, C / 4, C, x, C, f.r, C, attention_or_null,
                           attention_or_null ? 1 : 0, st));
-  return lin(r, Wo, bo, C, out, 1, x);
+  return lin(f.r, Wo, bo, C, out, 1, x);
 }
+
+namespace {
+// pz_group_mlp_maxpool's workspace: the int32 neighbour rows [B*S*K], then one layout per precision (pts = B * N source
+// points, centres = B * S)
+struct GroupMlpFp32 { float* F; };   // the feature half of layer 1 [pts, C1]
+size_t layout(Arena& a, size_t pts, size_t, int, int C1, int, GroupMlpFp32& s) {
+  s.F = a.take<float>(pts * C1);
+  return a.used;
+}
+struct GroupMlpBf16 { __nv_bfloat16 *feat, *P, *w1f, *w2; };   // feat [pts, D], P [pts, C1], W1[:,3:] [C1, D], W2 [C2, C1]
+size_t layout(Arena& a, size_t pts, size_t, int D, int C1, int C2, GroupMlpBf16& s) {
+  s.feat = a.take<__nv_bfloat16>(pts * D);
+  s.P = a.take<__nv_bfloat16>(pts * C1);
+  s.w1f = a.take<__nv_bfloat16>((size_t)C1 * D);
+  s.w2 = a.take<__nv_bfloat16>((size_t)C2 * C1);
+  return a.used;
+}
+struct GroupMlpSplit { h16 *feat[2], *w1f[2], *w2[2]; float *P, *Q; };   // [plane]; P [pts, C1], Q [centres, C1]
+size_t layout(Arena& a, size_t pts, size_t centres, int D, int C1, int C2, GroupMlpSplit& s) {
+  s.feat[0] = a.take<h16>(pts * D); s.feat[1] = a.take<h16>(pts * D);
+  s.P = a.take<float>(pts * C1);
+  s.Q = a.take<float>(centres * C1);
+  s.w1f[0] = a.take<h16>((size_t)C1 * D); s.w1f[1] = a.take<h16>((size_t)C1 * D);
+  s.w2[0] = a.take<h16>((size_t)C2 * C1); s.w2[1] = a.take<h16>((size_t)C2 * C1);
+  return a.used;
+}
+}  // namespace
 
 extern "C" size_t pz_group_mlp_workspace_bytes(int B, int N, int D, int S, int K, int C1, int C2) {
   if (B < 1 || N < 1 || S < 1 || K < 1 || C1 < 1 || C2 < 1 || D < 1) return 0;
-  const size_t fp32_path = align_up((size_t)B * N * C1 * sizeof(float), 256);
-  // bf16 path: feat_b [B*N, D], P [B*N, C1], Q [B*S, C1], W1f [C1, D], W2 [C2, C1] (all bf16)
-  const size_t bf16_path = align_up((size_t)B * N * D * 2, 256) + align_up((size_t)B * N * C1 * 2, 256) +
-                           align_up((size_t)B * S * C1 * 2, 256) + align_up((size_t)C1 * D * 2, 256) +
-                           align_up((size_t)C2 * C1 * 2, 256);
-  // split path: feat planes, P fp32, Q fp32, W1f planes, W2 planes
-  const size_t split_path = align_up((size_t)B * N * D * 2, 256) * 2 + align_up((size_t)B * N * C1 * 4, 256) +
-                            align_up((size_t)B * S * C1 * 4, 256) + align_up((size_t)C1 * D * 2, 256) * 2 +
-                            align_up((size_t)C2 * C1 * 2, 256) * 2;
-  const size_t m = fp32_path > bf16_path ? fp32_path : bf16_path;
-  return (m > split_path ? m : split_path) + align_up((size_t)B * S * K * sizeof(int), 256) + 1024;
+  auto bytes = [&](auto&& s) {
+    Arena a(nullptr, 0);
+    a.take<int>((size_t)B * S * K);
+    return layout(a, (size_t)B * N, (size_t)B * S, D, C1, C2, s);
+  };
+  return align_up(std::max({bytes(GroupMlpFp32()), bytes(GroupMlpBf16()), bytes(GroupMlpSplit())}), 256);
 }
 
 extern "C" int pz_group_mlp_maxpool(const float* xyz, const float* feat, const float* new_xyz, const int64_t* knn_idx,
@@ -1942,85 +1952,65 @@ extern "C" int pz_group_mlp_maxpool(const float* xyz, const float* feat, const f
              INT_MAX);
   PZ_REQUIRE(precision == PZ_PREC_FP32 || precision == PZ_PREC_BF16 || precision == PZ_PREC_SPLIT, PZ_ERR_ARG,
              "pz_group_mlp_maxpool: unknown precision %d", precision);
+  PZ_REQUIRE(precision == PZ_PREC_FP32 || (D % 64 == 0 && (C1 == 128 || C1 == 256) && (C2 == 128 || C2 == 256) &&
+                                             ((size_t)B * N) % 128 == 0 && ((size_t)B * S * K) % 256 == 0),
+             PZ_ERR_UNSUPPORTED,
+             "pz_group_mlp_maxpool(%s): needs D %% 64 == 0, C1,C2 in {128,256}, B*N %% 128 == 0, B*S %% 8 == 0",
+             precision == PZ_PREC_SPLIT ? "split" : "bf16");
   cudaStream_t st = as_stream(stream);
   Arena a(workspace, workspace_bytes);
-  const size_t total = (size_t)B * S * K;
+  const size_t total = (size_t)B * S * K, pts = (size_t)B * N, centres = (size_t)B * S;
   int* rows = a.take<int>(total);
-  if (precision == PZ_PREC_SPLIT) {
-    // split path: P = feat W1[:,3:]^T + b1 + W1[:,0:3] xyz and Q = W1[:,0:3] c in fp32, then the split gather GEMM
-    PZ_REQUIRE(D % 64 == 0 && (C1 == 128 || C1 == 256) && (C2 == 128 || C2 == 256) && ((size_t)B * N) % 128 == 0 &&
-                   total % 256 == 0,
-               PZ_ERR_UNSUPPORTED,
-               "pz_group_mlp_maxpool(split): needs D %% 64 == 0, C1,C2 in {128,256}, B*N %% 128 == 0, B*S %% 8 == 0");
-    typedef __nv_bfloat16 h16;
-    h16* fh = a.take<h16>((size_t)B * N * D); h16* fl = a.take<h16>((size_t)B * N * D);
-    float* P = a.take<float>((size_t)B * N * C1);
-    float* Q = a.take<float>((size_t)B * S * C1);
-    h16* w1h = a.take<h16>((size_t)C1 * D); h16* w1l = a.take<h16>((size_t)C1 * D);
-    h16* w2h = a.take<h16>((size_t)C2 * C1); h16* w2l = a.take<h16>((size_t)C2 * C1);
-    PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_group_mlp_maxpool: workspace %zu B < required %zu B",
-               workspace_bytes, a.used);
-    idx64_to_rows32_kernel<<<(int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096), 256, 0, st>>>(
-        knn_idx, total, (size_t)S * K, N, rows);
-    PZ_LAUNCH_CHECK();
-    PackJobs jobs;
-    jobs.j[0] = PackJob{W1 + 3, w1h, 3 + D, C1, D, D, 4};
-    jobs.j[1] = PackJob{W1 + 3, w1l, 3 + D, C1, D, D, 5};
-    jobs.j[2] = PackJob{W2, w2h, C1, C2, C1, C1, 4};
-    jobs.j[3] = PackJob{W2, w2l, C1, C2, C1, C1, 5};
-    jobs.n = 4;
-    pack_weights_kernel<<<dim3(16, 4), 256, 0, st>>>(jobs);
-    PZ_LAUNCH_CHECK();
-    PZ_TRY(launch_split_planes(feat, D, (size_t)B * N, D, fh, fl, D, st));
-    PZ_TRY(launch_centre_proj_f32(new_xyz, W1, W1, 3 + D, B * S, B * S, C1, Q, st));
-    TcGemm g1;
-    g1.X = fh; g1.Xlo = fl; g1.ldx = D; g1.W[0] = w1h; g1.Wlo[0] = w1l; g1.ldw = D; g1.bias[0] = b1; g1.M = B * N; g1.Nout = C1; g1.K = D;
-    g1.Yf = P; g1.ldyf = C1; g1.xyz = xyz; g1.W1x[0] = W1; g1.ldw1x = 3 + D;
-    PZ_TRY(launch_split_rowgemm(g1, st));
-    TcGemm g2;
-    g2.Xf = P; g2.ldx = C1; g2.Qf = Q; g2.rows = rows; g2.W[0] = w2h; g2.Wlo[0] = w2l; g2.ldw = C1; g2.bias[0] = b2; g2.M = (int)total;
-    g2.Nout = C2; g2.K = C1; g2.epi = 1; g2.relu = 1; g2.Yf = out; g2.ldyf = C2;
-    return launch_split_gather(g2, st);
-  }
-  if (precision == PZ_PREC_BF16) {
-    // tensor-core path: P = feat W1[:,3:]^T + b1 + W1[:,0:3] xyz (row GEMM), Q = W1[:,0:3] c, then the gathered GEMM
-    PZ_REQUIRE(D % 64 == 0 && (C1 == 128 || C1 == 256) && (C2 == 128 || C2 == 256) && ((size_t)B * N) % 128 == 0 &&
-                   total % 256 == 0,
-               PZ_ERR_UNSUPPORTED,
-               "pz_group_mlp_maxpool(bf16): needs D %% 64 == 0, C1,C2 in {128,256}, B*N %% 128 == 0, B*S %% 8 == 0");
-    __nv_bfloat16* feat_b = a.take<__nv_bfloat16>((size_t)B * N * D);
-    __nv_bfloat16* P = a.take<__nv_bfloat16>((size_t)B * N * C1);
-    __nv_bfloat16* Q = a.take<__nv_bfloat16>((size_t)B * S * C1);
-    __nv_bfloat16* w1f = a.take<__nv_bfloat16>((size_t)C1 * D);
-    __nv_bfloat16* w2b = a.take<__nv_bfloat16>((size_t)C2 * C1);
-    PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_group_mlp_maxpool: workspace %zu B < required %zu B",
-               workspace_bytes, a.used);
-    idx64_to_rows32_kernel<<<(int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096), 256, 0, st>>>(
-        knn_idx, total, (size_t)S * K, N, rows);
-    PZ_LAUNCH_CHECK();
-    PZ_TRY(launch_cvt_bf16(feat, D, B * N, D, feat_b, D, st));
-    PZ_TRY(launch_cvt_bf16(W1 + 3, 3 + D, C1, D, w1f, D, st));
-    PZ_TRY(launch_cvt_bf16(W2, C1, C2, C1, w2b, C1, st));
-    TcGemm g1;
-    g1.X = feat_b; g1.ldx = D; g1.W[0] = w1f; g1.ldw = D; g1.bias[0] = b1; g1.M = B * N; g1.Nout = C1; g1.K = D;
-    g1.Yb = P; g1.ldyb = C1; g1.xyz = xyz; g1.W1x[0] = W1; g1.ldw1x = 3 + D;
-    PZ_TRY(launch_tc_rowgemm(g1, st));
-    TcGemm g2;
-    g2.X = P; g2.ldx = C1; g2.rows = rows; g2.centers = new_xyz; g2.W1x[0] = W1; g2.ldw1x = 3 + D; (void)Q; g2.W[0] = w2b; g2.ldw = C1; g2.bias[0] = b2; g2.M = (int)total;
-    g2.Nout = C2; g2.K = C1; g2.epi = 1; g2.relu = 1; g2.Yf = out; g2.ldyf = C2;
-    return launch_tc_gemm(g2, st);
-  }
-  float* F = a.take<float>((size_t)B * N * C1);
+  GroupMlpFp32 f = {}; GroupMlpBf16 b = {}; GroupMlpSplit s = {};
+  if (precision == PZ_PREC_SPLIT) layout(a, pts, centres, D, C1, C2, s);
+  else if (precision == PZ_PREC_BF16) layout(a, pts, centres, D, C1, C2, b);
+  else layout(a, pts, centres, D, C1, C2, f);
   PZ_REQUIRE(workspace && a.ok(), PZ_ERR_WORKSPACE, "pz_group_mlp_maxpool: workspace %zu B < required %zu B",
              workspace_bytes, a.used);
   idx64_to_rows32_kernel<<<(int)((total + 255) / 256 < 4096 ? (total + 255) / 256 : 4096), 256, 0, st>>>(
       knn_idx, total, (size_t)S * K, N, rows);
   PZ_LAUNCH_CHECK();
+  if (precision == PZ_PREC_SPLIT) {
+    // split path: P = feat W1[:,3:]^T + b1 + W1[:,0:3] xyz and Q = W1[:,0:3] c in fp32, then the split gather GEMM
+    PackJobs jobs;
+    jobs.j[0] = PackJob{W1 + 3, s.w1f[0], 3 + D, C1, D, D, 4};
+    jobs.j[1] = PackJob{W1 + 3, s.w1f[1], 3 + D, C1, D, D, 5};
+    jobs.j[2] = PackJob{W2, s.w2[0], C1, C2, C1, C1, 4};
+    jobs.j[3] = PackJob{W2, s.w2[1], C1, C2, C1, C1, 5};
+    jobs.n = 4;
+    pack_weights_kernel<<<dim3(16, 4), 256, 0, st>>>(jobs);
+    PZ_LAUNCH_CHECK();
+    PZ_TRY(launch_split_planes(feat, D, pts, D, s.feat[0], s.feat[1], D, st));
+    PZ_TRY(launch_centre_proj_f32(new_xyz, W1, W1, 3 + D, B * S, B * S, C1, s.Q, st));
+    TcGemm g1;
+    g1.X = s.feat[0]; g1.Xlo = s.feat[1]; g1.ldx = D; g1.W[0] = s.w1f[0]; g1.Wlo[0] = s.w1f[1]; g1.ldw = D; g1.bias[0] = b1; g1.M = B * N; g1.Nout = C1; g1.K = D;
+    g1.Yf = s.P; g1.ldyf = C1; g1.xyz = xyz; g1.W1x[0] = W1; g1.ldw1x = 3 + D;
+    PZ_TRY(launch_split_rowgemm(g1, st));
+    TcGemm g2;
+    g2.Xf = s.P; g2.ldx = C1; g2.Qf = s.Q; g2.rows = rows; g2.W[0] = s.w2[0]; g2.Wlo[0] = s.w2[1]; g2.ldw = C1; g2.bias[0] = b2; g2.M = (int)total;
+    g2.Nout = C2; g2.K = C1; g2.epi = 1; g2.relu = 1; g2.Yf = out; g2.ldyf = C2;
+    return launch_split_gather(g2, st);
+  }
+  if (precision == PZ_PREC_BF16) {
+    // tensor-core path: P = feat W1[:,3:]^T + b1 + W1[:,0:3] xyz (row GEMM), then the gathered GEMM forms Q = W1[:,0:3] c
+    // per stage in shared memory
+    PZ_TRY(launch_cvt_bf16(feat, D, B * N, D, b.feat, D, st));
+    PZ_TRY(launch_cvt_bf16(W1 + 3, 3 + D, C1, D, b.w1f, D, st));
+    PZ_TRY(launch_cvt_bf16(W2, C1, C2, C1, b.w2, C1, st));
+    TcGemm g1;
+    g1.X = b.feat; g1.ldx = D; g1.W[0] = b.w1f; g1.ldw = D; g1.bias[0] = b1; g1.M = B * N; g1.Nout = C1; g1.K = D;
+    g1.Yb = b.P; g1.ldyb = C1; g1.xyz = xyz; g1.W1x[0] = W1; g1.ldw1x = 3 + D;
+    PZ_TRY(launch_tc_rowgemm(g1, st));
+    TcGemm g2;
+    g2.X = b.P; g2.ldx = C1; g2.rows = rows; g2.centers = new_xyz; g2.W1x[0] = W1; g2.ldw1x = 3 + D; g2.W[0] = b.w2; g2.ldw = C1; g2.bias[0] = b2; g2.M = (int)total;
+    g2.Nout = C2; g2.K = C1; g2.epi = 1; g2.relu = 1; g2.Yf = out; g2.ldyf = C2;
+    return launch_tc_gemm(g2, st);
+  }
   GemmF32 g1;
-  g1.A = feat; g1.lda = D; g1.W[0] = W1 + 3; g1.ldw = 3 + D; g1.Y = F; g1.ldy = C1; g1.M = B * N; g1.N = C1; g1.K = D;
+  g1.A = feat; g1.lda = D; g1.W[0] = W1 + 3; g1.ldw = 3 + D; g1.Y = f.F; g1.ldy = C1; g1.M = B * N; g1.N = C1; g1.K = D;
   PZ_TRY(launch_gemm_f32(g1, st));
   GemmF32 g2;
-  g2.A = F; g2.lda = C1; g2.rows = rows; g2.xyz = xyz; g2.centers = new_xyz; g2.W1[0] = W1; g2.b1[0] = b1;
+  g2.A = f.F; g2.lda = C1; g2.rows = rows; g2.xyz = xyz; g2.centers = new_xyz; g2.W1[0] = W1; g2.b1[0] = b1;
   g2.ldw1 = 3 + D; g2.W[0] = W2; g2.bias[0] = b2; g2.ldw = C1; g2.Y = out; g2.ldy = C2; g2.M = (int)total;
   g2.N = C2; g2.K = C1; g2.relu = 1; g2.group = 32;
   return launch_gemm_f32(g2, st);
