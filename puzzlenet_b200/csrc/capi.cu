@@ -107,8 +107,7 @@ int side_stream(SideStream** out, cudaStream_t caller) {
     e = &table->back();
     PZ_CUDA(cudaStreamCreateWithFlags(&e->s.stream, cudaStreamNonBlocking));
     PZ_CUDA(cudaEventCreateWithFlags(&e->s.fork, cudaEventDisableTiming));
-    PZ_CUDA(cudaEventCreateWithFlags(&e->s.join_a, cudaEventDisableTiming));
-    PZ_CUDA(cudaEventCreateWithFlags(&e->s.join_b, cudaEventDisableTiming));
+    PZ_CUDA(cudaEventCreateWithFlags(&e->s.join, cudaEventDisableTiming));
   } else {
     for (size_t tries = 0; tries < table->size() && !e; ++tries) {   // recycle an entry of the same device
       Entry& c = (*table)[next_victim++ % table->size()];

@@ -756,48 +756,6 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(const PackJobs jobs) 
   }
 }
 
-// Q[s, k] = W1[k, 0:3] . centre[s]  -- the centroid half of layer 1 of a grouped MLP (the per-neighbour
-// half, P, comes out of the layer-1 GEMM):  relu(W1 [xyz_j - c_s ; f_j] + b1) = relu(P_j - Q_s).  fp32 Q [rows, C1] for
-// the split path.  The three xyz weights of every channel (both weight sets) are staged in shared memory once per block
-// (they sit 3 + D floats apart in the weight matrix); a thread then walks consecutive (row, channel) elements, so the Q
-// stores are coalesced and the centre is a broadcast read.
-__global__ void __launch_bounds__(256) centre_proj_f32_kernel(const float* __restrict__ centres, const float* w1a,
-                                                              const float* w1b, int ldw1, int rows_per_set, int rows,
-                                                              int C1, float* __restrict__ Q) {
-  extern __shared__ float cp_w[];                 // [2 sets][C1][3]
-  for (int i = threadIdx.x; i < 2 * C1 * 3; i += 256) {
-    const int set = i / (C1 * 3), r = i - set * C1 * 3, k = r / 3, d = r - k * 3;
-    cp_w[i] = (set == 0 ? w1a : w1b)[(size_t)k * ldw1 + d];   // model parameters: never written by a kernel
-  }
-  pdl_enter();
-  __syncthreads();
-  // four consecutive channels of a row per thread: one 16-byte store, 32-bit index arithmetic (C1 % 4 == 0, rows * C1 < 2^31)
-  const unsigned c4 = (unsigned)C1 >> 2, total4 = (unsigned)rows * c4;
-  for (unsigned e = blockIdx.x * 256u + threadIdx.x; e < total4; e += gridDim.x * 256u) {
-    const unsigned s = e / c4, k = (e - s * c4) * 4;
-    const float* w = cp_w + (((int)s / rows_per_set == 0 ? 0 : C1) + (int)k) * 3;
-    const float* c = centres + (size_t)s * 3;
-    const float cx = c[0], cy = c[1], cz = c[2];
-    float4 q;
-    q.x = fmaf(w[0], cx, fmaf(w[1], cy, w[2] * cz));
-    q.y = fmaf(w[3], cx, fmaf(w[4], cy, w[5] * cz));
-    q.z = fmaf(w[6], cx, fmaf(w[7], cy, w[8] * cz));
-    q.w = fmaf(w[9], cx, fmaf(w[10], cy, w[11] * cz));
-    *reinterpret_cast<float4*>(Q + (size_t)s * C1 + k) = q;
-  }
-}
-static int launch_centre_proj_f32(const float* centres, const float* w1a, const float* w1b, int ldw1, int rows_per_set, int rows,
-                                  int C1, float* Q, cudaStream_t st) {
-  PZ_REQUIRE(C1 % 4 == 0 && (size_t)rows * C1 < (1ull << 31) && ((uintptr_t)Q & 15) == 0, PZ_ERR_UNSUPPORTED,
-             "centre projection: needs C1 %% 4 == 0, rows * C1 < 2^31 and a 16-byte aligned Q");
-  const size_t total = (size_t)rows * C1 / 4, want = (total + 255) / 256;
-  const unsigned blocks = (unsigned)(want < (size_t)kNumSMs * 8 ? want : (size_t)kNumSMs * 8);
-  PZ_CUDA(launch_pdl(centre_proj_f32_kernel, dim3(blocks), dim3(256), (size_t)2 * C1 * 3 * sizeof(float), st, centres, w1a, w1b, ldw1,
-                     rows_per_set, rows, C1, Q));
-  PZ_LAUNCH_CHECK();
-  return 0;
-}
-
 // ======================================================================== orchestration
 static StemW stem_of(const PzEncoderWeights& w) {
   return StemW{w.mlp1_w, w.mlp1_b, w.mlp2_w, w.mlp2_b, w.bn1_w, w.bn1_b, w.bn1_mean, w.bn1_var,
@@ -897,6 +855,23 @@ static void carve(int C, Arena& a, SplitScratch& s) {
   s.bqkv = a.take<float>(2 * 4 * 384);
 }
 
+// The geometry of a forward -- FPS, kNN and, on the split path, the centre projection Q of each grouped MLP, for both
+// stages -- as one launch (geometry.cu: geometry_c2_kernel).  Q1 / Q2 null: no centre projections.
+static_assert(NPTS == 1024 && S1 == 512 && S2 == 256 && KNN == 32, "launch_encoder_geometry covers this shape only");
+static int encoder_geometry(const PzEncoderWeights& wa, const PzEncoderWeights& wb, int B, int C, const float* xyz,
+                            const int64_t* start1, const int64_t* start2, const PzEncoderOutputs& o, const EncoderCommon& c,
+                            float* Q1, float* Q2, cudaStream_t st) {
+  EncoderGeometry g;
+  g.xyz = xyz; g.start1 = start1; g.start2 = start2;
+  g.fps1 = o.fps1; g.knn1 = o.knn1; g.fps2 = o.fps2; g.knn2 = o.knn2;
+  g.nx1 = c.nx1; g.nx2 = c.nx2; g.knn1r = c.knn1r; g.knn2r = c.knn2r;
+  g.Q1 = Q1; g.Q2 = Q2;
+  g.w1[0] = wa.mlp3_w; g.w1[1] = wb.mlp3_w; g.ldw1 = 3 + D0;
+  g.w2[0] = wa.mlp5_w; g.w2[1] = wb.mlp5_w; g.ldw2 = 3 + C1B;
+  g.clouds_per_set = B;
+  return launch_encoder_geometry(g, C, st);
+}
+
 // ---------------------------------------------------------------------------------------------
 // bf16 path: every dense layer on tcgen05 (gemm_tc.cu), geometry + softmax in fp32.
 // Layer 1 of each grouped MLP is split as  W1 [xyz_j - c_s ; f_j] + b1 = P_j - Q_s  with
@@ -955,8 +930,8 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
   const __nv_bfloat16* wpa = s.wpack;
   const __nv_bfloat16* wpb = s.wpack + (size_t)(E - 1) * WP_TOTAL;
 
-  // ---- geometry (FPS -> kNN, both stages, plus the centroid halves Q of layer 1) depends on coordinates only:
-  // it runs on the side stream while the feature chain (stem, layer-1 GEMM) runs on the caller's stream.
+  // ---- geometry (FPS -> kNN, both stages) depends on coordinates only: it runs on the side stream while the feature
+  // chain (stem, layer-1 GEMMs) runs on the caller's stream.
   SideStream* ss = nullptr;
   PZ_TRY(side_stream(&ss, st));
   const bool serial = prof_serial();
@@ -965,16 +940,9 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
   PZ_CUDA(cudaEventRecord(ss->fork, st));
   PZ_CUDA(cudaStreamWaitEvent(sg, ss->fork, 0));
   prof_mark("_side_begin", sg, gl);
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, sg));
-  prof_mark("fps1", sg, gl);
-  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, sg));
-  prof_mark("knn1", sg, gl);
-  PZ_CUDA(cudaEventRecord(ss->join_a, sg));
-  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, sg));
-  prof_mark("fps2", sg, gl);
-  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, sg));
-  prof_mark("knn2", sg, gl);
-  PZ_CUDA(cudaEventRecord(ss->join_b, sg));
+  PZ_TRY(encoder_geometry(wa, wb, B, C, xyz, start1, start2, o, c, nullptr, nullptr, sg));
+  prof_mark("geometry", sg, gl);
+  PZ_CUDA(cudaEventRecord(ss->join, sg));
 
   PZ_CUDA(cudaFuncSetAttribute(stem_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)STEM_TC_SMEM));
   stem_tc_kernel<false><<<C * NPTS / (128 * HD_REPS), 128, STEM_TC_SMEM, st>>>(xyz, stem_of(wa), stem_of(wb), wpa + WP_STEM,
@@ -990,8 +958,8 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     prof_mark("sg1_layer1", st);
   }
   if (after_stem) PZ_TRY((*after_stem)(c.xfeat));
-  PZ_CUDA(cudaStreamWaitEvent(st, ss->join_a, 0));   // kNN of stage 1 (and FPS 1, Q1) are done
-  prof_mark("_wait_geometry1", st);
+  PZ_CUDA(cudaStreamWaitEvent(st, ss->join, 0));   // the geometry of both stages is done (side stream joined)
+  prof_mark("_wait_geometry", st);
   {
     TcGemm g;  // f1f = max_k relu(W4 relu(P1[j] - Q1[s]) + b4)
     g.X = s.P1; g.ldx = C1A; g.rows = c.knn1r; g.centers = c.nx1; g.W1x[0] = wa.mlp3_w; g.W1x[1] = wb.mlp3_w; g.ldw1x = 3 + D0; g.W[0] = wpa + WP_W4; g.W[1] = wpb + WP_W4; g.ldw = C1A;
@@ -1008,8 +976,6 @@ static int encoder_forward_bf16(const PzEncoderWeights* w, int E, int B, const f
     PZ_TRY(launch_tc_rowgemm(g, st));
     prof_mark("sg2_layer1", st);
   }
-  PZ_CUDA(cudaStreamWaitEvent(st, ss->join_b, 0));   // stage-2 geometry is done (side stream joined)
-  prof_mark("_wait_geometry2", st);
   __nv_bfloat16* cat_b = s.att_cat;             // [C*256, 1280] bf16: cat(att1..att4, f2f)
   float* cat_f = o.att_cat;                     // fp32 copy only when the caller asks for it
   {
@@ -1122,22 +1088,16 @@ static int encoder_forward_split(const PzEncoderWeights* w, int E, int B, const 
   // programmatic launch chain is broken by the memset node
   PZ_CUDA(cudaMemsetAsync(s.flags, 0, (size_t)3 * C * sizeof(int), st));
 
-  // ---- geometry (FPS -> centre projection -> kNN, both stages): ahead of the feature chain on the caller's stream.
+  // ---- geometry (FPS, kNN and the centre projections Q1 / Q2, both stages, one launch): ahead of the feature chain on the
+  // caller's stream.
   // ONE chain: every GEMM CTA of this path fills an SM (shared memory), so a geometry kernel on a second stream does not
   // share SMs with them, it delays some of the CTAs of a persistent GEMM and the whole launch waits for those (eager
   // forward 1.70 ms with a side stream, 1.59 without, 1.51 with programmatic dependent launch on the one chain; the
   // 4-stream graph schedule 1.39 vs 1.37 ms per step).
   prof_mark("_side_begin", st);
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, st));
-  prof_mark("fps1", st);
-  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, st));
-  prof_mark("knn1", st);
-  PZ_TRY(launch_centre_proj_f32(c.nx1, wa.mlp3_w, wb.mlp3_w, 3 + D0, B * S1, C * S1, C1A, s.Q1, st));
-  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, st));
-  prof_mark("fps2", st);
-  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, st));
-  prof_mark("knn2", st);
-  PZ_TRY(launch_centre_proj_f32(c.nx2, wa.mlp5_w, wb.mlp5_w, 3 + C1B, B * S2, C * S2, C2A, s.Q2, st));
+  static_assert(C1A == 128 && C2A == 256, "geometry_c2_kernel writes Q1 / Q2 rows of 128 / 256 channels");
+  PZ_TRY(encoder_geometry(wa, wb, B, C, xyz, start1, start2, o, c, s.Q1, s.Q2, st));
+  prof_mark("geometry", st);
 
   // ---- feature chain
   // stem: layer 2 as a split-fp16 mma.sync product (x_feature within ~1e-6 of the fp32 stem), the fp16 hi / lo planes of
@@ -1260,11 +1220,10 @@ static int encoder_forward_fp32(const PzEncoderWeights* w, int E, int B, const f
   prof_mark("stem", st);
   if (after_stem) PZ_TRY((*after_stem)(c.xfeat));
 
-  // ---- stage 1: FPS 1024->512, kNN 32, grouped MLP 67->128->128, max over K
-  PZ_TRY(launch_fps(xyz, C, NPTS, start1, S1, o.fps1, nullptr, c.nx1, st));
-  prof_mark("fps1", st);
-  PZ_TRY(launch_knn(c.nx1, xyz, C, S1, NPTS, KNN, o.knn1, c.knn1r, nullptr, st));
-  prof_mark("knn1", st);
+  // ---- geometry of both stages: FPS 1024->512, kNN 32, FPS 512->256 on the stage-1 centroids, kNN 32
+  PZ_TRY(encoder_geometry(wa, wb, B, C, xyz, start1, start2, o, c, nullptr, nullptr, st));
+  prof_mark("geometry", st);
+  // ---- stage 1: grouped MLP 67->128->128, max over K
   {
     GemmF32 g;  // F1 = x_feature * mlp3.weight[:, 3:]^T   (bias + xyz part are added per neighbour)
     g.A = c.xfeat; g.lda = D0; g.W[0] = wa.mlp3_w + 3; g.W[1] = wb.mlp3_w + 3; g.ldw = 3 + D0;
@@ -1282,11 +1241,7 @@ static int encoder_forward_fp32(const PzEncoderWeights* w, int E, int B, const f
     PZ_TRY(launch_gemm_f32(g, st));
     prof_mark("sg1_gather_layer2_maxpool", st);
   }
-  // ---- stage 2: FPS 512->256 on the stage-1 centroids, kNN 32, grouped MLP 131->256->256
-  PZ_TRY(launch_fps(c.nx1, C, S1, start2, S2, o.fps2, nullptr, c.nx2, st));
-  prof_mark("fps2", st);
-  PZ_TRY(launch_knn(c.nx2, c.nx1, C, S2, S1, KNN, o.knn2, c.knn2r, nullptr, st));
-  prof_mark("knn2", st);
+  // ---- stage 2: grouped MLP 131->256->256
   {
     GemmF32 g;
     g.A = f1f; g.lda = C1B; g.W[0] = wa.mlp5_w + 3; g.W[1] = wb.mlp5_w + 3; g.ldw = 3 + C1B;

@@ -9,6 +9,7 @@
 #include <stdlib.h>
 
 #include "pz_common.cuh"
+#include "tc_common.cuh"
 
 namespace pz {
 
@@ -408,6 +409,127 @@ __device__ __forceinline__ void knn_insert(unsigned& td, unsigned& ti, unsigned 
   ti = lt ? (ltp ? pi : xi) : ti;
 }
 
+// The selection of one query (every lane holds its coordinates) over the cnt candidates of x / y / z planes pts (plane
+// stride pstride, 16-byte aligned, the tail of the last 1024-candidate sub-chunk filled with far-away points) whose
+// indices are base + position.  (td, ti): the query's ascending list so far, lane l = the l-th smallest key; first:
+// nothing is selected yet.  myq: the warp's 64-entry candidate queue.
+__device__ __forceinline__ void knn_select(const float* pts, int pstride, int base, int cnt, bool first, float qx, float qy,
+                                           float qz, unsigned& td, unsigned& ti, uint2* myq, int lane, unsigned kmask,
+                                           unsigned lt_mask) {
+  unsigned tau = __shfl_sync(0xffffffffu, td, 31);              // distance bits of the current 32nd smallest
+#pragma unroll 1
+  for (int sub = 0; sub < cnt; sub += 1024) {
+    unsigned db[32];   // db[4 t4 + j] = candidate sub + 4 (32 t4 + lane) + j
+    unsigned m0 = 0xffffffffu, m1 = 0xffffffffu;
+#pragma unroll
+    for (int t4 = 0; t4 < 8; ++t4) {
+      const int i0 = sub + (t4 * 32 + lane) * 4;
+      const float4 X = *reinterpret_cast<const float4*>(pts + i0);
+      const float4 Y = *reinterpret_cast<const float4*>(pts + pstride + i0);
+      const float4 Z = *reinterpret_cast<const float4*>(pts + 2 * pstride + i0);
+      const float xs[4] = {X.x, X.y, X.z, X.w}, ys[4] = {Y.x, Y.y, Y.z, Y.w}, zs[4] = {Z.x, Z.y, Z.z, Z.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const unsigned x = __float_as_uint(sqdist3(qx, qy, qz, xs[j], ys[j], zs[j]));
+        db[t4 * 4 + j] = x;
+        m1 = min(m1, max(m0, x));
+        m0 = min(m0, x);
+      }
+    }
+    unsigned thr = tau;
+    if (thr == 0xffffffffu) {   // warp-uniform
+      unsigned hi = __reduce_max_sync(0xffffffffu, m0);   // >= 32 candidates are <= the largest lane minimum
+      unsigned lo = __reduce_min_sync(0xffffffffu, m1);
+      if (lo < hi) {
+#pragma unroll 1
+        for (int it = 0; it < 8 && lo < hi; ++it) {
+          const unsigned mid = lo + ((hi - lo) >> 1);
+          const int c = __reduce_add_sync(0xffffffffu, (m0 <= mid ? 1 : 0) + (m1 <= mid ? 1 : 0));
+          if (c >= 32) hi = mid; else lo = mid + 1;
+        }
+      }
+      thr = hi;
+    }
+    thr = min(thr, 0xfffffffeu);   // the "no candidate" pattern never passes
+    int mine = 0;
+#pragma unroll
+    for (int t = 0; t < 32; ++t) mine += db[t] <= thr ? 1 : 0;
+    int incl = mine;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      const int v = __shfl_up_sync(0xffffffffu, incl, o);
+      if (lane >= o) incl += v;
+    }
+    const int c = __shfl_sync(0xffffffffu, incl, 31);
+    if (c == 0) continue;           // warp-uniform
+    if (c <= 64) {
+      uint2* slot = myq + (incl - mine);
+      const unsigned idx0 = (unsigned)(base + sub + lane * 4);
+#pragma unroll
+      for (int t = 0; t < 32; ++t) {
+        if (db[t] <= thr) *slot++ = make_uint2(db[t], idx0 + (unsigned)((t >> 2) * 128 + (t & 3)));
+      }
+      __syncwarp();
+      int o = 0;
+      if (first && sub == 0 && c >= 32) {   // nothing selected yet: the sorted first 32 entries are the list
+        const uint2 e = myq[lane];
+        const uint2 r = knn_sort_call(e.x, e.y, kmask);
+        td = r.x;
+        ti = r.y;
+        o = 32;
+      }
+      if (c - o > 12) {
+        for (; o < c; o += 32) {
+          const uint2 e = o + lane < c ? myq[o + lane] : make_uint2(0xffffffffu, 0xffffffffu);
+          knn_merge(td, ti, e.x, e.y, lane, kmask);
+        }
+      } else {
+#pragma unroll 1
+        for (; o < c; ++o) {
+          const uint2 e = myq[o];
+          knn_insert(td, ti, e.x, e.y, lane);
+        }
+      }
+      tau = __shfl_sync(0xffffffffu, td, 31);
+      __syncwarp();                 // the queue is rewritten by the next sub-chunk / query
+      continue;
+    }
+    // ---- incremental path: more than 64 candidates under the bound (ties)
+    int qn = 0;
+#pragma unroll 1
+    for (int t = 0; t < 32; ++t) {
+      unsigned dt = 0;               // db[t] without dynamic register indexing
+#pragma unroll
+      for (int u = 0; u < 32; ++u) dt = u == t ? db[u] : dt;
+      const bool pass = dt <= thr;
+      const unsigned m = __ballot_sync(0xffffffffu, pass);
+      if (m == 0u) continue;
+      if (pass)
+        myq[qn + __popc(m & lt_mask)] = make_uint2(dt, (unsigned)(base + sub + ((t >> 2) * 32 + lane) * 4 + (t & 3)));
+      qn += __popc(m);
+      __syncwarp();
+      if (qn >= 32) {
+        const uint2 e = myq[lane];
+        knn_merge(td, ti, e.x, e.y, lane, kmask);
+        tau = __shfl_sync(0xffffffffu, td, 31);
+        thr = min(thr, tau);
+        const int rem = qn - 32;
+        const uint2 carry = lane < rem ? myq[32 + lane] : make_uint2(0u, 0u);
+        __syncwarp();
+        if (lane < rem) myq[lane] = carry;
+        __syncwarp();
+        qn = rem;
+      }
+    }
+    if (qn > 0) {   // flush so that the next sub-chunk starts from an exact 32nd distance
+      const uint2 e = lane < qn ? myq[lane] : make_uint2(0xffffffffu, 0xffffffffu);
+      knn_merge(td, ti, e.x, e.y, lane, kmask);
+      tau = __shfl_sync(0xffffffffu, td, 31);
+      __syncwarp();
+    }
+  }
+}
+
 __global__ void __launch_bounds__(KNN_WARPS * 32, 3) knn_kernel(const float* __restrict__ query,
                                                              const float* __restrict__ xyz, int S,
                                                              int N, int K,
@@ -452,118 +574,7 @@ __global__ void __launch_bounds__(KNN_WARPS * 32, 3) knn_kernel(const float* __r
       const float qx = qp[0], qy = qp[1], qz = qp[2];
       unsigned td = first ? 0xffffffffu : park_d[warp][w][lane];   // lane l holds the l-th smallest key so far
       unsigned ti = first ? 0xffffffffu : park_i[warp][w][lane];
-      unsigned tau = __shfl_sync(0xffffffffu, td, 31);              // distance bits of the current 32nd smallest
-#pragma unroll 1
-      for (int sub = 0; sub < cnt; sub += 1024) {
-        unsigned db[32];   // db[4 t4 + j] = candidate sub + 4 (32 t4 + lane) + j
-        unsigned m0 = 0xffffffffu, m1 = 0xffffffffu;
-#pragma unroll
-        for (int t4 = 0; t4 < 8; ++t4) {
-          const int i0 = sub + (t4 * 32 + lane) * 4;
-          const float4 X = *reinterpret_cast<const float4*>(pts + i0);
-          const float4 Y = *reinterpret_cast<const float4*>(pts + KNN_PSTRIDE + i0);
-          const float4 Z = *reinterpret_cast<const float4*>(pts + 2 * KNN_PSTRIDE + i0);
-          const float xs[4] = {X.x, X.y, X.z, X.w}, ys[4] = {Y.x, Y.y, Y.z, Y.w}, zs[4] = {Z.x, Z.y, Z.z, Z.w};
-#pragma unroll
-          for (int j = 0; j < 4; ++j) {
-            const unsigned x = __float_as_uint(sqdist3(qx, qy, qz, xs[j], ys[j], zs[j]));
-            db[t4 * 4 + j] = x;
-            m1 = min(m1, max(m0, x));
-            m0 = min(m0, x);
-          }
-        }
-        unsigned thr = tau;
-        if (thr == 0xffffffffu) {   // warp-uniform
-          unsigned hi = __reduce_max_sync(0xffffffffu, m0);   // >= 32 candidates are <= the largest lane minimum
-          unsigned lo = __reduce_min_sync(0xffffffffu, m1);
-          if (lo < hi) {
-#pragma unroll 1
-            for (int it = 0; it < 8 && lo < hi; ++it) {
-              const unsigned mid = lo + ((hi - lo) >> 1);
-              const int c = __reduce_add_sync(0xffffffffu, (m0 <= mid ? 1 : 0) + (m1 <= mid ? 1 : 0));
-              if (c >= 32) hi = mid; else lo = mid + 1;
-            }
-          }
-          thr = hi;
-        }
-        thr = min(thr, 0xfffffffeu);   // the "no candidate" pattern never passes
-        int mine = 0;
-#pragma unroll
-        for (int t = 0; t < 32; ++t) mine += db[t] <= thr ? 1 : 0;
-        int incl = mine;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int v = __shfl_up_sync(0xffffffffu, incl, o);
-          if (lane >= o) incl += v;
-        }
-        const int c = __shfl_sync(0xffffffffu, incl, 31);
-        if (c == 0) continue;           // warp-uniform
-        if (c <= 64) {
-          uint2* slot = myq + (incl - mine);
-          const unsigned idx0 = (unsigned)(base + sub + lane * 4);
-#pragma unroll
-          for (int t = 0; t < 32; ++t) {
-            if (db[t] <= thr) *slot++ = make_uint2(db[t], idx0 + (unsigned)((t >> 2) * 128 + (t & 3)));
-          }
-          __syncwarp();
-          int o = 0;
-          if (first && sub == 0 && c >= 32) {   // nothing selected yet: the sorted first 32 entries are the list
-            const uint2 e = myq[lane];
-            const uint2 r = knn_sort_call(e.x, e.y, kmask);
-            td = r.x;
-            ti = r.y;
-            o = 32;
-          }
-          if (c - o > 12) {
-            for (; o < c; o += 32) {
-              const uint2 e = o + lane < c ? myq[o + lane] : make_uint2(0xffffffffu, 0xffffffffu);
-              knn_merge(td, ti, e.x, e.y, lane, kmask);
-            }
-          } else {
-#pragma unroll 1
-            for (; o < c; ++o) {
-              const uint2 e = myq[o];
-              knn_insert(td, ti, e.x, e.y, lane);
-            }
-          }
-          tau = __shfl_sync(0xffffffffu, td, 31);
-          __syncwarp();                 // the queue is rewritten by the next sub-chunk / query
-          continue;
-        }
-        // ---- incremental path: more than 64 candidates under the bound (ties)
-        int qn = 0;
-#pragma unroll 1
-        for (int t = 0; t < 32; ++t) {
-          unsigned dt = 0;               // db[t] without dynamic register indexing
-#pragma unroll
-          for (int u = 0; u < 32; ++u) dt = u == t ? db[u] : dt;
-          const bool pass = dt <= thr;
-          const unsigned m = __ballot_sync(0xffffffffu, pass);
-          if (m == 0u) continue;
-          if (pass)
-            myq[qn + __popc(m & lt_mask)] = make_uint2(dt, (unsigned)(base + sub + ((t >> 2) * 32 + lane) * 4 + (t & 3)));
-          qn += __popc(m);
-          __syncwarp();
-          if (qn >= 32) {
-            const uint2 e = myq[lane];
-            knn_merge(td, ti, e.x, e.y, lane, kmask);
-            tau = __shfl_sync(0xffffffffu, td, 31);
-            thr = min(thr, tau);
-            const int rem = qn - 32;
-            const uint2 carry = lane < rem ? myq[32 + lane] : make_uint2(0u, 0u);
-            __syncwarp();
-            if (lane < rem) myq[lane] = carry;
-            __syncwarp();
-            qn = rem;
-          }
-        }
-        if (qn > 0) {   // flush so that the next sub-chunk starts from an exact 32nd distance
-          const uint2 e = lane < qn ? myq[lane] : make_uint2(0xffffffffu, 0xffffffffu);
-          knn_merge(td, ti, e.x, e.y, lane, kmask);
-          tau = __shfl_sync(0xffffffffu, td, 31);
-          __syncwarp();
-        }
-      }
+      knn_select(pts, KNN_PSTRIDE, base, cnt, first, qx, qy, qz, td, ti, myq, lane, kmask, lt_mask);
       if (!last) {
         park_d[warp][w][lane] = td;
         park_i[warp][w][lane] = ti;
@@ -1158,6 +1169,239 @@ int launch_knn(const float* query, const float* xyz, int B, int S, int N, int K,
   PZ_CUDA(launch_pdl(knn_kernel, grid, dim3(KNN_WARPS * 32), 0, st, query, xyz, S, N, K, out64, out_rows32, out_d2));
   PZ_LAUNCH_CHECK();
   return 0;
+}
+
+// ======================================================================================
+// Centre projection  Q[s, k] = W1[k, 0:3] . centre[s]  -- the centroid half of layer 1 of a grouped MLP (the
+// per-neighbour half, P, comes out of the layer-1 GEMM):  relu(W1 [xyz_j - c_s ; f_j] + b1) = relu(P_j - Q_s).  fp32 Q
+// [rows, C1] for the split path.  centre_proj4 is the one evaluation order: geometry_c2_kernel writes the Q rows of its
+// picks with it, bit-identical to this kernel's.
+// ======================================================================================
+// four consecutive channels; w = their [4][3] xyz weights
+__device__ __forceinline__ float4 centre_proj4(const float* w, float cx, float cy, float cz) {
+  float4 q;
+  q.x = fmaf(w[0], cx, fmaf(w[1], cy, w[2] * cz));
+  q.y = fmaf(w[3], cx, fmaf(w[4], cy, w[5] * cz));
+  q.z = fmaf(w[6], cx, fmaf(w[7], cy, w[8] * cz));
+  q.w = fmaf(w[9], cx, fmaf(w[10], cy, w[11] * cz));
+  return q;
+}
+// The three xyz weights of every channel (both weight sets) are staged in shared memory once per block (they sit 3 + D
+// floats apart in the weight matrix); a thread then walks consecutive (row, channel) elements, so the Q stores are
+// coalesced and the centre is a broadcast read.
+__global__ void __launch_bounds__(256) centre_proj_f32_kernel(const float* __restrict__ centres, const float* w1a,
+                                                              const float* w1b, int ldw1, int rows_per_set, int rows,
+                                                              int C1, float* __restrict__ Q) {
+  extern __shared__ float cp_w[];                 // [2 sets][C1][3]
+  for (int i = threadIdx.x; i < 2 * C1 * 3; i += 256) {
+    const int set = i / (C1 * 3), r = i - set * C1 * 3, k = r / 3, d = r - k * 3;
+    cp_w[i] = (set == 0 ? w1a : w1b)[(size_t)k * ldw1 + d];   // model parameters: never written by a kernel
+  }
+  pdl_enter();
+  __syncthreads();
+  // four consecutive channels of a row per thread: one 16-byte store, 32-bit index arithmetic (C1 % 4 == 0, rows * C1 < 2^31)
+  const unsigned c4 = (unsigned)C1 >> 2, total4 = (unsigned)rows * c4;
+  for (unsigned e = blockIdx.x * 256u + threadIdx.x; e < total4; e += gridDim.x * 256u) {
+    const unsigned s = e / c4, k = (e - s * c4) * 4;
+    const float* w = cp_w + (((int)s / rows_per_set == 0 ? 0 : C1) + (int)k) * 3;
+    const float* c = centres + (size_t)s * 3;
+    *reinterpret_cast<float4*>(Q + (size_t)s * C1 + k) = centre_proj4(w, c[0], c[1], c[2]);
+  }
+}
+int launch_centre_proj_f32(const float* centres, const float* w1a, const float* w1b, int ldw1, int rows_per_set, int rows,
+                           int C1, float* Q, cudaStream_t st) {
+  PZ_REQUIRE(C1 % 4 == 0 && (size_t)rows * C1 < (1ull << 31) && ((uintptr_t)Q & 15) == 0, PZ_ERR_UNSUPPORTED,
+             "centre projection: needs C1 %% 4 == 0, rows * C1 < 2^31 and a 16-byte aligned Q");
+  const size_t total = (size_t)rows * C1 / 4, want = (total + 255) / 256;
+  const unsigned blocks = (unsigned)(want < (size_t)kNumSMs * 8 ? want : (size_t)kNumSMs * 8);
+  PZ_CUDA(launch_pdl(centre_proj_f32_kernel, dim3(blocks), dim3(256), (size_t)2 * C1 * 3 * sizeof(float), st, centres, w1a, w1b, ldw1,
+                     rows_per_set, rows, C1, Q));
+  PZ_LAUNCH_CHECK();
+  return 0;
+}
+
+// ======================================================================================
+// The encoder's geometry in ONE launch, one CTA per cloud (the C2 shape: FPS 1024 -> 512, kNN 32 of the picks among the
+// 1024 points, FPS 512 -> 256 over the picks, kNN 32 of those among the 512, and on the split path the Q rows of both
+// grouped MLPs).  Warp-specialised:
+//   FPS warps (8)   fps_kernel's arg-max chains (same keys, tie rule and start clamp) over the cloud's planes in shared
+//                   memory, synchronised by named barrier 1 over these 256 threads only.  Pick s goes to sel[s] as soon
+//                   as it is known; every 32 picks complete one mbarrier.  Between the stages they turn the 512 picks
+//                   into the planes of the stage-2 cloud.
+//   kNN workers (W) query q of the sequence kNN 1 0..511, kNN 2 0..255 belongs to worker q mod W.  It waits for the
+//                   mbarrier of the query's block of picks, runs knn_select over the planes, writes the neighbours and
+//                   the query's Q row.
+// A lone FPS chain leaves almost all of an SM's issue slots idle (one dependent arg-max per ~200 ns); the workers fill
+// them with kNN work that needs nothing but this cloud's points.  kNN 1's queries are FPS 1's picks and kNN 2's are FPS
+// 2's picks over FPS 1's, read from the same planes and selected by the same code as knn_kernel, so every index (and Q)
+// equals that of fps_kernel + knn_kernel + centre_proj_f32_kernel bit for bit.
+// ======================================================================================
+constexpr int GEO_N = 1024, GEO_S1 = 512, GEO_S2 = 256, GEO_C1 = 128, GEO_C2 = 256;
+constexpr int GEO_FPS_T = 256;             // FPS threads: warps 0-7
+constexpr int GEO_PS = GEO_N + 4;          // plane stride (floats; keeps the float4 candidate loads aligned)
+constexpr int GEO_BLK = 32;                // picks per hand-off mbarrier
+constexpr int GEO_NBAR = GEO_S1 / GEO_BLK + GEO_S2 / GEO_BLK;
+constexpr int GEO_W = 16;                  // kNN worker warps (measured: scripts/bench_geometry.py)
+
+__device__ __forceinline__ void geo_fps_sync() { asm volatile("bar.sync 1, %0;" ::"n"(GEO_FPS_T) : "memory"); }
+
+// fps_kernel's loop over the n <= PPT * 256 points of planes xs (stride GEO_PS), run by the 256 FPS threads: S picks
+// from `far` into sel; pick 32 b + 31 completes mbarrier bars[b]
+template <int PPT>
+__device__ __forceinline__ void geo_fps_chain(const float* xs, int n, int S, int far, int* sel, const uint64_t* bars,
+                                              unsigned (*whi)[32], unsigned (*wlo)[32], int t) {
+  const float* ys = xs + GEO_PS;
+  const float* zs = ys + GEO_PS;
+  const int lane = t & 31, warp = t >> 5;
+  float px[PPT], py[PPT], pz_[PPT], md[PPT];
+#pragma unroll
+  for (int j = 0; j < PPT; ++j) {
+    const int i = t + j * GEO_FPS_T;
+    const bool ok = i < n;
+    px[j] = ok ? xs[i] : 0.f;
+    py[j] = ok ? ys[i] : 0.f;
+    pz_[j] = ok ? zs[i] : 0.f;
+    md[j] = ok ? 1e10f : 0.f;
+  }
+  for (int s = 0; s < S; ++s) {
+    if (t == 0) {
+      sel[s] = far;
+      if (s % GEO_BLK == GEO_BLK - 1) tc::mbar_arrive(tc::smem_u32(bars + s / GEO_BLK));   // release: orders sel[]
+    }
+    if (s + 1 == S) break;
+    const float cx = xs[far], cy = ys[far], cz = zs[far];
+    float best = -1.f;
+    int bestj = 0;
+#pragma unroll
+    for (int j = 0; j < PPT; ++j) {
+      md[j] = fminf(md[j], sqdist3(px[j], py[j], pz_[j], cx, cy, cz));
+      const bool gt = md[j] > best;
+      best = gt ? md[j] : best;
+      bestj = gt ? j : bestj;
+    }
+    const unsigned int hi = __float_as_uint(best);
+    const unsigned int lo = ~(unsigned int)(t + bestj * GEO_FPS_T);
+    const unsigned int mhi = __reduce_max_sync(0xffffffffu, hi);
+    const unsigned int mlo = __reduce_max_sync(0xffffffffu, hi == mhi ? lo : 0u);
+    const int par = s & 1;
+    if (lane == 0) {
+      whi[par][warp] = mhi;
+      wlo[par][warp] = mlo;
+    }
+    geo_fps_sync();
+    const unsigned int h2 = whi[par][lane];
+    const unsigned int l2 = wlo[par][lane];
+    const unsigned int ghi = __reduce_max_sync(0xffffffffu, h2);
+    const unsigned int glo = __reduce_max_sync(0xffffffffu, h2 == ghi ? l2 : 0u);
+    far = (int)(~glo);
+  }
+}
+
+template <int W>
+__global__ void __launch_bounds__(GEO_FPS_T + 32 * W, 1) geometry_c2_kernel(const EncoderGeometry g) {
+  static_assert(GEO_S1 % GEO_BLK == 0 && GEO_S2 % GEO_BLK == 0, "whole blocks of picks");
+  __shared__ __align__(16) float p0[3 * GEO_PS];     // the cloud: x / y / z planes
+  __shared__ __align__(16) float p1[3 * GEO_PS];     // FPS 1's picks, in pick order; 512 .. 1023 far away (knn_kernel's pad)
+  __shared__ int sel1[GEO_S1], sel2[GEO_S2];
+  __shared__ unsigned whi[2][32], wlo[2][32];
+  __shared__ uint2 qkey[W > 0 ? W : 1][64];          // per-worker candidate queue
+  __shared__ float cw[(GEO_C1 + GEO_C2) * 3];        // this cloud's xyz weights of both layers, [channel][3]
+  __shared__ __align__(8) uint64_t bars[GEO_NBAR + 1];   // the blocks of picks, then "p1 is complete"
+  const int c = blockIdx.x;
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+  const uint64_t* p1_ready = bars + GEO_NBAR;
+
+  if (g.Q1) {   // model parameters: never written by a kernel
+    const int set = c < g.clouds_per_set ? 0 : 1;
+    for (int i = t; i < (GEO_C1 + GEO_C2) * 3; i += blockDim.x) {
+      const int k = i / 3, d = i - 3 * k;
+      cw[i] = k < GEO_C1 ? g.w1[set][(size_t)k * g.ldw1 + d] : g.w2[set][(size_t)(k - GEO_C1) * g.ldw2 + d];
+    }
+  }
+  if (t < 64) (&whi[0][0])[t] = 0u, (&wlo[0][0])[t] = 0u;   // slots of absent warps stay 0 = "no candidate"
+  if (t == 0) {
+    for (int b = 0; b < GEO_NBAR; ++b) tc::mbar_init(tc::smem_u32(bars + b), 1);
+    tc::mbar_init(tc::smem_u32(p1_ready), GEO_FPS_T);
+  }
+  pdl_enter();
+  const float* p = g.xyz + (size_t)c * GEO_N * 3;
+  for (int i = t; i < GEO_N * 3; i += blockDim.x) {
+    const int pt = i / 3, d = i - pt * 3;
+    p0[d * GEO_PS + pt] = p[i];
+  }
+  __syncthreads();   // the only CTA-wide barrier: from here on the FPS warps and the workers meet at mbarriers only
+
+  if (warp < GEO_FPS_T / 32) {
+    // ---- stage 1: FPS 1024 -> 512
+    geo_fps_chain<GEO_N / GEO_FPS_T>(p0, GEO_N, GEO_S1, min(max((int)g.start1[c], 0), GEO_N - 1), sel1, bars, whi, wlo, t);
+    geo_fps_sync();
+    for (int s = t; s < GEO_PS; s += GEO_FPS_T) {   // the stage-2 cloud, and fps1 / nx1
+      const int f = s < GEO_S1 ? sel1[s] : 0;
+#pragma unroll
+      for (int d = 0; d < 3; ++d) {
+        const float v = p0[d * GEO_PS + f];
+        p1[d * GEO_PS + s] = s < GEO_S1 ? v : 1e18f;
+        if (s < GEO_S1) g.nx1[((size_t)c * GEO_S1 + s) * 3 + d] = v;
+      }
+      if (s < GEO_S1 && g.fps1) g.fps1[(size_t)c * GEO_S1 + s] = f;
+    }
+    tc::mbar_arrive(tc::smem_u32(p1_ready));
+    geo_fps_sync();
+    // ---- stage 2: FPS 512 -> 256 over the picks
+    geo_fps_chain<GEO_S1 / GEO_FPS_T>(p1, GEO_S1, GEO_S2, min(max((int)g.start2[c], 0), GEO_S1 - 1), sel2,
+                                      bars + GEO_S1 / GEO_BLK, whi, wlo, t);
+    geo_fps_sync();
+    for (int s = t; s < GEO_S2; s += GEO_FPS_T) {
+      const int f = sel2[s];
+#pragma unroll
+      for (int d = 0; d < 3; ++d) g.nx2[((size_t)c * GEO_S2 + s) * 3 + d] = p1[d * GEO_PS + f];
+      if (g.fps2) g.fps2[(size_t)c * GEO_S2 + s] = f;
+    }
+    return;
+  }
+  if constexpr (W > 0) {
+    const int wk = warp - GEO_FPS_T / 32;
+    const unsigned kmask = bitonic_keep_mask(lane);
+    const unsigned lt_mask = (1u << lane) - 1u;
+    uint2* myq = qkey[wk];
+#pragma unroll 1
+    for (int q = wk; q < GEO_S1 + GEO_S2; q += W) {
+      const bool two = q >= GEO_S1;
+      const int s = two ? q - GEO_S1 : q, S = two ? GEO_S2 : GEO_S1, N = two ? GEO_S1 : GEO_N;
+      if (two) tc::mbar_wait(tc::smem_u32(p1_ready), 0);
+      tc::mbar_wait(tc::smem_u32(bars + q / GEO_BLK), 0);   // the blocks of both stages are consecutive
+      const float* pts = two ? p1 : p0;
+      const int f = (two ? sel2 : sel1)[s];
+      const float qx = pts[f], qy = pts[GEO_PS + f], qz = pts[2 * GEO_PS + f];
+      unsigned td = 0xffffffffu, ti = 0xffffffffu;
+      knn_select(pts, GEO_PS, 0, N, true, qx, qy, qz, td, ti, myq, lane, kmask, lt_mask);
+      const size_t row = (size_t)c * S + s;
+      int64_t* out64 = two ? g.knn2 : g.knn1;
+      if (out64) out64[row * 32 + lane] = (int64_t)ti;
+      (two ? g.knn2r : g.knn1r)[row * 32 + lane] = c * N + (int)ti;
+      if (g.Q1) {   // this query's Q row: 128 (stage 1) or 256 (stage 2) channels, four per lane and pass
+        const int C1 = two ? GEO_C2 : GEO_C1;
+        float* Q = (two ? g.Q2 : g.Q1) + row * C1;
+        const float* w = cw + (two ? GEO_C1 * 3 : 0);
+        for (int k = lane * 4; k < C1; k += 128)
+          *reinterpret_cast<float4*>(Q + k) = centre_proj4(w + k * 3, qx, qy, qz);
+      }
+    }
+  }
+}
+
+template <int W>
+int launch_encoder_geometry_w(const EncoderGeometry& g, int C, cudaStream_t st) {
+  PZ_REQUIRE(C >= 1 && g.xyz && g.start1 && g.start2 && g.nx1 && g.nx2 && (W == 0 || (g.knn1r && g.knn2r)), PZ_ERR_ARG,
+             "encoder geometry: missing buffers");
+  PZ_REQUIRE(!g.Q1 || (g.Q2 && ((uintptr_t)g.Q1 & 15) == 0 && ((uintptr_t)g.Q2 & 15) == 0), PZ_ERR_ARG,
+             "encoder geometry: Q1 / Q2 must both be given and 16-byte aligned");
+  PZ_CUDA(launch_pdl(geometry_c2_kernel<W>, dim3(C), dim3(GEO_FPS_T + 32 * W), 0, st, g));
+  PZ_LAUNCH_CHECK();
+  return 0;
+}
+int launch_encoder_geometry(const EncoderGeometry& g, int C, cudaStream_t st) {
+  return launch_encoder_geometry_w<GEO_W>(g, C, st);
 }
 
 // ======================================================================================

@@ -85,7 +85,7 @@ void prof_mark(const char* stage, cudaStream_t st, int lane = 0);   // lane 1 = 
 // and reused by every call on that stream (capturable: the side stream is always joined back into the caller's stream).
 struct SideStream {
   cudaStream_t stream = nullptr;
-  cudaEvent_t fork = nullptr, join_a = nullptr, join_b = nullptr;
+  cudaEvent_t fork = nullptr, join = nullptr;
 };
 int side_stream(SideStream** out, cudaStream_t caller);
 bool prof_serial();   // pz_profile_enable(2): run the geometry chain on the caller's stream (clean per-stage times)
@@ -118,6 +118,26 @@ int launch_fps(const float* xyz, int B, int N, const int64_t* start64, int S, in
                int* out_rows32, float* new_xyz, cudaStream_t st);
 int launch_knn(const float* query, const float* xyz, int B, int S, int N, int K, int64_t* out64,
                int* out_rows32, float* out_d2, cudaStream_t st);
+// Q[s, k] = W1[k, 0:3] . centres[s] with weight set s / rows_per_set (0 or 1), fp32 [rows, C1]
+int launch_centre_proj_f32(const float* centres, const float* w1a, const float* w1b, int ldw1, int rows_per_set, int rows,
+                           int C1, float* Q, cudaStream_t st);
+// The encoder's geometry in one launch per cloud, C clouds [C, 1024, 3]: FPS 1024 -> 512 from start1, kNN 32 of the picks,
+// FPS 512 -> 256 over the picks from start2, kNN 32 of those; on the split path also the centre projections Q1 / Q2 of the
+// two grouped MLPs.  Every output equals that of launch_fps, launch_knn and launch_centre_proj_f32 at these shapes.
+struct EncoderGeometry {
+  const float* xyz = nullptr;
+  const int64_t *start1 = nullptr, *start2 = nullptr;                           // [C]
+  int64_t *fps1 = nullptr, *knn1 = nullptr, *fps2 = nullptr, *knn2 = nullptr;   // optional: [C,512] [C,512,32] [C,256] [C,256,32]
+  float *nx1 = nullptr, *nx2 = nullptr;                                         // picked points [C,512,3] / [C,256,3]
+  int *knn1r = nullptr, *knn2r = nullptr;                                       // neighbours as rows c * N + index
+  // optional (split path): Q1 [C*512, 128] and Q2 [C*256, 256] from the xyz columns of w1 / w2 (row strides ldw1 / ldw2);
+  // cloud c uses weight set c < clouds_per_set ? 0 : 1
+  float *Q1 = nullptr, *Q2 = nullptr;
+  const float* w1[2] = {nullptr, nullptr};
+  const float* w2[2] = {nullptr, nullptr};
+  int ldw1 = 0, ldw2 = 0, clouds_per_set = 0;
+};
+int launch_encoder_geometry(const EncoderGeometry& g, int C, cudaStream_t st);
 
 // gemm_f32.cu
 struct GemmF32 {
